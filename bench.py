@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload prove|msm|ntt] [--k K] [--log-n L]
   python bench.py --impl reference ...     # CPU arm: the oracle's restatement of halo2's CPU
                                            # prover / best_multiexp / best_fft on this box's cores
+  python bench.py --dump-outputs DIR ...   # also write what the last timed step computed to DIR/*.npy
 
 Workloads (one "step" = one pass of the hot path over one batch of synthetic input):
   prove (default) : create_proof for the reference's Merkle Sum Tree circuit (chips.py: Poseidon
@@ -24,6 +25,7 @@ block: one MSM 2^26 by point range and one NTT 2^26 four-step over the same N GP
 2^24.  --mode replicas gives the round-1 behaviour (one independent proof per GPU, weak scaling).
 """
 import argparse
+import atexit
 import ctypes
 import importlib
 import json
@@ -37,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (it may be read-only)
 
 # measured on this pool's B200 with tools/imad_bench.cu (profiles/r01_imad_microbench.jsonl):
 # IMAD.WIDE.U32 issues at 32 lanes/clk/SM -> 9.19e12 wide multiply-adds per second
@@ -105,6 +108,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.device), f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)         # a run that fails before stop() leaves no sampler behind
         except Exception:
             self.proc = None
 
@@ -206,6 +210,7 @@ def run_gpu(args):
             "data": "synthetic", "impl": "b200zk"}
     extra = {}
     sharded_proof = False
+    restore = None                              # ntt: puts the seeded input back before the last timed step
     if args.workload == "prove":
         k = args.k
         n = 1 << k
@@ -244,6 +249,9 @@ def run_gpu(args):
         def step_e2e():
             return pk.create_proof(h_cols, inst, h_wide, tr_repr)
 
+        def outputs(proof):
+            return {"proof": np.frombuffer(proof, dtype=np.uint8)}
+
         unit, metric, hib = "ms", "create_proof_ms", False
         h2d, d2h = int(h_adv.nbytes + h_wide.nbytes), pk.proof_size
         dtype = "u32x8 Montgomery (bn256 Fr/Fq, IMAD pipe)"
@@ -271,6 +279,9 @@ def run_gpu(args):
         def step_e2e():
             return sc.commit(h_scalars)
 
+        def outputs(point):
+            return {"msm": point}
+
         unit, metric, hib = "Mpts/s", "msm_mpts_per_s", True
         units_per_step = n / 1e6                                  # per rank; value multiplies by world
         if world > 1:
@@ -293,6 +304,12 @@ def run_gpu(args):
         def step_e2e():
             be._check(zk.lib().b200zk_fft(be._ctx, h_a.ctypes.data_as(ctypes.c_void_p), omega.ctypes.data_as(ctypes.c_void_p), L))
 
+        def restore():
+            d_a.upload(h_a)
+
+        def outputs(_):
+            return {"ntt": d_a.download((n, 4))}                   # transformed in place
+
         if world > 1:
             # ONE transform of 2^L elements sharded four-step (strong scaling): column blocks ->
             # column step -> NCCL all-to-all over NVLink -> row step (halo2-experiments_b200/sharded.py)
@@ -312,7 +329,13 @@ def run_gpu(args):
             pinned_np = pinned.numpy()
 
             def step_dev():
-                fs.forward(block, omega, omega_c)
+                return fs.forward(block, omega, omega_c)
+
+            def restore():                                          # the NCCL path's column step overwrites the block
+                block.copy_(pinned, non_blocking=False)
+
+            def outputs(rows):                                      # this rank's output rows
+                return {"ntt": rows.download((n, 4)) if fused else rows.cpu().numpy().view(np.uint64).reshape(n, 4)}
 
             def step_e2e():
                 block.copy_(pinned, non_blocking=False)
@@ -332,15 +355,30 @@ def run_gpu(args):
         workload = WORKLOAD_TEXT["ntt"].format(L=L)
 
     # ---- device-timed region: inputs resident in HBM --------------------------------
-    last = None
     for _ in range(max(args.warmup, 3)):
-        last = step_dev()
+        step_dev()
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     l0 = be.launch_count()
-    ms = timed(be, dist, local, args.steps, step_dev)
+    result = [None]
+
+    def step_kept():
+        result[0] = None                        # no step's output is held while the next step runs
+        result[0] = step_dev()
+
+    if restore is None:
+        ms = timed(be, dist, local, args.steps, step_kept)
+    else:
+        # the transform runs in place, so the last timed step starts again from the seeded input: what it computes
+        # (and --dump-outputs writes) is the transform of that input; the copy stays outside both timed windows
+        ms = timed(be, dist, local, args.steps - 1, step_kept)
+        restore()
+        ms += timed(be, dist, local, 1, step_kept)
     launches = (be.launch_count() - l0) // args.steps
+    last = result[0]                            # what the last timed step computed: verified and dumped below
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, outputs(last))
     if args.workload == "prove":
         extra["phase_ms"] = pk.last_phase_ms()
         extra["timeline_ms"] = pk.last_trace()
@@ -627,7 +665,6 @@ def cpu_sample(args):
     from __graft_entry__ import load_package
     from oracle import binding as orc
     from oracle import pyref
-    orc.build()
     if args.workload == "prove":
         zk = load_package()
         ks = args.k if args.cpu_k is None else min(args.k, args.cpu_k)
@@ -673,23 +710,16 @@ def cpu_baseline(args, gpu_proof=None):
 def run_reference(args):
     """--impl reference: halo2's CPU algorithm (oracle restatement; the Rust crate cannot be built here) on this
     box's host cores, same metric and config.  prove: every step is one complete create_proof at the benchmarked k
-    (about a minute on 16 cores), so the run times as many of the requested steps as fit in --ref-budget-s
-    (a few minutes for the whole run; at least one) and says how many in `steps_timed`; nothing is extrapolated."""
+    (about a minute on 16 cores); the run times exactly --steps of them; nothing is extrapolated."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     from oracle import binding as orc
-    t_begin = time.perf_counter()                       # the budget covers key generation and the warm-up proof as well
     fn, units, desc, size = cpu_sample(args)
     cores = orc.get_threads()
-    budget = args.ref_budget_s if args.workload == "prove" else float("inf")
-    warm, t_w = 0, time.perf_counter()
     for _ in range(min(args.warmup, 1)):
-        fn(); warm += 1
-    per = (time.perf_counter() - t_w) / max(warm, 1)
+        fn()
     times = []
     while len(times) < args.steps:
-        if times and (time.perf_counter() - t_begin) + max(per, np.mean(times)) > budget:
-            break
         t0 = time.perf_counter()
         fn()
         times.append(time.perf_counter() - t0)
@@ -710,6 +740,25 @@ def run_reference(args):
           "config": {"workload": workload, "same_config_as_gpu_arm": size == (args.k if args.workload == "prove" else args.log_n)},
           "cpu_baseline": {"value": v, "unit": unit, "cores": cores, "kind": "port", "sample": sample},
           "e2e": {"value": v, "unit": unit, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}})
+
+
+DUMP_ROWS, DUMP_SEED = 1 << 16, 1234
+
+
+def write_outputs(path, arrays):
+    """--dump-outputs: every array as path/<name>.npy in float64, so that two builds can be compared output for output.
+    Integers are stored exactly (a 64-bit limb as its two 32-bit halves, low half first).  An output of more than
+    DUMP_ROWS rows is replaced by the same seeded sample of its rows in every run; their indices go to <name>_rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        if a.dtype == np.uint64:
+            a = a.view(np.uint32)
+        if a.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.Generator(np.random.PCG64(DUMP_SEED)).choice(a.shape[0], DUMP_ROWS, replace=False))
+            a = a[rows]
+            np.save(os.path.join(path, name + "_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
 
 
 _JSON_OUT = None
@@ -738,7 +787,6 @@ def main():
     ap.add_argument("--k", type=int, default=20, help="prove: circuit size")
     ap.add_argument("--circuit", default="mst", choices=sorted(CIRCUITS), help="prove: circuit shape")
     ap.add_argument("--cpu-k", type=int, default=None, help="prove: size of the CPU arm's proof (default: the benchmarked k; smaller only for quick local runs)")
-    ap.add_argument("--ref-budget-s", type=float, default=300.0, help="--impl reference, prove: wall-clock budget of the whole run (key generation, one warm-up proof, timed proofs); at least one complete proof is timed")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--log-n", type=int, default=24, help="msm / ntt size")
     ap.add_argument("--cpu-log-n", type=int, default=None, help="msm / ntt: size of the bounded CPU sample")
@@ -747,7 +795,13 @@ def main():
     ap.add_argument("--no-sharded-sweep", action="store_true", help="prove: skip the MSM / NTT 2^26 block")
     ap.add_argument("--sweep-log-n", type=int, default=26)
     ap.add_argument("--sweep-verify-log-n", type=int, default=24)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0: the proof, the MSM point or the NTT output) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path")
     if args.cpu_log_n is None:
         args.cpu_log_n = 20 if args.workload == "msm" else 22
     if args.impl == "reference":
