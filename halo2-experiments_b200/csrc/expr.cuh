@@ -5,20 +5,24 @@
 // intermediates stay on chip.
 //
 // The program is the constraint system's expressions in postfix order over a small value
-// stack, plus FOLD instructions that implement the Horner folds upstream expresses as
-// Calculation::Horner:  acc <- acc * factor + pop().
-//   custom gates : every gate polynomial followed by FOLD(acc0, y)
+// stack, plus instructions that accumulate them:
+//   custom gates : every gate polynomial followed by WSUM:  acc0 <- acc0 + pop() * w[i], where
+//                  w[i] = y^e_i is gate i's power of y in evaluate_h (uploaded per proof, see
+//                  quot_plan.hpp) — one multiplication per gate, as upstream's Horner fold in y,
+//                  but independent of which other gates the program holds, so that gates of
+//                  different degree can run as separate programs on different numbers of cosets
 //   lookups      : input expressions with FOLD(acc0, theta), table expressions with FOLD(acc1, theta)
+//                  (FOLD is the Horner step acc <- acc * factor + pop())
 // Like upstream's GraphEvaluator (which interns every Calculation once), repeated sub-expressions
-// are evaluated once per row: the host (ex_share_common in prover.cu) hash-conses the expression
+// are evaluated once per row: the host (ex_share_common in expr_share.hpp) hash-conses the expression
 // trees, and a shared node is computed at its first use, kept with TEE(slot) and re-read with
 // TMP(slot).  In the Merkle Sum Tree circuit the five (state + rc)^5 terms of Pow5Chip's
 // "full round" gate appear in five polynomials each, and the compressed-selector products
 // q(1-q)(2-q).. in every polynomial they gate: 281 -> ~150 multiplications per row.
 // Consecutive gate polynomials with a common factor (every constraint of a gate is
-// selector * poly) are folded as  acc0 <- acc0 * y^m + s * (p_0 y^(m-1) + ... + p_(m-1)):  the inner
-// Horner sum runs in acc1 (SET1 / FOLD), GROUP(m) multiplies it by the factor once — m - 1
-// multiplications less than folding s * p_i one by one.
+// selector * poly) are accumulated as  acc0 <- acc0 + s * (p_0 w_0 + ... + p_(m-1) w_(m-1)):  the inner
+// sum runs in acc1 (WSUM into acc1), GROUP multiplies it by the factor once — m - 1
+// multiplications less than accumulating s * p_i one by one.
 // Upstream orders the same arithmetic differently; the value per row is the same field element,
 // hence bit-exact.
 #pragma once
@@ -26,7 +30,9 @@
 
 namespace b200zk {
 
-enum : uint32_t { EX_CONST = 0, EX_FIXED = 1, EX_ADVICE = 2, EX_INSTANCE = 3, EX_NEG = 4, EX_ADD = 5, EX_MUL = 6, EX_SCALE = 7, EX_FOLD = 8, EX_TEE = 9, EX_TMP = 10, EX_SET1 = 11, EX_GROUP = 12 };
+enum : uint32_t { EX_CONST = 0, EX_FIXED = 1, EX_ADVICE = 2, EX_INSTANCE = 3, EX_NEG = 4, EX_ADD = 5, EX_MUL = 6, EX_SCALE = 7, EX_FOLD = 8, EX_TEE = 9, EX_TMP = 10, EX_WSUM = 11, EX_GROUP = 12 };
+// WSUM argument: weight index | target (acc0 += v w, acc1 += v w, acc1 = v w)
+enum : uint32_t { EXW_ACC0 = 0u << 20, EXW_ACC1 = 1u << 20, EXW_SET1 = 2u << 20, EXW_INDEX = (1u << 20) - 1 };
 enum : uint32_t { EXF_THETA = 0, EXF_BETA = 1, EXF_GAMMA = 2, EXF_Y = 3 };
 // output modes
 enum : uint32_t {
@@ -53,7 +59,7 @@ struct ExprArgs {
     uint32_t row0;                      // first row (a rank of a sharded proof evaluates its own cosets only)
     uint32_t rot_scale;                 // 1
     fe_t factors[4];                    // theta, beta, gamma, y
-    fe_t ypow[9];                       // y^m for GROUP(m), m <= 8 (gate programs only)
+    const fe_t* wts;                    // per-gate weights y^e_i of WSUM (gate programs only)
     uint32_t mode;
     fe_t* out0;
     fe_t* out1;
@@ -89,12 +95,15 @@ ZK_D void expr_eval_row(const ExprArgs& a, uint32_t idx) {
                 else acc1 = Fr::add(Fr::mul(acc1, f), v);
                 break;
             }
-            case EX_SET1: acc1 = stk[--sp]; break;
-            case EX_GROUP: {
-                fe_t v = stk[--sp];
-                acc0 = Fr::add(Fr::mul(acc0, a.ypow[arg]), Fr::mul(v, acc1));
+            case EX_WSUM: {
+                fe_t v = Fr::mul(stk[--sp], a.wts[arg & EXW_INDEX]);
+                const uint32_t to = arg & ~EXW_INDEX;
+                if (to == EXW_ACC0) acc0 = Fr::add(acc0, v);
+                else if (to == EXW_ACC1) acc1 = Fr::add(acc1, v);
+                else acc1 = v;
                 break;
             }
+            case EX_GROUP: acc0 = Fr::add(acc0, Fr::mul(stk[--sp], acc1)); break;
             case EX_TEE: tmp[arg] = stk[sp - 1]; break;
             case EX_TMP: stk[sp++] = tmp[arg]; break;
             default: break;

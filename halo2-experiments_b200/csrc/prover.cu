@@ -8,7 +8,9 @@
 #include "comm.hpp"
 #include "cs_desc.hpp"
 #include "expr.cuh"
+#include "expr_share.hpp"
 #include "prover_kernels.cuh"
+#include "quot_plan.hpp"
 #include "transcript.hpp"
 #include <algorithm>
 #include <array>
@@ -67,9 +69,10 @@ __global__ void __launch_bounds__(PK_THREADS) quot_lookup_kernel(const QuotLooku
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < a.rows) quot_lookup_row(a, a.row0 + i);
 }
-__global__ void __launch_bounds__(PK_THREADS) coset_interpolate_kernel(const fe_t* g, const fe_t* inv_pow, const fe_t* vinv, uint32_t C, size_t n, fe_t* out, const fe_t* extra) {
+__global__ void __launch_bounds__(PK_THREADS) coset_interpolate_kernel(const fe_t* g, const fe_t* inv_pow, const fe_t* vinv, uint32_t C, size_t n, fe_t* out, const fe_t* extra,
+                                                                      const fe_t* lin) {
     size_t r = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r < n) coset_interpolate_row(g, inv_pow, vinv, C, n, out, r, extra);
+    if (r < n) coset_interpolate_row(g, inv_pow, vinv, C, n, out, r, extra, lin);
 }
 __global__ void __launch_bounds__(PK_THREADS) lookup_extrapolate_kernel(fe_t* g, const fe_t* inv_pow, const fe_t* lambda, const fe_t* tinv, uint32_t CL, uint32_t C, size_t n) {
     size_t r = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -130,15 +133,20 @@ struct b200zk_pk {
     fe_t *coset_pow = nullptr, *coset_pow_inv = nullptr;      // c_j^r and c_j^-r, [q][n]
     fe_t *coset_fac = nullptr, *vinv = nullptr;               // extended_omega^j [q]; inverse Vandermonde of c_j^n [q*q]
     std::vector<HFr> coset_t;                                  // 1 / (c_j^n - 1): the vanishing polynomial on coset j
-    // lookup terms on lk_cosets_n < q cosets (prover_kernels.cuh, lookup_extrapolate_row); == q: not split
+    // lookup terms and low-degree gates on lk_cosets_n = plan.low < q cosets (prover_kernels.cuh, lookup_extrapolate_row);
+    // == q: not split (no lookups, or lookups of the full degree)
     uint32_t lk_cosets_n = 0;
+    QuotPlan plan;
     // lookup cosets and table values of ALL lookups kept side by side (4 arrays of lk_cosets_n * n per lookup), so that they
     // are computed on the side stream while the transcript-bound phases run; false = one lookup at a time after y (less memory)
     bool lk_early = false;
-    fe_t *lk_lambda = nullptr, *coset_t_dev = nullptr;        // extrapolation weights [(q - CL) x CL]; coset_t on the device [q]
+    fe_t* lk_lambda = nullptr;                                 // extrapolation weights [(q - CL) x CL]
     // device program data
-    uint32_t* d_prog = nullptr;                       // gates program | lookup programs
-    uint32_t gates_len = 0;
+    uint32_t* d_prog = nullptr;                       // gate programs of the three classes (quot_plan.hpp) | lookup programs
+    std::pair<uint32_t, uint32_t> gate_prog[3] = {};             // (off, len) into d_prog, by class
+    std::vector<uint32_t> gate_exp;                   // gate i enters the accumulator of its class with weight y^gate_exp[i]
+    fe_t* d_wts = nullptr;                            // those weights for the current proof (ExprArgs::wts)
+    fe_t* h_wts = nullptr;                            // their pinned staging buffer
     std::vector<std::pair<uint32_t, uint32_t>> lookup_prog;     // (off, len) into d_prog
     fe_t* d_consts = nullptr;
     int32_t *d_q_adv = nullptr, *d_q_fix = nullptr, *d_q_inst = nullptr;
@@ -195,7 +203,7 @@ static size_t arena_need(const b200zk_pk* pk) {
     size_t draws = b200zk_pk_rng_draws(pk);
     size_t elems = 2 * A * n + 2 * I * n + draws + 7 * L * n + S * n + S * ext + 3 * n   // columns, lookups, perm, tmp
                    + ext * (1 + A + I + 4 + 1)                                            // h, cosets, lookup cosets + table_value, h_L
-                   + n * (1 + 8 + 4 + 8);                                                 // h_poly, shplonk set sums, hx/lx/tmp, per-set quotients (sharded)
+                   + n * (1 + 8 + 4 + 8 + 1);                                                 // h_poly, shplonk set sums, hx/lx/tmp, per-set quotients (sharded), linear gates
     if (pk->lk_early) elems += 4 * L * (size_t)pk->lk_cosets_n * n + 64;
     return elems * sizeof(fe_t) + (size_t)draws * 64 + (64 << 10);
 }
@@ -329,121 +337,9 @@ static ExprArgs expr_args(const b200zk_pk* pk, uint32_t prog_off, uint32_t prog_
     a.rows = extended ? pk->ext_n : pk->n;
     a.rot_scale = 1u;
     for (int i = 0; i < 4; ++i) a.factors[i] = to_dev(ch[i]);
-    { HFr yp = HFr::one(); for (int i = 0; i < 9; ++i) { a.ypow[i] = to_dev(yp); yp = yp * ch[EXF_Y]; } }
+    a.wts = pk->d_wts;
     a.mode = mode; a.out0 = out0; a.out1 = out1;
     return a;
-}
-
-// ------------------------------------------------------------------ common sub-expressions
-// One evaluator program = a list of expressions (postfix ranges of cs.prog), each followed by a
-// FOLD word.  The trees are hash-consed (ADD / MUL operands unordered); a node that the emission
-// reaches more than once and that contains at least one multiplication is computed once and kept
-// in a TEE/TMP slot (expr.cuh).  When more than EX_TMPS nodes qualify, those saving the most
-// multiplications win.
-struct ExFold { uint32_t off, len, fold_word; };
-
-static bool ex_share_common(const std::vector<uint32_t>& src, const std::vector<ExFold>& items, std::vector<uint32_t>& out,
-                            bool group_common_factor = false) {
-    struct Node { uint32_t op, arg; int l, r; uint32_t muls; };
-    std::vector<Node> nodes;
-    std::map<std::array<int64_t, 4>, int> intern;
-    auto make = [&](uint32_t op, uint32_t arg, int l, int r) {
-        int a = l, b = r;
-        if ((op == EX_ADD || op == EX_MUL) && a > b) std::swap(a, b);
-        std::array<int64_t, 4> key{(int64_t)op, (int64_t)arg, a, b};
-        auto it = intern.find(key);
-        if (it != intern.end()) return it->second;
-        uint32_t muls = (op == EX_MUL || op == EX_SCALE ? 1u : 0u) + (l >= 0 ? nodes[l].muls : 0u) + (r >= 0 ? nodes[r].muls : 0u);
-        nodes.push_back({op, arg, l, r, muls});
-        intern[key] = (int)nodes.size() - 1;
-        return (int)nodes.size() - 1;
-    };
-    std::vector<int> roots;
-    for (auto& it : items) {
-        std::vector<int> st;
-        for (uint32_t i = it.off; i < it.off + it.len; ++i) {
-            uint32_t op = src[i] & 0xff, arg = src[i] >> 8;
-            if (op <= EX_INSTANCE) st.push_back(make(op, arg, -1, -1));
-            else if (op == EX_NEG || op == EX_SCALE) { if (st.empty()) return false; st.back() = make(op, arg, st.back(), -1); }
-            else if (op == EX_ADD || op == EX_MUL) {
-                if (st.size() < 2) return false;
-                int r = st.back(); st.pop_back();
-                st.back() = make(op, 0, st.back(), r);
-            } else return false;
-        }
-        if (st.size() != 1) return false;
-        roots.push_back(st[0]);
-    }
-    // how often the emission asks for each node when shared nodes are expanded once
-    std::vector<uint32_t> req(nodes.size(), 0);
-    std::vector<int> work;
-    for (int root : roots) {
-        work.push_back(root);
-        while (!work.empty()) {
-            int id = work.back(); work.pop_back();
-            if (++req[id] == 1) { if (nodes[id].l >= 0) work.push_back(nodes[id].l); if (nodes[id].r >= 0) work.push_back(nodes[id].r); }
-        }
-    }
-    std::vector<int> cand;
-    for (size_t id = 0; id < nodes.size(); ++id) if (req[id] >= 2 && nodes[id].muls >= 1) cand.push_back((int)id);
-    std::sort(cand.begin(), cand.end(), [&](int a, int b) {
-        uint64_t sa = (uint64_t)(req[a] - 1) * nodes[a].muls, sb = (uint64_t)(req[b] - 1) * nodes[b].muls;
-        return sa != sb ? sa > sb : a < b;
-    });
-    if (cand.size() > (size_t)EX_TMPS) cand.resize(EX_TMPS);
-    std::vector<int> slot(nodes.size(), -1);
-    for (size_t i = 0; i < cand.size(); ++i) slot[cand[i]] = (int)i;
-    std::vector<char> done(nodes.size(), 0);
-    // iterative postfix emission: (node, phase)
-    auto emit = [&](int root) {
-        std::vector<std::pair<int, int>> stk{{root, 0}};
-        while (!stk.empty()) {
-            auto [id, phase] = stk.back(); stk.pop_back();
-            const Node& nd = nodes[id];
-            if (phase == 0) {
-                if (slot[id] >= 0 && done[id]) { out.push_back(EX_TMP | ((uint32_t)slot[id] << 8)); continue; }
-                stk.push_back({id, 1});
-                if (nd.r >= 0) stk.push_back({nd.r, 0});
-                if (nd.l >= 0) stk.push_back({nd.l, 0});
-            } else {
-                out.push_back(nd.op | (nd.arg << 8));
-                if (slot[id] >= 0) { out.push_back(EX_TEE | ((uint32_t)slot[id] << 8)); done[id] = 1; }
-            }
-        }
-    };
-    // common factor of two product roots (-1 if none)
-    auto common = [&](int a, int b) {
-        if (nodes[a].op != EX_MUL || nodes[b].op != EX_MUL) return -1;
-        for (int x : {nodes[a].l, nodes[a].r}) if (x == nodes[b].l || x == nodes[b].r) return x;
-        return -1;
-    };
-    for (size_t k = 0; k < roots.size();) {
-        size_t m = 1;
-        int f = -1;
-        if (group_common_factor && k + 1 < roots.size()) {
-            f = common(roots[k], roots[k + 1]);
-            if (f >= 0) {
-                m = 2;
-                while (k + m < roots.size() && m < 8 && nodes[roots[k + m]].op == EX_MUL &&
-                       (nodes[roots[k + m]].l == f || nodes[roots[k + m]].r == f)) ++m;
-            }
-        }
-        if (f < 0) {
-            emit(roots[k]);
-            out.push_back(items[k].fold_word);
-            ++k;
-            continue;
-        }
-        for (size_t j = 0; j < m; ++j) {                        // cofactors into acc1 by Horner in y
-            const Node& nd = nodes[roots[k + j]];
-            emit(nd.l == f ? nd.r : nd.l);
-            out.push_back(j == 0 ? (uint32_t)EX_SET1 : (EX_FOLD | ((1u << 4 | EXF_Y) << 8)));
-        }
-        emit(f);
-        out.push_back(EX_GROUP | ((uint32_t)m << 8));
-        k += m;
-    }
-    return true;
 }
 
 // ------------------------------------------------------------------ one proof over several ranks
@@ -602,15 +498,16 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
     fe_t* advice_cosets = ar.take<fe_t>(A * ext);
     fe_t* inst_cosets = ar.take<fe_t>(I * ext);
     fe_t* lk_cosets = ar.take<fe_t>(4 * ext);                    // z, a', s', table_value
-    fe_t* h_lk = ar.take<fe_t>(ext);                             // lookup part of the quotient when it runs on fewer cosets
-    const uint32_t CL = pk->lk_cosets_n;
-    const bool lk_split = L && CL < pk->q;
-    const size_t lk_span = (size_t)(lk_split ? CL : pk->q) * n;  // rows of one lookup coset array
+    fe_t* h_lk = ar.take<fe_t>(ext);                             // lookup and low-degree gate part of the quotient when it runs on fewer cosets
+    fe_t* h_lin = ar.take<fe_t>(n);                              // linear gates on coset 0
+    const uint32_t CL = pk->lk_cosets_n;                         // == q unless the lookup terms and the low gates run on fewer cosets
+    const bool lk_split = CL < pk->q;
+    const size_t lk_span = (size_t)CL * n;                       // rows of one lookup coset array
     fe_t* lk_all = pk->lk_early ? ar.take<fe_t>(4 * (size_t)L * lk_span) : nullptr;
     // arrays of lookup l: product z, permuted input a', permuted table s', table value (all indexed by global coset row)
     auto LKC = [&](uint32_t l, uint32_t which) { return pk->lk_early ? lk_all + ((size_t)l * 4 + which) * lk_span : lk_cosets + (size_t)which * ext; };
     // this rank's share of the cosets the lookup terms run on
-    const uint32_t lj0 = std::min(cj0, lk_split ? CL : pk->q), lj1 = std::min(cj1, lk_split ? CL : pk->q);
+    const uint32_t lj0 = std::min(cj0, CL), lj1 = std::min(cj1, CL);
     const uint32_t lk_row0 = lj0 * (uint32_t)n, lk_rows = (lj1 - lj0) * (uint32_t)n;
     auto lookup_table_value = [&](uint32_t l, const HFr* chv) {  // (compressed input + beta)(compressed table + gamma) on this rank's lookup cosets
         PhaseTimer t(pk, PH_QUOT);
@@ -745,9 +642,10 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
                 ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys + (size_t)c * n, advice_values + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
                 ZK_TRY(lagrange_to_coeff(pk, advice_polys + (size_t)c * n));
             }
-            ZK_TRY(my_cosets(advice_polys + (size_t)c * n, advice_cosets + (size_t)c * ext, cj0, cj1));
+            ZK_TRY(my_cosets(advice_polys + (size_t)c * n, advice_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.adv_need[c])));
         }
-        for (uint32_t c = 0; c < I; ++c) ZK_TRY(my_cosets(inst_polys + (size_t)c * n, inst_cosets + (size_t)c * ext, cj0, cj1));
+        // only the cosets a consumer reads (QuotPlan::adv_need / inst_need): the higher ones are never written
+        for (uint32_t c = 0; c < I; ++c) ZK_TRY(my_cosets(inst_polys + (size_t)c * n, inst_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.inst_need[c])));
     }
     if (random_early && !split_upload) ZK_TRY(commit_random());
     if (A && !split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[A - 1], 0));
@@ -946,6 +844,14 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
     tr.write_point(random_pt);
     ch[EXF_Y] = tr.squeeze_challenge();
     const HFr y = ch[EXF_Y];
+    if (!pk->gate_exp.empty()) {                                  // the gates' powers of y (ExprArgs::wts)
+        std::vector<HFr> ypow(1, HFr::one());
+        for (uint32_t i = 0; i < cs.gates.size(); ++i) {
+            while (ypow.size() <= pk->gate_exp[i]) ypow.push_back(ypow.back() * y);
+            ((fe_t*)pk->h_wts)[i] = to_dev(ypow[pk->gate_exp[i]]);
+        }
+        ZK_CUDA(ctx, cudaMemcpyAsync(pk->d_wts, pk->h_wts, cs.gates.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
+    }
 
     // ---- step 10: advice / instance cosets were started on the side stream after the advice commitments
     ZK_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_join, 0));
@@ -953,16 +859,25 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
     // ---- step 11: evaluate_h
     // this rank's rows of the quotient: its cosets [cj0, cj1) (all of them on a single GPU)
     const uint32_t my_row0 = cj0 * (uint32_t)n, my_rows = (cj1 - cj0) * (uint32_t)n;
-    if (my_rows) {
+    // one gate program per class, each on its own rows (quot_plan.hpp); a class without gates starts its accumulator at 0
+    auto gate_class = [&](uint32_t cls, fe_t* out, uint32_t row0, uint32_t rows) -> int32_t {
+        if (!rows) return B200ZK_OK;
         PhaseTimer t(pk, PH_QUOT);
-        if (pk->gates_len) {
-            ExprArgs ea = expr_args(pk, 0, pk->gates_len, true, EXM_ACC0, ch, h, nullptr);
-            ea.row0 = my_row0; ea.rows = my_rows;
-            expr_kernel<<<nb(my_rows), PK_THREADS, 0, st>>>(ea);
-            ctx->launches++;
-        } else {
-            ZK_CUDA(ctx, cudaMemsetAsync(h + my_row0, 0, (size_t)my_rows * sizeof(fe_t), st));
+        if (!pk->gate_prog[cls].second) {
+            ZK_CUDA(ctx, cudaMemsetAsync(out + row0, 0, (size_t)rows * sizeof(fe_t), st));
+            return B200ZK_OK;
         }
+        ExprArgs ea = expr_args(pk, pk->gate_prog[cls].first, pk->gate_prog[cls].second, true, EXM_ACC0, ch, out, nullptr);
+        ea.row0 = row0; ea.rows = rows;
+        expr_kernel<<<nb(rows), PK_THREADS, 0, st>>>(ea);
+        ctx->launches++;
+        return B200ZK_OK;
+    };
+    const bool lin_mine = pk->gate_prog[QC_LINEAR].second && sh.coset_owner(0) == sh.R;
+    if (lin_mine) ZK_TRY(gate_class(QC_LINEAR, h_lin, 0, (uint32_t)n));
+    if (my_rows) {
+        ZK_TRY(gate_class(QC_MAIN, h, my_row0, my_rows));
+        PhaseTimer t(pk, PH_QUOT);
         if (S) {
             QuotPermAArgs qa{};
             qa.h = h; qa.y = to_dev(y); qa.l0 = pk->l0; qa.l_last = pk->l_last; qa.nsets = S;
@@ -990,7 +905,7 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
     }
     // lookup terms: on all q cosets straight into h, or — when their degree allows — on the first CL cosets into
     // h_lk, extended to the other cosets after the per-coset iNTT (lookup_extrapolate_row)
-    if (lk_split && lk_rows) ZK_CUDA(ctx, cudaMemsetAsync(h_lk + lk_row0, 0, (size_t)lk_rows * sizeof(fe_t), st));
+    if (lk_split) ZK_TRY(gate_class(QC_LOW, h_lk, lk_row0, lk_rows));
     for (uint32_t l = 0; l < L && lk_rows; ++l) {
         fe_t *zc = LKC(l, 0), *ac = LKC(l, 1), *sc = LKC(l, 2), *tv = LKC(l, 3);
         if (!pk->lk_early) {
@@ -1017,9 +932,10 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
         PhaseTimer t(pk, PH_NTT);
         HFr y_lk = HFr::one();                                    // h = h_gates_perm * y^(5 L) + h_lk
         if (lk_split) {
-            for (uint32_t i = 0; i < 5 * L; ++i) y_lk = y_lk * y;
-            for (uint32_t j = lj0; j < lj1; ++j) {
-                HFr post[3] = {dom->ifft_divisor, dom->ifft_divisor, dom->ifft_divisor};
+            for (uint32_t i = 0; i < 5 * L; ++i) y_lk = y_lk * y;       // (the low gates' weights leave this factor to the lookup kernels)
+            for (uint32_t j = lj0; j < lj1; ++j) {                     // divided by the vanishing polynomial before the extrapolation
+                HFr f = dom->ifft_divisor * pk->coset_t[j];
+                HFr post[3] = {f, f, f};
                 ZK_TRY(ntt_run(ctx, h_lk + j * n, (uint32_t)n, h_lk + j * n, dom->k, dom->omega_inv, nullptr, post));
             }
         }
@@ -1028,17 +944,24 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
             HFr post[3] = {f, f, f};
             ZK_TRY(ntt_run(ctx, h + j * n, (uint32_t)n, h + j * n, dom->k, dom->omega_inv, nullptr, post));
         }
+        if (lin_mine) {                                           // the linear gates' part of h, degree < n: coefficients in X / c_0
+            HFr f = dom->ifft_divisor * pk->coset_t[0];
+            HFr post[3] = {f, f, f};
+            ZK_TRY(ntt_run(ctx, h_lin, (uint32_t)n, h_lin, dom->k, dom->omega_inv, nullptr, post));
+        }
         if (sh.on()) {                                            // every coset's coefficients to every rank: q (+ CL) x n elements
             std::vector<CommPiece> pieces;
             for (uint32_t j = 0; j < pk->q; ++j) pieces.push_back({h + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
             if (lk_split) for (uint32_t j = 0; j < CL; ++j) pieces.push_back({h_lk + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
+            if (pk->gate_prog[QC_LINEAR].second) pieces.push_back({h_lin, n * sizeof(fe_t), sh.coset_owner(0)});
             ZK_TRY(sh.cm->share(ctx, pieces.data(), pieces.size(), st));
         }
         if (lk_split) {
-            lookup_extrapolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h_lk, pk->coset_pow_inv, pk->lk_lambda, pk->coset_t_dev, CL, pk->q, n);
+            lookup_extrapolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h_lk, pk->coset_pow_inv, pk->lk_lambda, nullptr, CL, pk->q, n);
             ctx->launches++;
         }
-        coset_interpolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h, pk->coset_pow_inv, pk->vinv, pk->q, n, lk_cosets, lk_split ? h_lk : nullptr);
+        coset_interpolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h, pk->coset_pow_inv, pk->vinv, pk->q, n, lk_cosets, lk_split ? h_lk : nullptr,
+                                                                 pk->gate_prog[QC_LINEAR].second ? h_lin : nullptr);
         ctx->launches++;
         ZK_CUDA(ctx, cudaGetLastError());
         h = lk_cosets;                                            // q pieces of n coefficients
@@ -1338,27 +1261,22 @@ int32_t b200zk_pk_debug_buffer(b200zk_pk* pk, const char* name, void* host_out, 
     return B200ZK_OK;
 }
 
-// Field multiplications evaluate_h executes per row, as launched: out[0] custom gates (one row of every quotient coset),
-// out[1] permutation terms (same rows), out[2] all lookups together (rows of the lk_cosets_n cosets the lookup terms run
-// on), out[3] = q, out[4] = lk_cosets_n.  bench.py's roofline_quotient: work = n * (q * (gates + perm) + CL * lookups).
+// Field multiplications evaluate_h executes per row, as launched: out[0] custom gates, out[1] permutation terms (one row of
+// every quotient coset), out[2] all lookups together (rows of the lk_cosets_n cosets the lookup terms run on), out[3] = q,
+// out[4] = lk_cosets_n.  bench.py's roofline_quotient: work = n * (q * (gates + perm) + CL * lookups).  The gates run as
+// three programs on q, lk_cosets_n and 1 cosets (quot_plan.hpp), so out[0] is their coset-weighted total divided by q,
+// rounded: q * out[0] is the gate work launched per row of one coset.
 int32_t b200zk_pk_quotient_muls(const b200zk_pk* pk, uint32_t out5[5]) {
     if (!pk || !out5) return B200ZK_EINVAL;
-    std::vector<uint32_t> prog(pk->gates_len + 1);
     // the programs live on the device; count from a host copy
-    uint32_t total = pk->gates_len;
+    uint32_t total = 0;
+    for (auto& gp : pk->gate_prog) total = std::max(total, gp.first + gp.second);
     for (auto& lp : pk->lookup_prog) total = std::max(total, lp.first + lp.second);
-    prog.resize(total);
+    std::vector<uint32_t> prog(total);
     if (total && cudaMemcpy(prog.data(), pk->d_prog, total * 4, cudaMemcpyDeviceToHost) != cudaSuccess) return B200ZK_ECUDA;
-    auto count = [&](uint32_t off, uint32_t len) {
-        uint32_t m = 0;
-        for (uint32_t i = off; i < off + len; ++i) {
-            uint32_t op = prog[i] & 0xff;
-            if (op == EX_MUL || op == EX_SCALE || op == EX_FOLD) m += 1;
-            else if (op == EX_GROUP) m += 2;
-        }
-        return m;
-    };
-    out5[0] = count(0, pk->gates_len);
+    uint64_t gate_work = 0;
+    for (uint32_t c = 0; c < 3; ++c) gate_work += (uint64_t)pk->plan.cosets(c) * ex_program_muls(prog.data() + pk->gate_prog[c].first, pk->gate_prog[c].second);
+    out5[0] = (uint32_t)((gate_work + pk->q / 2) / pk->q);
     uint32_t perm = 0;
     if (pk->S) {
         perm = 5 + 2 * (pk->S - 1);
@@ -1366,7 +1284,7 @@ int32_t b200zk_pk_quotient_muls(const b200zk_pk* pk, uint32_t out5[5]) {
     }
     out5[1] = perm;
     uint32_t lk = 0;
-    for (auto& lp : pk->lookup_prog) lk += count(lp.first, lp.second) + 1 + 13;       // table value product + quot_lookup_row
+    for (auto& lp : pk->lookup_prog) lk += ex_program_muls(prog.data() + lp.first, lp.second) + 1 + 13;       // table value product + quot_lookup_row
     out5[2] = lk; out5[3] = pk->q; out5[4] = pk->lk_cosets_n;
     return B200ZK_OK;
 }
@@ -1413,6 +1331,7 @@ void b200zk_pk_destroy(b200zk_pk* pk) {
     cudaSetDevice(pk->ctx->device);
     if (pk->copy_stream) { cudaStreamSynchronize(pk->copy_stream); cudaStreamDestroy(pk->copy_stream); }
     if (pk->ev_rnd) cudaEventDestroy(pk->ev_rnd);
+    if (pk->h_wts) cudaFreeHost(pk->h_wts);
     for (cudaEvent_t e : pk->col_events) cudaEventDestroy(e);
     cudaStreamSynchronize(pk->ctx->stream);
     for (void* p : pk->owned) cudaFree(p);
@@ -1494,31 +1413,18 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
         for (uint32_t t = 0; t < C; ++t) for (uint32_t j = 0; j < C; ++j) vin[(size_t)t * C + j] = to_dev(m[t][C + j]);
         PK_CUDA(cudaMemcpyAsync(pk->coset_fac, fac.data(), C * sizeof(fe_t), cudaMemcpyHostToDevice, st));
         PK_CUDA(cudaMemcpyAsync(pk->vinv, vin.data(), vin.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
-        // cosets the lookup terms need: their degree is < (2 + deg input + deg table) * n  (circuit.rs, lookup
-        // Argument::required_degree without the max(4, .) floor being relevant: it is >= 4 already)
-        uint32_t CL = C;
-        if (!cs.lookups.empty()) {
-            uint32_t need = 0;
-            for (auto& lk : cs.lookups) {
-                uint32_t di = 1, dt = 1;
-                for (auto& e : lk.ins) di = std::max(di, expr_degree(cs, e.first, e.second));
-                for (auto& e : lk.tabs) dt = std::max(dt, expr_degree(cs, e.first, e.second));
-                need = std::max(need, 2 + di + dt);
-            }
-            CL = std::min(C, need);
-        }
+        pk->plan = quot_plan(cs, C, lookup_cosets(cs, C));
+        const uint32_t CL = pk->plan.low;
         pk->lk_cosets_n = CL;
-        std::vector<fe_t> lam((size_t)std::max<uint32_t>(C - CL, 1) * CL), tdev(C);
-        for (uint32_t j = 0; j < C; ++j) tdev[j] = to_dev(pk->coset_t[j]);
+        std::vector<fe_t> lam((size_t)std::max<uint32_t>(C - CL, 1) * CL);
         for (uint32_t jp = CL; jp < C; ++jp)
             for (uint32_t j = 0; j < CL; ++j) {
                 HFr num = HFr::one(), den = HFr::one();
                 for (uint32_t m2 = 0; m2 < CL; ++m2) { if (m2 == j) continue; num = num * (y[jp] - y[m2]); den = den * (y[j] - y[m2]); }
                 lam[(size_t)(jp - CL) * CL + j] = to_dev(num * den.inv());
             }
-        PK_TRY(dev_alloc(pk, &pk->lk_lambda, lam.size())); PK_TRY(dev_alloc(pk, &pk->coset_t_dev, C));
+        PK_TRY(dev_alloc(pk, &pk->lk_lambda, lam.size()));
         PK_CUDA(cudaMemcpyAsync(pk->lk_lambda, lam.data(), lam.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
-        PK_CUDA(cudaMemcpyAsync(pk->coset_t_dev, tdev.data(), C * sizeof(fe_t), cudaMemcpyHostToDevice, st));
         PK_CUDA(cudaStreamSynchronize(st));
     }
     // fixed columns
@@ -1564,15 +1470,30 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
         one_minus_sum_kernel<<<nb(ext), PK_THREADS, 0, st>>>(pk->l_last, lb, pk->l_active, ext);
         ctx->launches++;
     }
-    // programs: gates with FOLD(acc0, y); lookups with FOLD(acc0/acc1, theta)
+    // programs: gates of each class with WSUM(acc0, gate); lookups with FOLD(acc0/acc1, theta)
     {
         std::vector<uint32_t> prog;
-        {
-            std::vector<ExFold> items;
-            for (auto& g : cs.gates) items.push_back({g.first, g.second, EX_FOLD | ((0u << 4 | EXF_Y) << 8)});
-            if (!ex_share_common(cs.prog, items, prog, true)) return bail(fail(ctx, B200ZK_EINVAL, "pk_create", "malformed expression program"));
+        // the gates, then the permutation terms (2 S + 1), then the lookup terms (5 L) fold in y in evaluate_h: gate i has
+        // weight y^(G - 1 - i + 2 S + 1 + 5 L) in h.  The main class is multiplied by y^(2 S + 1) in the permutation kernels
+        // and by y^(5 L) in the iNTT (or the lookup kernels when they share its cosets), the low class by y^(5 L) in the
+        // lookup kernels; the linear class is added as it is.
+        const uint32_t G = (uint32_t)cs.gates.size(), perm_terms = pk->S ? 2 * pk->S + 1 : 0;
+        if (G >= EXW_INDEX) return bail(fail(ctx, B200ZK_EINVAL, "pk_create", "too many gate polynomials for this build"));
+        for (uint32_t i = 0; i < G; ++i) {
+            const uint32_t cls = pk->plan.gate_class[i];
+            pk->gate_exp.push_back(G - 1 - i + (cls == QC_MAIN ? 0 : perm_terms) + (cls == QC_LINEAR ? 5 * pk->L : 0));
         }
-        pk->gates_len = (uint32_t)prog.size();
+        for (uint32_t cls = 0; cls < 3; ++cls) {
+            std::vector<ExFold> items;
+            for (uint32_t i = 0; i < G; ++i) if (pk->plan.gate_class[i] == cls) items.push_back({cs.gates[i].first, cs.gates[i].second, EX_WSUM | ((EXW_ACC0 | i) << 8)});
+            const uint32_t off = (uint32_t)prog.size();
+            if (!ex_share_common(cs.prog, items, prog, true)) return bail(fail(ctx, B200ZK_EINVAL, "pk_create", "malformed expression program"));
+            pk->gate_prog[cls] = {off, (uint32_t)prog.size() - off};
+        }
+        if (G) {
+            PK_TRY(dev_alloc(pk, &pk->d_wts, G));
+            PK_CUDA(cudaMallocHost((void**)&pk->h_wts, G * sizeof(fe_t)));
+        }
         for (auto& lk : cs.lookups) {
             uint32_t off = (uint32_t)prog.size();
             std::vector<ExFold> items;
@@ -1585,7 +1506,7 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
         int depth = 0, maxd = 0;
         for (uint32_t w : prog) {
             uint32_t op = w & 0xff;
-            if (op <= EX_INSTANCE || op == EX_TMP) ++depth; else if (op == EX_ADD || op == EX_MUL || op == EX_FOLD || op == EX_SET1 || op == EX_GROUP) --depth;
+            if (op <= EX_INSTANCE || op == EX_TMP) ++depth; else if (op == EX_ADD || op == EX_MUL || op == EX_FOLD || op == EX_WSUM || op == EX_GROUP) --depth;
             maxd = std::max(maxd, depth);
             if (depth < 0) return bail(fail(ctx, B200ZK_EINVAL, "pk_create", "malformed expression program"));
         }

@@ -171,8 +171,10 @@ ZK_D void quot_lookup_row(const QuotLookupArgs& q, uint32_t idx) {
 // inverse Vandermonde matrix of the points c_j^n:   out[t*n + r] = sum_j vinv[t*C + j] * H_r(c_j^n).
 // `extra` (optional): a second summand already in H-space, extra[j*n + r] = H'_r(c_j^n) — the lookup part of the
 // quotient when it was evaluated on fewer cosets (lookup_extrapolate_row).
+// `lin` (optional): a part of h of degree < n, lin[r] = its r-th coefficient in Y = X / c_0 (the per-coset iNTT of coset 0);
+// it adds lin[r] * c_0^(-r) to piece 0.
 ZK_D void coset_interpolate_row(const fe_t* g, const fe_t* inv_pow, const fe_t* vinv, uint32_t C, size_t n, fe_t* out, size_t r,
-                                const fe_t* extra = nullptr) {
+                                const fe_t* extra = nullptr, const fe_t* lin = nullptr) {
     fe_t v[ZK_MAXCOSETS];
     for (uint32_t j = 0; j < C; ++j) {
         fe_t x = g[(size_t)j * n + r], w = inv_pow[(size_t)j * n + r];
@@ -182,27 +184,30 @@ ZK_D void coset_interpolate_row(const fe_t* g, const fe_t* inv_pow, const fe_t* 
     for (uint32_t t = 0; t < C; ++t) {
         fe_t acc = Fr::mul(v[0], vinv[t * C]);
         for (uint32_t j = 1; j < C; ++j) acc = Fr::add(acc, Fr::mul(v[j], vinv[t * C + j]));
+        if (t == 0 && lin) acc = Fr::add(acc, Fr::mul(lin[r], inv_pow[r]));
         out[(size_t)t * n + r] = acc;
     }
 }
 
-// ---- lookup terms on fewer cosets ----
+// ---- lookup terms and low-degree gates on fewer cosets ----
 // The lookup terms of evaluate_h have degree < CL * n with CL = 2 + deg(input) + deg(table) (4 for a plain column
-// lookup) while the gates need all C = d - 1 cosets.  Their sum h_L is therefore evaluated on the first CL cosets
-// only — the three coset extensions per lookup and the two lookup kernels shrink by CL / C — and carried to the
-// other cosets in H-space: with h_L(X) = sum_r X^r H_r(X^n), deg H_r < CL, the per-coset iNTT gives
-// g[j][r] = c_j^r H_r(y_j) (y_j = c_j^n) for j < CL, and H_r(y_j') for j' >= CL is the Lagrange extrapolation
-// sum_j lambda[j' - CL][j] H_r(y_j).  Output (in place, C * n elements): H_r(y_j) / (y_j - 1) for every coset j,
-// the summand coset_interpolate_row adds to the gate / permutation part.
+// lookup) while the gates of the highest degree need all C = d - 1 cosets; gates of degree <= CL + 1 join them
+// (quot_plan.hpp).  Their sum h_L is therefore evaluated on the first CL cosets only — the three coset extensions per
+// lookup and the two lookup kernels shrink by CL / C — and carried to the other cosets in H-space: with
+// h_L(X) = sum_r X^r H_r(X^n), deg H_r < CL, the per-coset iNTT gives g[j][r] = c_j^r H_r(y_j) (y_j = c_j^n) for j < CL,
+// and H_r(y_j') for j' >= CL is the Lagrange extrapolation sum_j lambda[j' - CL][j] H_r(y_j).  Output (in place, C * n
+// elements): H_r(y_j) * tinv[j] for every coset j (tinv null: 1), the summand coset_interpolate_row adds to the gate /
+// permutation part.  The prover divides by the vanishing polynomial in the iNTT already (tinv null): the numerator of a
+// gate of degree CL + 1 has degree CL * n + n - CL - 1, more than CL cosets determine, its quotient has degree < CL * n.
 ZK_D void lookup_extrapolate_row(fe_t* g, const fe_t* inv_pow, const fe_t* lambda, const fe_t* tinv, uint32_t CL, uint32_t C, size_t n, size_t r) {
     fe_t u[ZK_MAXCOSETS];
     for (uint32_t j = 0; j < CL; ++j) { fe_t x = g[(size_t)j * n + r], w = inv_pow[(size_t)j * n + r]; u[j] = Fr::mul(x, w); }
     for (uint32_t jp = CL; jp < C; ++jp) {
         fe_t acc = Fr::mul(u[0], lambda[(jp - CL) * CL]);
         for (uint32_t j = 1; j < CL; ++j) acc = Fr::add(acc, Fr::mul(u[j], lambda[(jp - CL) * CL + j]));
-        g[(size_t)jp * n + r] = Fr::mul(acc, tinv[jp]);
+        g[(size_t)jp * n + r] = tinv ? Fr::mul(acc, tinv[jp]) : acc;
     }
-    for (uint32_t j = 0; j < CL; ++j) g[(size_t)j * n + r] = Fr::mul(u[j], tinv[j]);
+    for (uint32_t j = 0; j < CL; ++j) g[(size_t)j * n + r] = tinv ? Fr::mul(u[j], tinv[j]) : u[j];
 }
 
 // ---- vanishing::evaluate: h_poly = sum_j (x^n)^j piece_j  (pieces contiguous, n apart) ----
