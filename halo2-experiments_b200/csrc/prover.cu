@@ -13,9 +13,7 @@
 #include "quot_plan.hpp"
 #include "transcript.hpp"
 #include <algorithm>
-#include <array>
 #include <map>
-#include <memory>
 #include <new>
 #include <set>
 #include <chrono>
@@ -198,9 +196,32 @@ struct Arena {
     }
 };
 
+// Where create_proof reads the caller's rng stream: one 64-byte draw per Fr::random of upstream create_proof, in its call
+// order (SURVEY.md §8(a7)).  Upstream also draws a Blind for every commitment, which KZG does not use: those draws are
+// gaps, drawn by the caller and never read.
+struct DrawLayout {
+    size_t bf1, advice, advice_blinds, lookups, sets, lk_products, random, random_blind, h_blinds, total;
+    explicit DrawLayout(const b200zk_pk* pk) : bf1(pk->cs.bf + 1) {
+        advice = 0;                                        // bf + 1 blinding rows per advice column
+        advice_blinds = advice + pk->cs.A * bf1;           // gap: a Blind per advice column
+        lookups = advice_blinds + pk->cs.A;                // per lookup: bf + 1 rows of the permuted input, bf + 1 of the permuted table, 2 Blinds (gap)
+        sets = lookups + pk->L * (2 * bf1 + 2);            // per permutation set: bf blinding rows of its product, a Blind (gap)
+        lk_products = sets + pk->S * bf1;                  // per lookup: bf blinding rows of its product, a Blind (gap)
+        random = lk_products + pk->L * bf1;                // the n coefficients of the vanishing argument's random polynomial
+        random_blind = random + pk->n;                     // gap
+        h_blinds = random_blind + 1;                       // gap: a Blind per piece of h
+        total = h_blinds + pk->q;
+    }
+    size_t advice_rows(uint32_t c) const { return advice + c * bf1; }
+    size_t lookup_input_rows(uint32_t l) const { return lookups + l * (2 * bf1 + 2); }
+    size_t lookup_table_rows(uint32_t l) const { return lookup_input_rows(l) + bf1; }
+    size_t set_rows(uint32_t s) const { return sets + s * bf1; }
+    size_t lookup_product_rows(uint32_t l) const { return lk_products + l * bf1; }
+};
+
 static size_t arena_need(const b200zk_pk* pk) {
     size_t n = pk->n, ext = pk->ext_n, A = pk->cs.A, I = pk->cs.I, L = pk->L, S = pk->S;
-    size_t draws = b200zk_pk_rng_draws(pk);
+    size_t draws = DrawLayout(pk).total;
     size_t elems = 2 * A * n + 2 * I * n + draws + 7 * L * n + S * n + S * ext + 3 * n   // columns, lookups, perm, tmp
                    + ext * (1 + A + I + 4 + 1)                                            // h, cosets, lookup cosets + table_value, h_L
                    + n * (1 + 8 + 4 + 8 + 1);                                                 // h_poly, shplonk set sums, hx/lx/tmp, per-set quotients (sharded), linear gates
@@ -298,20 +319,18 @@ static int32_t commit_multi_dev(b200zk_pk* pk, const std::vector<const fe_t*>& c
     }
     return B200ZK_OK;
 }
-// `count` contiguous Lagrange columns to coefficient form in one launch per pass
-static int32_t lagrange_to_coeff_batch(b200zk_pk* pk, fe_t* d_a, uint32_t count) {
-    PhaseTimer t(pk, PH_NTT);
-    HFr post[3] = {pk->dom->ifft_divisor, pk->dom->ifft_divisor, pk->dom->ifft_divisor};
-    pk->ctx->ntt_sparse_hint = true;
-    int32_t rc = ntt_rows_run(pk->ctx, d_a, count, pk->dom->omega_inv, pk->dom->k, post);
-    pk->ctx->ntt_sparse_hint = false;
-    return rc;
+// inverse NTT of `count` contiguous size-n columns in place, every output multiplied by `factor`; more than one column
+// runs as one launch per pass
+static int32_t intt_scaled(b200zk_pk* pk, fe_t* d_a, uint32_t count, const HFr& factor) {
+    HFr post[3] = {factor, factor, factor};
+    if (count == 1) return ntt_run(pk->ctx, d_a, pk->n, d_a, pk->dom->k, pk->dom->omega_inv, nullptr, post);
+    return ntt_rows_run(pk->ctx, d_a, count, pk->dom->omega_inv, pk->dom->k, post);
 }
-static int32_t lagrange_to_coeff(b200zk_pk* pk, fe_t* d_a) {
+// `count` contiguous Lagrange columns to coefficient form
+static int32_t lagrange_to_coeff(b200zk_pk* pk, fe_t* d_a, uint32_t count = 1) {
     PhaseTimer t(pk, PH_NTT);
-    HFr post[3] = {pk->dom->ifft_divisor, pk->dom->ifft_divisor, pk->dom->ifft_divisor};
     pk->ctx->ntt_sparse_hint = true;
-    int32_t rc = ntt_run(pk->ctx, d_a, pk->n, d_a, pk->dom->k, pk->dom->omega_inv, nullptr, post);
+    int32_t rc = intt_scaled(pk, d_a, count, pk->dom->ifft_divisor);
     pk->ctx->ntt_sparse_hint = false;
     return rc;
 }
@@ -319,9 +338,6 @@ static int32_t lagrange_to_coeff(b200zk_pk* pk, fe_t* d_a) {
 static int32_t coeff_to_extended(b200zk_pk* pk, const fe_t* d_coeffs, fe_t* d_out, uint32_t cosets = 0) {
     PhaseTimer t(pk, PH_NTT);
     return ntt_run_cosets(pk->ctx, d_coeffs, d_out, pk->dom->k, pk->dom->omega, pk->coset_pow, cosets ? cosets : pk->q);
-}
-static int32_t eval_dev(b200zk_pk* pk, const fe_t* d_poly, size_t len, const HFr& x, HFr* out) {
-    return recurrence_run(pk->ctx, d_poly, nullptr, len, x, out);
 }
 
 static ExprArgs expr_args(const b200zk_pk* pk, uint32_t prog_off, uint32_t prog_len, bool extended, uint32_t mode,
@@ -440,96 +456,155 @@ static int32_t commit_multi_range(b200zk_pk* pk, const Shard& sh, const std::vec
 }
 
 // ------------------------------------------------------------------ create_proof
-static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_device, const void* const* advice_host,
-                     const void* const* instance_columns, const uint32_t* instance_lens, const void* rng_wide, bool rng_on_device,
-                     const HFr& transcript_repr, std::vector<uint8_t>& proof_out) {
+// One create_proof on this rank: the state its steps (SURVEY.md §3.2) share.  prove() calls the steps in order and squeezes
+// the challenges between them.
+struct Prover {
+    b200zk_pk* pk;
     b200zk_ctx* ctx = pk->ctx;
     const CsDesc& cs = pk->cs;
     const b200zk_domain* dom = pk->dom;
     cudaStream_t st = ctx->stream;
-    for (uint32_t c = 0; c < cs.I; ++c) if (instance_lens[c] && !instance_columns[c]) return fail(ctx, B200ZK_EINVAL, "create_proof", "null instance column");
-    if (!advice_on_device) for (uint32_t c = 0; c < cs.A; ++c) if (!advice_host[c]) return fail(ctx, B200ZK_EINVAL, "create_proof", "null advice column");
-    cudaStreamSynchronize(ctx->stream2);                          // nothing of an earlier (failed) proof may still be writing the arena
-    if (pk->copy_stream) cudaStreamSynchronize(pk->copy_stream);
+    Shard sh{pk};
+    const DrawLayout dl{pk};
+    const bool advice_on_device;
+    // Sharded proof from host buffers: the host -> device traffic is split as well — every rank uploads 1/G of the rng
+    // stream and its own advice columns over its PCIe link, and the ranks exchange them over NVLink.
+    const bool split_upload;
     const size_t n = pk->n, ext = pk->ext_n;
     const uint32_t A = cs.A, I = cs.I, F = cs.F, L = pk->L, S = pk->S, bf = cs.bf;
     const size_t usable = n - (bf + 1);
-    const uint32_t rot_scale = 1u;                               // rotations stay inside a coset (prover_kernels.cuh)
-    for (float& f : pk->phase_ms) f = 0;
-    pk->timer_used = 0;
-    ZK_CUDA(ctx, cudaSetDevice(ctx->device));
-    Shard sh(pk);
-    sh.assign(pk->L, pk->S, pk->cs.A + pk->cs.I + pk->S + 3 * pk->L);
-    pk->trace.clear();
-    const auto t_start = std::chrono::steady_clock::now();
-    auto mark = [&](const char* label) {              // called right after a host synchronisation: where the wall clock of the proof goes
+    const uint32_t CL = pk->lk_cosets_n;                          // == q unless the lookup terms and the low gates run on fewer cosets
+    const bool lk_split = CL < pk->q;
+    const uint32_t cj0 = sh.coset_lo(sh.R), cj1 = sh.coset_lo(sh.R + 1);       // quotient cosets this rank extends and evaluates
+    const uint32_t lj0 = std::min(cj0, CL), lj1 = std::min(cj1, CL);           // this rank's share of the cosets the lookup terms run on
+    const uint32_t lk_row0 = lj0 * (uint32_t)n, lk_rows = (lj1 - lj0) * (uint32_t)n;
+    const std::chrono::steady_clock::time_point t_start = std::chrono::steady_clock::now();
+    host::Transcript tr;
+    HFr ch[4] = {HFr::zero(), HFr::zero(), HFr::zero(), HFr::zero()};   // theta, beta, gamma, y
+    HFr x;                                                        // the opening point
+    HAffine random_pt = {host::HFq::zero(), host::HFq::zero()};
+    // arena buffers, see carve
+    fe_t *advice_values, *advice_polys, *inst_values, *inst_polys, *rnd, *lk_bufs, *perm_polys, *perm_cosets, *tmp_n, *h;
+    fe_t *advice_cosets, *inst_cosets, *lk_cosets, *h_lk, *h_lin, *lk_all, *h_poly, *set_sums, *set_quot, *hx, *lx, *t0, *t1;
+    uint32_t* wide;
+    // openings: every (polynomial, point) pair in multiopen order, its distinct pairs and their values
+    struct Query { const fe_t* poly; HFr point; };
+    std::vector<Query> queries, pairs;
+    std::vector<HFr> values;
+    // SHPLONK's rotation sets, the low-degree equivalent of each of their polynomials, all points
+    struct RotSet { std::vector<HFr> pts; std::vector<const fe_t*> polys; };
+    std::vector<RotSet> rot_sets;
+    std::vector<std::vector<std::vector<HFr>>> low;
+    std::set<HFr, FrLess> super_points;
+
+    Prover(b200zk_pk* p, bool advice_dev, bool rng_dev) : pk(p), advice_on_device(advice_dev), split_upload(sh.on() && !advice_dev && !rng_dev) { sh.assign(L, S, A + I + S + 3 * L); }
+
+    // arrays of lookup l: LK as listed at lk_bufs; LKC product z, permuted input a', permuted table s', table value
+    // (all indexed by global coset row)
+    fe_t* LK(uint32_t l, uint32_t which) const { return lk_bufs + ((size_t)l * 7 + which) * n; }
+    fe_t* LKC(uint32_t l, uint32_t which) const {
+        return pk->lk_early ? lk_all + ((size_t)l * 4 + which) * CL * n : lk_cosets + (size_t)which * ext;
+    }
+    // column idx of type 0 advice, 1 fixed, 2 instance: its values, its quotient cosets
+    const fe_t* column_values(uint32_t type, uint32_t idx) const { return (type == 0 ? advice_values : type == 1 ? pk->fixed_values : inst_values) + (size_t)idx * n; }
+    const fe_t* column_cosets(uint32_t type, uint32_t idx) const { return (type == 0 ? advice_cosets : type == 1 ? pk->fixed_cosets : inst_cosets) + (size_t)idx * ext; }
+    bool lin_mine() const { return pk->gate_prog[QC_LINEAR].second && sh.coset_owner(0) == sh.R; }
+
+    void mark(const char* label) {                  // called right after a host synchronisation: where the wall clock of the proof goes
         pk->trace.push_back({label, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count()});
-    };
-    // quotient cosets this rank extends and evaluates
-    const uint32_t cj0 = sh.coset_lo(sh.R), cj1 = sh.coset_lo(sh.R + 1);
-    if (sh.on()) ZK_TRY(sh.cm->set_window(ctx, pk->arena, pk->arena_bytes));
-    auto share = [&](const std::vector<CommPiece>& pieces) -> int32_t {
+    }
+    cudaError_t copy_rows(fe_t* dst, const fe_t* src, size_t count) {
+        return cudaMemcpyAsync(dst, src, count * sizeof(fe_t), cudaMemcpyDeviceToDevice, st);
+    }
+    int32_t share(const std::vector<CommPiece>& pieces) {
         if (!sh.on() || pieces.empty()) return B200ZK_OK;
         PhaseTimer t(pk, PH_OTHER);
         return sh.cm->share(ctx, pieces.data(), pieces.size(), ctx->stream);
-    };
-    auto my_cosets = [&](const fe_t* d_coeffs, fe_t* d_out, uint32_t j0, uint32_t j1) -> int32_t {     // cosets [j0, j1) of d_out
+    }
+    int32_t my_cosets(const fe_t* d_coeffs, fe_t* d_out, uint32_t j0, uint32_t j1) {     // cosets [j0, j1) of d_out
         if (j0 >= j1) return B200ZK_OK;
         PhaseTimer t(pk, PH_NTT);
-        return ntt_run_cosets(ctx, d_coeffs, d_out + (size_t)j0 * pk->n, pk->dom->k, pk->dom->omega, pk->coset_pow + (size_t)j0 * pk->n, j1 - j0);
-    };
-    ZK_CUDA(ctx, cudaMemsetAsync(pk->d_err, 0, 4, st));
-    host::Transcript tr;
-    Arena ar{pk->arena, pk->arena_bytes};
-    const size_t draws = b200zk_pk_rng_draws(pk);
-
-    // ---- arena carve-up
-    fe_t* advice_values = ar.take<fe_t>(A * n);
-    fe_t* advice_polys = ar.take<fe_t>(A * n);
-    fe_t* inst_values = ar.take<fe_t>(I * n);
-    fe_t* inst_polys = ar.take<fe_t>(I * n);
-    uint32_t* wide = ar.take<uint32_t>(draws * 16);
-    fe_t* rnd = ar.take<fe_t>(draws);
-    fe_t* lk_bufs = ar.take<fe_t>(7 * (size_t)L * n);            // per lookup: cin ctab pin ptab pin_poly ptab_poly z_poly
-    fe_t* perm_polys = ar.take<fe_t>((size_t)S * n);
-    fe_t* perm_cosets = ar.take<fe_t>((size_t)S * ext);
-    fe_t* tmp_n = ar.take<fe_t>(3 * n);
-    fe_t* h = ar.take<fe_t>(ext);
-    fe_t* advice_cosets = ar.take<fe_t>(A * ext);
-    fe_t* inst_cosets = ar.take<fe_t>(I * ext);
-    fe_t* lk_cosets = ar.take<fe_t>(4 * ext);                    // z, a', s', table_value
-    fe_t* h_lk = ar.take<fe_t>(ext);                             // lookup and low-degree gate part of the quotient when it runs on fewer cosets
-    fe_t* h_lin = ar.take<fe_t>(n);                              // linear gates on coset 0
-    const uint32_t CL = pk->lk_cosets_n;                         // == q unless the lookup terms and the low gates run on fewer cosets
-    const bool lk_split = CL < pk->q;
-    const size_t lk_span = (size_t)CL * n;                       // rows of one lookup coset array
-    fe_t* lk_all = pk->lk_early ? ar.take<fe_t>(4 * (size_t)L * lk_span) : nullptr;
-    // arrays of lookup l: product z, permuted input a', permuted table s', table value (all indexed by global coset row)
-    auto LKC = [&](uint32_t l, uint32_t which) { return pk->lk_early ? lk_all + ((size_t)l * 4 + which) * lk_span : lk_cosets + (size_t)which * ext; };
-    // this rank's share of the cosets the lookup terms run on
-    const uint32_t lj0 = std::min(cj0, CL), lj1 = std::min(cj1, CL);
-    const uint32_t lk_row0 = lj0 * (uint32_t)n, lk_rows = (lj1 - lj0) * (uint32_t)n;
-    auto lookup_table_value = [&](uint32_t l, const HFr* chv) {  // (compressed input + beta)(compressed table + gamma) on this rank's lookup cosets
+        return ntt_run_cosets(ctx, d_coeffs, d_out + (size_t)j0 * n, dom->k, dom->omega, pk->coset_pow + (size_t)j0 * n, j1 - j0);
+    }
+    // Lagrange commitments to `cols`, column i computed by rank owners[i], into the transcript
+    int32_t commit_columns(const std::vector<const fe_t*>& cols, const std::vector<int>& owners, const char* label, uint32_t* flag = nullptr) {
+        std::vector<HAffine> pts;
+        ZK_TRY(commit_multi_split(pk, sh, cols, owners, n, true, pts, flag));
+        for (auto& pt : pts) tr.write_point(pt);
+        mark(label);
+        return B200ZK_OK;
+    }
+    int32_t commit_random() {
+        std::vector<HAffine> pts;
+        ZK_TRY(commit_multi_range(pk, sh, {rnd + dl.random}, n, false, pts));
+        random_pt = pts[0];
+        return B200ZK_OK;
+    }
+    void lookup_table_value(uint32_t l) {            // (compressed input + beta)(compressed table + gamma) on this rank's lookup cosets
         PhaseTimer t(pk, PH_QUOT);
-        ExprArgs ea = expr_args(pk, pk->lookup_prog[l].first, pk->lookup_prog[l].second, true, EXM_LOOKUP_PROD, chv, LKC(l, 3), nullptr);
+        ExprArgs ea = expr_args(pk, pk->lookup_prog[l].first, pk->lookup_prog[l].second, true, EXM_LOOKUP_PROD, ch, LKC(l, 3), nullptr);
         ea.row0 = lk_row0; ea.rows = lk_rows;
         expr_kernel<<<nb(lk_rows), PK_THREADS, 0, ctx->stream>>>(ea);
         ctx->launches++;
-    };
-    fe_t* h_poly = ar.take<fe_t>(n);
-    fe_t* set_sums = ar.take<fe_t>(8 * n);
-    fe_t* sh_tmp = ar.take<fe_t>(4 * n);
-    fe_t* set_quot = ar.take<fe_t>(8 * n);                       // sharded proof: Q_i of every rotation set, computed by its owner
-    if (!ar.ok) return fail(ctx, B200ZK_ENOMEM, "create_proof", "arena too small");
-    auto LK = [&](uint32_t l, uint32_t which) { return lk_bufs + ((size_t)l * 7 + which) * n; };
-    pk->dbg.clear();
-    pk->dbg["advice_values"] = {advice_values, A * n}; pk->dbg["advice_polys"] = {advice_polys, A * n};
-    pk->dbg["lookups"] = {lk_bufs, 7 * (size_t)L * n}; pk->dbg["perm_polys"] = {perm_polys, (size_t)S * n};
-    pk->dbg["h"] = {h, ext}; pk->dbg["rnd"] = {rnd, draws}; pk->dbg["tmp_n"] = {tmp_n, 3 * n};
-    pk->dbg["advice_cosets"] = {advice_cosets, A * ext}; pk->dbg["h_poly"] = {h_poly, n};
+    }
+    // one gate program per class, each on its own rows (quot_plan.hpp); a class without gates starts its accumulator at 0
+    int32_t gate_class(uint32_t cls, fe_t* out, uint32_t row0, uint32_t rows) {
+        if (!rows) return B200ZK_OK;
+        PhaseTimer t(pk, PH_QUOT);
+        if (!pk->gate_prog[cls].second) {
+            ZK_CUDA(ctx, cudaMemsetAsync(out + row0, 0, (size_t)rows * sizeof(fe_t), st));
+            return B200ZK_OK;
+        }
+        ExprArgs ea = expr_args(pk, pk->gate_prog[cls].first, pk->gate_prog[cls].second, true, EXM_ACC0, ch, out, nullptr);
+        ea.row0 = row0; ea.rows = rows;
+        expr_kernel<<<nb(rows), PK_THREADS, 0, st>>>(ea);
+        ctx->launches++;
+        return B200ZK_OK;
+    }
+    int32_t opened(const fe_t* poly, const HFr& pt, HFr* out) const {
+        for (size_t i = 0; i < pairs.size(); ++i)
+            if (pairs[i].poly == poly && pairs[i].point == pt) { *out = values[i]; return B200ZK_OK; }
+        return fail(ctx, B200ZK_EINVAL, "create_proof", "internal: evaluation of a pair that is not opened");
+    }
+    int32_t write_eval(const fe_t* poly, const HFr& pt) {
+        HFr e = HFr::zero();
+        ZK_TRY(opened(poly, pt, &e));
+        tr.write_scalar(e);
+        return B200ZK_OK;
+    }
 
-    // ---- pointer tables for this proof
-    {
+    int32_t carve() {
+        Arena ar{pk->arena, pk->arena_bytes};
+        advice_values = ar.take<fe_t>(A * n);
+        advice_polys = ar.take<fe_t>(A * n);
+        inst_values = ar.take<fe_t>(I * n);
+        inst_polys = ar.take<fe_t>(I * n);
+        wide = ar.take<uint32_t>(dl.total * 16);
+        rnd = ar.take<fe_t>(dl.total);                                // the rng stream as field elements, laid out as dl says
+        lk_bufs = ar.take<fe_t>(7 * (size_t)L * n);                   // per lookup: cin ctab pin ptab pin_poly ptab_poly z_poly
+        perm_polys = ar.take<fe_t>((size_t)S * n);
+        perm_cosets = ar.take<fe_t>((size_t)S * ext);
+        tmp_n = ar.take<fe_t>(3 * n);
+        h = ar.take<fe_t>(ext);
+        advice_cosets = ar.take<fe_t>(A * ext);
+        inst_cosets = ar.take<fe_t>(I * ext);
+        lk_cosets = ar.take<fe_t>(4 * ext);                           // z, a', s', table_value; after vanishing_construct the q pieces of h
+        h_lk = ar.take<fe_t>(ext);                                    // lookup and low-degree gate part of the quotient when it runs on fewer cosets
+        h_lin = ar.take<fe_t>(n);                                     // linear gates on coset 0
+        lk_all = pk->lk_early ? ar.take<fe_t>(4 * (size_t)L * CL * n) : nullptr;    // the lookup cosets of all lookups side by side
+        h_poly = ar.take<fe_t>(n);
+        set_sums = ar.take<fe_t>(8 * n);
+        fe_t* sh_tmp = ar.take<fe_t>(4 * n);                          // SHPLONK work space: hx lx t0 t1
+        set_quot = ar.take<fe_t>(8 * n);                              // sharded proof: Q_i of every rotation set, computed by its owner
+        if (!ar.ok) return fail(ctx, B200ZK_ENOMEM, "create_proof", "arena too small");
+        hx = sh_tmp; lx = sh_tmp + n; t0 = sh_tmp + 2 * n; t1 = sh_tmp + 3 * n;
+        pk->dbg.clear();
+        pk->dbg["advice_values"] = {advice_values, A * n}; pk->dbg["advice_polys"] = {advice_polys, A * n};
+        pk->dbg["lookups"] = {lk_bufs, 7 * (size_t)L * n}; pk->dbg["perm_polys"] = {perm_polys, (size_t)S * n};
+        pk->dbg["h"] = {h, ext}; pk->dbg["rnd"] = {rnd, dl.total}; pk->dbg["tmp_n"] = {tmp_n, 3 * n};
+        pk->dbg["advice_cosets"] = {advice_cosets, A * ext}; pk->dbg["h_poly"] = {h_poly, n};
+
+        // pointer tables for this proof
         PtrTab pt{F, A, I};
         std::vector<const fe_t*> tab(pt.total());
         for (uint32_t c = 0; c < F; ++c) { tab[pt.fixed_values() + c] = pk->fixed_values + (size_t)c * n; tab[pt.fixed_cosets() + c] = pk->fixed_cosets + (size_t)c * ext; }
@@ -537,197 +612,164 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
         for (uint32_t c = 0; c < I; ++c) { tab[pt.inst_values() + c] = inst_values + (size_t)c * n; tab[pt.inst_cosets() + c] = inst_cosets + (size_t)c * ext; }
         ZK_CUDA(ctx, cudaMemcpyAsync(pk->d_ptrs, tab.data(), tab.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
         ZK_CUDA(ctx, cudaStreamSynchronize(st));
+        return B200ZK_OK;
     }
 
-    // ---- step 0/1: vk.hash_into, instances
-    tr.common_scalar(transcript_repr);
-    ZK_CUDA(ctx, cudaMemsetAsync(inst_values, 0, I * n * sizeof(fe_t), st));
-    for (uint32_t c = 0; c < I; ++c) {
-        uint32_t len = instance_lens[c];
-        if (len > usable) return fail(ctx, B200ZK_ESYNTH, "create_proof", "InstanceTooLarge");
-        const uint64_t* v = (const uint64_t*)instance_columns[c];
-        for (uint32_t i = 0; i < len; ++i) tr.common_scalar(HFr::from_limbs(v + 4 * i));
-        if (len) ZK_CUDA(ctx, cudaMemcpyAsync(inst_values + (size_t)c * n, v, (size_t)len * sizeof(fe_t), cudaMemcpyHostToDevice, st));
-    }
-    ZK_CUDA(ctx, cudaMemcpyAsync(inst_polys, inst_values, I * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, st));
-    for (uint32_t c = 0; c < I; ++c) ZK_TRY(lagrange_to_coeff(pk, inst_polys + (size_t)c * n));
-
-    // ---- randomness: Fr::random = from_u512 of the caller's 64-byte draws, consumed in upstream order
-    // Sharded proof from host buffers: the host -> device traffic is split as well — every rank uploads 1/G of the rng
-    // stream and its own advice columns over its PCIe link, and the ranks exchange them over NVLink.
-    const bool split_upload = sh.on() && !advice_on_device && !rng_on_device;
-    if (split_upload) {
-        const size_t d0 = draws * (size_t)sh.R / sh.G, d1 = draws * (size_t)(sh.R + 1) / sh.G;
-        ZK_CUDA(ctx, cudaMemcpyAsync(wide + d0 * 16, (const char*)rng_wide + d0 * 64, (d1 - d0) * 64, cudaMemcpyHostToDevice, st));
-        if (d1 > d0) { from_u512_kernel<<<nb(d1 - d0), PK_THREADS, 0, st>>>(wide + d0 * 16, rnd + d0, d1 - d0); ctx->launches++; }
-        std::vector<CommPiece> pieces;
-        for (int r = 0; r < sh.G; ++r) {
-            const size_t a0 = draws * (size_t)r / sh.G, a1 = draws * (size_t)(r + 1) / sh.G;
-            pieces.push_back({rnd + a0, (a1 - a0) * sizeof(fe_t), r});
+    // step 0/1: vk.hash_into, instances
+    int32_t instances(const void* const* instance_columns, const uint32_t* instance_lens, const HFr& transcript_repr) {
+        tr.common_scalar(transcript_repr);
+        ZK_CUDA(ctx, cudaMemsetAsync(inst_values, 0, I * n * sizeof(fe_t), st));
+        for (uint32_t c = 0; c < I; ++c) {
+            uint32_t len = instance_lens[c];
+            if (len > usable) return fail(ctx, B200ZK_ESYNTH, "create_proof", "InstanceTooLarge");
+            const uint64_t* v = (const uint64_t*)instance_columns[c];
+            for (uint32_t i = 0; i < len; ++i) tr.common_scalar(HFr::from_limbs(v + 4 * i));
+            if (len) ZK_CUDA(ctx, cudaMemcpyAsync(inst_values + (size_t)c * n, v, (size_t)len * sizeof(fe_t), cudaMemcpyHostToDevice, st));
         }
-        ZK_TRY(share(pieces));
-    } else {
-        if (rng_on_device) ZK_CUDA(ctx, cudaMemcpyAsync(wide, rng_wide, draws * 64, cudaMemcpyDeviceToDevice, st));
-        else ZK_CUDA(ctx, cudaMemcpyAsync(wide, rng_wide, draws * 64, cudaMemcpyHostToDevice, st));
+        ZK_CUDA(ctx, cudaMemcpyAsync(inst_polys, inst_values, I * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, st));
+        for (uint32_t c = 0; c < I; ++c) ZK_TRY(lagrange_to_coeff(pk, inst_polys + (size_t)c * n));
+        return B200ZK_OK;
+    }
+
+    // randomness: Fr::random = from_u512 of the caller's 64-byte draws
+    int32_t upload_rng(const void* rng_wide, bool rng_on_device) {
+        const size_t draws = dl.total;
+        if (split_upload) {
+            const size_t d0 = draws * (size_t)sh.R / sh.G, d1 = draws * (size_t)(sh.R + 1) / sh.G;
+            ZK_CUDA(ctx, cudaMemcpyAsync(wide + d0 * 16, (const char*)rng_wide + d0 * 64, (d1 - d0) * 64, cudaMemcpyHostToDevice, st));
+            if (d1 > d0) { from_u512_kernel<<<nb(d1 - d0), PK_THREADS, 0, st>>>(wide + d0 * 16, rnd + d0, d1 - d0); ctx->launches++; }
+            std::vector<CommPiece> pieces;
+            for (int r = 0; r < sh.G; ++r) {
+                const size_t a0 = draws * (size_t)r / sh.G, a1 = draws * (size_t)(r + 1) / sh.G;
+                pieces.push_back({rnd + a0, (a1 - a0) * sizeof(fe_t), r});
+            }
+            return share(pieces);
+        }
+        ZK_CUDA(ctx, cudaMemcpyAsync(wide, rng_wide, draws * 64, rng_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
         from_u512_kernel<<<nb(draws), PK_THREADS, 0, st>>>(wide, rnd, draws);
         ctx->launches++;
+        return B200ZK_OK;
     }
-    size_t rpos = 0;
-    auto rng_take = [&](size_t count) { fe_t* p = rnd + rpos; rpos += count; return p; };
-    auto copy_rows = [&](fe_t* dst, const fe_t* src, size_t count) {
-        return cudaMemcpyAsync(dst, src, count * sizeof(fe_t), cudaMemcpyDeviceToDevice, st);
-    };
 
-    // ---- step 2: advice columns: blinding rows, blinds, commitments.
+    // step 2: advice columns: blinding rows, blinds, commitments.
     // The columns arrive on the pk's copy stream one at a time (H2D from the caller's buffers, 32 MiB each at
     // k = 20, or D2D), each followed by its blinding rows; col_events[c] marks column c complete.  Everything that
     // does not need the transcript starts under that transfer: on the side stream the coefficient form and the
     // quotient cosets of column c as soon as it has landed (step 10, moved up), and — when the columns come from
     // the host — on the main stream the commitment to the vanishing argument's random polynomial (step 8), which
     // depends on the rng stream only.  The main stream then waits for the last column and commits all of them.
-    if (!pk->copy_stream) {
-        ZK_CUDA(ctx, cudaStreamCreateWithFlags(&pk->copy_stream, cudaStreamNonBlocking));
-        ZK_CUDA(ctx, cudaEventCreateWithFlags(&pk->ev_rnd, cudaEventDisableTiming));
-    }
-    while (pk->col_events.size() < A) {
-        cudaEvent_t e;
-        ZK_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        pk->col_events.push_back(e);
-    }
-    const size_t rpos_advice = rpos;
-    rng_take((size_t)A * (bf + 1));
-    rng_take(A);                                                  // Blind per column (unused by KZG)
-    ZK_CUDA(ctx, cudaEventRecord(pk->ev_rnd, st));
-    ZK_CUDA(ctx, cudaStreamWaitEvent(pk->copy_stream, pk->ev_rnd, 0));      // rnd (and the arena's previous users on st) first
-    for (uint32_t c = 0; c < A; ++c) {
-        fe_t* col = advice_values + (size_t)c * n;
-        if (split_upload && !sh.mine(c)) continue;                // arrives from its owner below
-        if (advice_on_device) ZK_CUDA(ctx, cudaMemcpyAsync(col, d_advice_in + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, pk->copy_stream));
-        else ZK_CUDA(ctx, cudaMemcpyAsync(col, advice_host[c], n * sizeof(fe_t), cudaMemcpyHostToDevice, pk->copy_stream));
-        ZK_CUDA(ctx, cudaMemcpyAsync(col + usable, rnd + rpos_advice + (size_t)c * (bf + 1), (bf + 1) * sizeof(fe_t), cudaMemcpyDeviceToDevice, pk->copy_stream));
-        ZK_CUDA(ctx, cudaEventRecord(pk->col_events[c], pk->copy_stream));
-    }
-    // position of the random polynomial in the rng stream (draw order: SURVEY.md 8(a7))
-    const size_t rpos_random = rpos + (size_t)L * (2 * (bf + 1) + 2) + (size_t)S * (bf + 1) + (size_t)L * (bf + 1);
-    HAffine random_pt = {host::HFq::zero(), host::HFq::zero()};
-    const bool random_early = !advice_on_device;
-    auto commit_random = [&]() -> int32_t {
-        std::vector<HAffine> pts;
-        ZK_TRY(commit_multi_range(pk, sh, {rnd + rpos_random}, n, false, pts));
-        random_pt = pts[0];
-        return B200ZK_OK;
-    };
-    if (split_upload) {                                           // random-polynomial commit under the upload, then the column exchange
-        ZK_TRY(commit_random());
-        std::vector<CommPiece> pieces;
-        for (uint32_t c = 0; c < A; ++c) {
-            if (sh.mine(c)) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[c], 0));
-            pieces.push_back({advice_values + (size_t)c * n, n * sizeof(fe_t), sh.owner(c)});
+    int32_t advice(const fe_t* d_advice_in, const void* const* advice_host) {
+        if (!pk->copy_stream) {
+            ZK_CUDA(ctx, cudaStreamCreateWithFlags(&pk->copy_stream, cudaStreamNonBlocking));
+            ZK_CUDA(ctx, cudaEventCreateWithFlags(&pk->ev_rnd, cudaEventDisableTiming));
         }
-        ZK_TRY(share(pieces));
-    }
-    {
-        SideStream side(ctx);
-        // columns that are already on the device arrive at once: all their inverse transforms as one batched launch per pass
-        // (columns from the host keep the per-column pipeline under the upload)
-        const bool batch_intt = advice_on_device && A > 1 && ((uint64_t)A << dom->k) <= 0xFFFFFFFFull;
-        if (batch_intt) {
-            ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, pk->col_events[A - 1], 0));
-            ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys, advice_values, (size_t)A * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
-            ZK_TRY(lagrange_to_coeff_batch(pk, advice_polys, A));
+        while (pk->col_events.size() < A) {
+            cudaEvent_t e;
+            ZK_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            pk->col_events.push_back(e);
         }
+        ZK_CUDA(ctx, cudaEventRecord(pk->ev_rnd, st));
+        ZK_CUDA(ctx, cudaStreamWaitEvent(pk->copy_stream, pk->ev_rnd, 0));      // rnd (and the arena's previous users on st) first
         for (uint32_t c = 0; c < A; ++c) {
-            if (!batch_intt) {
-                if (!split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, pk->col_events[c], 0));
-                ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys + (size_t)c * n, advice_values + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
-                ZK_TRY(lagrange_to_coeff(pk, advice_polys + (size_t)c * n));
+            fe_t* col = advice_values + (size_t)c * n;
+            if (split_upload && !sh.mine(c)) continue;                // arrives from its owner below
+            if (advice_on_device) ZK_CUDA(ctx, cudaMemcpyAsync(col, d_advice_in + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, pk->copy_stream));
+            else ZK_CUDA(ctx, cudaMemcpyAsync(col, advice_host[c], n * sizeof(fe_t), cudaMemcpyHostToDevice, pk->copy_stream));
+            ZK_CUDA(ctx, cudaMemcpyAsync(col + usable, rnd + dl.advice_rows(c), (bf + 1) * sizeof(fe_t), cudaMemcpyDeviceToDevice, pk->copy_stream));
+            ZK_CUDA(ctx, cudaEventRecord(pk->col_events[c], pk->copy_stream));
+        }
+        if (split_upload) {                                           // random-polynomial commit under the upload, then the column exchange
+            ZK_TRY(commit_random());
+            std::vector<CommPiece> pieces;
+            for (uint32_t c = 0; c < A; ++c) {
+                if (sh.mine(c)) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[c], 0));
+                pieces.push_back({advice_values + (size_t)c * n, n * sizeof(fe_t), sh.owner(c)});
             }
-            ZK_TRY(my_cosets(advice_polys + (size_t)c * n, advice_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.adv_need[c])));
+            ZK_TRY(share(pieces));
         }
-        // only the cosets a consumer reads (QuotPlan::adv_need / inst_need): the higher ones are never written
-        for (uint32_t c = 0; c < I; ++c) ZK_TRY(my_cosets(inst_polys + (size_t)c * n, inst_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.inst_need[c])));
-    }
-    if (random_early && !split_upload) ZK_TRY(commit_random());
-    if (A && !split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[A - 1], 0));
-    {
+        {
+            SideStream side(ctx);
+            // columns that are already on the device arrive at once: all their inverse transforms as one batched launch per pass
+            // (columns from the host keep the per-column pipeline under the upload)
+            const bool batch_intt = advice_on_device && A > 1 && ((uint64_t)A << dom->k) <= 0xFFFFFFFFull;
+            if (batch_intt) {
+                ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, pk->col_events[A - 1], 0));
+                ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys, advice_values, (size_t)A * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
+                ZK_TRY(lagrange_to_coeff(pk, advice_polys, A));
+            }
+            for (uint32_t c = 0; c < A; ++c) {
+                if (!batch_intt) {
+                    if (!split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, pk->col_events[c], 0));
+                    ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys + (size_t)c * n, advice_values + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
+                    ZK_TRY(lagrange_to_coeff(pk, advice_polys + (size_t)c * n));
+                }
+                ZK_TRY(my_cosets(advice_polys + (size_t)c * n, advice_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.adv_need[c])));
+            }
+            // only the cosets a consumer reads (QuotPlan::adv_need / inst_need): the higher ones are never written
+            for (uint32_t c = 0; c < I; ++c) ZK_TRY(my_cosets(inst_polys + (size_t)c * n, inst_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.inst_need[c])));
+        }
+        if (!advice_on_device && !split_upload) ZK_TRY(commit_random());
+        if (A && !split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[A - 1], 0));
         std::vector<const fe_t*> cols;
         std::vector<int> owners;
-        std::vector<HAffine> pts;
         for (uint32_t c = 0; c < A; ++c) { cols.push_back(advice_values + (size_t)c * n); owners.push_back(sh.owner(c)); }
-        ZK_TRY(commit_multi_split(pk, sh, cols, owners, n, true, pts));
-        for (uint32_t c = 0; c < A; ++c) tr.write_point(pts[c]);
-        mark("advice_commits");
+        return commit_columns(cols, owners, "advice_commits");
     }
-    HFr ch[4];                                                    // theta, beta, gamma, y
-    ch[EXF_THETA] = tr.squeeze_challenge();
-    ch[EXF_BETA] = ch[EXF_GAMMA] = ch[EXF_Y] = HFr::zero();
 
-    // ---- step 4: lookups, commit_permuted
-    // lookup l lives on rank l mod G from here to its grand product; every rank walks the rng stream
-    for (uint32_t l = 0; l < L; ++l) {
-        fe_t *cin = LK(l, 0), *ctab = LK(l, 1), *pin = LK(l, 2), *ptab = LK(l, 3), *pin_poly = LK(l, 4), *ptab_poly = LK(l, 5);
-        if (!sh.lk_mine(l)) { rng_take(2 * (bf + 1) + 2); continue; }
-        {
-            PhaseTimer t(pk, PH_LOOKUP);
-            ExprArgs ea = expr_args(pk, pk->lookup_prog[l].first, pk->lookup_prog[l].second, false, EXM_ACC01, ch, cin, ctab);
-            expr_kernel<<<nb(n), PK_THREADS, 0, st>>>(ea);
-            ctx->launches++;
-            ZK_TRY(lookup_permute_run(ctx, cin, ctab, (uint32_t)usable, pin, ptab, pk->d_err));
+    // step 4: lookups, commit_permuted.  Lookup l lives on rank sh.lk_owner(l) from here to its grand product.
+    int32_t lookup_permute() {
+        for (uint32_t l = 0; l < L; ++l) {
+            if (!sh.lk_mine(l)) continue;
+            fe_t *cin = LK(l, 0), *ctab = LK(l, 1), *pin = LK(l, 2), *ptab = LK(l, 3), *pin_poly = LK(l, 4), *ptab_poly = LK(l, 5);
+            {
+                PhaseTimer t(pk, PH_LOOKUP);
+                ExprArgs ea = expr_args(pk, pk->lookup_prog[l].first, pk->lookup_prog[l].second, false, EXM_ACC01, ch, cin, ctab);
+                expr_kernel<<<nb(n), PK_THREADS, 0, st>>>(ea);
+                ctx->launches++;
+                ZK_TRY(lookup_permute_run(ctx, cin, ctab, (uint32_t)usable, pin, ptab, pk->d_err));
+            }
+            ZK_CUDA(ctx, copy_rows(pin + usable, rnd + dl.lookup_input_rows(l), bf + 1));
+            ZK_CUDA(ctx, copy_rows(ptab + usable, rnd + dl.lookup_table_rows(l), bf + 1));
+            ZK_CUDA(ctx, copy_rows(pin_poly, pin, n));
+            ZK_TRY(lagrange_to_coeff(pk, pin_poly));
+            ZK_CUDA(ctx, copy_rows(ptab_poly, ptab, n));
+            ZK_TRY(lagrange_to_coeff(pk, ptab_poly));
         }
-        ZK_CUDA(ctx, copy_rows(pin + usable, rng_take(bf + 1), bf + 1));
-        ZK_CUDA(ctx, copy_rows(ptab + usable, rng_take(bf + 1), bf + 1));
-        ZK_CUDA(ctx, copy_rows(pin_poly, pin, n));
-        ZK_TRY(lagrange_to_coeff(pk, pin_poly));
-        rng_take(1);
-        ZK_CUDA(ctx, copy_rows(ptab_poly, ptab, n));
-        ZK_TRY(lagrange_to_coeff(pk, ptab_poly));
-        rng_take(1);
-    }
-    {
-        uint32_t err = 0;
         ZK_CUDA(ctx, cudaMemcpyAsync(ctx->pinned, pk->d_err, 4, cudaMemcpyDeviceToHost, st));
         ZK_CUDA(ctx, cudaStreamSynchronize(st));
-        err = *(const uint32_t*)ctx->pinned;
-        if (L) {                                                  // permuted input / table commitments of all lookups, one batch
+        uint32_t err = *(const uint32_t*)ctx->pinned;
+        if (L) {                                                      // permuted input / table commitments of all lookups, one batch
             std::vector<const fe_t*> cols;
             std::vector<int> owners;
-            std::vector<HAffine> pts;
             for (uint32_t l = 0; l < L; ++l) { cols.push_back(LK(l, 2)); cols.push_back(LK(l, 3)); owners.push_back(sh.lk_owner(l)); owners.push_back(sh.lk_owner(l)); }
-            ZK_TRY(commit_multi_split(pk, sh, cols, owners, n, true, pts, &err));
-            for (auto& pt : pts) tr.write_point(pt);
-            mark("lookup_permuted_commits");
+            ZK_TRY(commit_columns(cols, owners, "lookup_permuted_commits", &err));
         }
         if (err) return fail(ctx, B200ZK_ESYNTH, "create_proof", "ConstraintSystemFailure: lookup input not in table");
         // the permuted polynomials in coefficient form: every rank opens them, the coset owners extend them
         std::vector<CommPiece> pieces;
         for (uint32_t l = 0; l < L; ++l) { pieces.push_back({LK(l, 4), n * sizeof(fe_t), sh.lk_owner(l)}); pieces.push_back({LK(l, 5), n * sizeof(fe_t), sh.lk_owner(l)}); }
-        ZK_TRY(share(pieces));
+        return share(pieces);
     }
-    ch[EXF_BETA] = tr.squeeze_challenge();
-    ch[EXF_GAMMA] = tr.squeeze_challenge();
-    const HFr beta = ch[EXF_BETA], gamma = ch[EXF_GAMMA];
-    if (pk->lk_early && lk_rows) {                               // side stream: a', s' cosets and the table values (theta, beta, gamma known)
+
+    // side stream, once theta, beta and gamma are known: the a', s' cosets and the table values of every lookup
+    int32_t lookup_cosets_early() {
+        if (!pk->lk_early || !lk_rows) return B200ZK_OK;
         SideStream side(ctx);
         for (uint32_t l = 0; l < L; ++l) {
             ZK_TRY(my_cosets(LK(l, 4), LKC(l, 1), lj0, lj1));
             ZK_TRY(my_cosets(LK(l, 5), LKC(l, 2), lj0, lj1));
-            lookup_table_value(l, ch);
+            lookup_table_value(l);
         }
+        return B200ZK_OK;
     }
 
-    // ---- step 6: permutation argument
-    auto column_values = [&](uint32_t type, uint32_t idx) -> const fe_t* {
-        return type == 0 ? advice_values + (size_t)idx * n : type == 1 ? pk->fixed_values + (size_t)idx * n : inst_values + (size_t)idx * n;
-    };
-    auto column_cosets = [&](uint32_t type, uint32_t idx) -> const fe_t* {
-        return type == 0 ? advice_cosets + (size_t)idx * ext : type == 1 ? pk->fixed_cosets + (size_t)idx * ext : inst_cosets + (size_t)idx * ext;
-    };
-    {
-        // Upstream chains the sets through z_s[0] = z_{s-1}[n - (bf + 1)].  On one GPU that is a 32-byte read-back per
-        // set.  Sharded, set s lives on rank s mod G: every rank runs its sets from z[0] = 1, the S totals
-        // t_s = z'_s[n - (bf + 1)] are exchanged, and set s is scaled by t_0 ... t_{s-1} — the same field elements.
+    // step 6: permutation argument.
+    // Upstream chains the sets through z_s[0] = z_{s-1}[n - (bf + 1)].  On one GPU that is a 32-byte read-back per
+    // set.  Sharded, set s lives on rank sh.set_owner(s): every rank runs its sets from z[0] = 1, the S totals
+    // t_s = z'_s[n - (bf + 1)] are exchanged, and set s is scaled by t_0 ... t_{s-1} — the same field elements.
+    int32_t permutation_products() {
+        const HFr beta = ch[EXF_BETA], gamma = ch[EXF_GAMMA];
         HFr last_z = HFr::one(), deltaomega = HFr::one();
-        std::vector<const fe_t*> blind_rows(S);
         for (uint32_t s = 0; s < S; ++s) {
             fe_t* z = perm_polys + (size_t)s * n;
             uint32_t c0 = s * pk->chunk, c1 = std::min<uint32_t>(c0 + pk->chunk, pk->P);
@@ -739,8 +781,6 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
                 pa.coef[j - c0] = to_dev(deltaomega * beta);
                 deltaomega = deltaomega * host::fr_delta();
             }
-            blind_rows[s] = rng_take(bf);
-            rng_take(1);
             if (!sh.set_mine(s)) continue;
             {
                 PhaseTimer t(pk, PH_PERM);
@@ -754,7 +794,7 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
             }
             ZK_CUDA(ctx, cudaMemcpyAsync((fe_t*)ctx->pinned + (sh.on() ? sh.set_slot[s] : 0), z + (n - (bf + 1)), sizeof(fe_t), cudaMemcpyDeviceToHost, st));
             if (!sh.on()) {
-                ZK_CUDA(ctx, copy_rows(z + (n - bf), blind_rows[s], bf));
+                ZK_CUDA(ctx, copy_rows(z + (n - bf), rnd + dl.set_rows(s), bf));
                 ZK_CUDA(ctx, cudaStreamSynchronize(st));
                 last_z = HFr::from_limbs(ctx->pinned);
             }
@@ -773,455 +813,419 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
                 fe_t* z = perm_polys + (size_t)s * n;
                 if (sh.set_mine(s)) {
                     if (s) { scale_kernel<<<nb(n - bf), PK_THREADS, 0, st>>>(z, to_dev(carry), n - bf); ctx->launches++; }
-                    ZK_CUDA(ctx, copy_rows(z + (n - bf), blind_rows[s], bf));
+                    ZK_CUDA(ctx, copy_rows(z + (n - bf), rnd + dl.set_rows(s), bf));
                 }
                 carry = carry * all_t[(size_t)sh.set_owner(s) * slots + sh.set_slot[s]];
             }
             mark("perm_products");
         }
-        if (S) {                                                  // the S grand products: one batch of commitments, then coefficients and cosets
+        if (S) {                                                      // the S grand products: one batch of commitments, then coefficients and cosets
             std::vector<const fe_t*> cols;
             std::vector<int> owners;
-            std::vector<HAffine> pts;
             for (uint32_t s = 0; s < S; ++s) { cols.push_back(perm_polys + (size_t)s * n); owners.push_back(sh.set_owner(s)); }
-            ZK_TRY(commit_multi_split(pk, sh, cols, owners, n, true, pts));
-            for (auto& pt : pts) tr.write_point(pt);
-            mark("permutation_commits");
+            ZK_TRY(commit_columns(cols, owners, "permutation_commits"));
         }
-        {
-            std::vector<CommPiece> pieces;
-            const bool batch_intt = !sh.on() && S > 1 && ((uint64_t)S << dom->k) <= 0xFFFFFFFFull;      // one rank: all sets in one launch per pass
-            if (batch_intt) ZK_TRY(lagrange_to_coeff_batch(pk, perm_polys, S));
-            for (uint32_t s = 0; s < S; ++s) {
-                fe_t* z = perm_polys + (size_t)s * n;
-                if (!batch_intt && sh.set_mine(s)) ZK_TRY(lagrange_to_coeff(pk, z));
-                pieces.push_back({z, n * sizeof(fe_t), sh.set_owner(s)});
-            }
-            ZK_TRY(share(pieces));
-            for (uint32_t s = 0; s < S; ++s) ZK_TRY(my_cosets(perm_polys + (size_t)s * n, perm_cosets + (size_t)s * ext, cj0, cj1));
+        std::vector<CommPiece> pieces;
+        const bool batch_intt = !sh.on() && S > 1 && ((uint64_t)S << dom->k) <= 0xFFFFFFFFull;      // one rank: all sets in one launch per pass
+        if (batch_intt) ZK_TRY(lagrange_to_coeff(pk, perm_polys, S));
+        for (uint32_t s = 0; s < S; ++s) {
+            fe_t* z = perm_polys + (size_t)s * n;
+            if (!batch_intt && sh.set_mine(s)) ZK_TRY(lagrange_to_coeff(pk, z));
+            pieces.push_back({z, n * sizeof(fe_t), sh.set_owner(s)});
         }
+        ZK_TRY(share(pieces));
+        for (uint32_t s = 0; s < S; ++s) ZK_TRY(my_cosets(perm_polys + (size_t)s * n, perm_cosets + (size_t)s * ext, cj0, cj1));
+        return B200ZK_OK;
     }
 
-    // ---- step 7: lookups, commit_product
-    for (uint32_t l = 0; l < L; ++l) {
-        fe_t* z = LK(l, 6);
-        if (!sh.lk_mine(l)) { rng_take(bf + 1); continue; }
-        {
-            PhaseTimer t(pk, PH_LOOKUP);
-            LookupProdArgs la{LK(l, 2), LK(l, 3), LK(l, 0), LK(l, 1), to_dev(beta), to_dev(gamma), tmp_n, (uint32_t)n};
-            lookup_den_kernel<<<nb(n), PK_THREADS, 0, st>>>(la);
-            ctx->launches++;
-            ZK_TRY(batch_invert_run(ctx, tmp_n, n, 0));
-            lookup_num_kernel<<<nb(n), PK_THREADS, 0, st>>>(la);
-            ctx->launches++;
-            ZK_TRY(prefix_product_run(ctx, tmp_n, z, n, HFr::one()));
+    // step 7: lookups, commit_product
+    int32_t lookup_products() {
+        for (uint32_t l = 0; l < L; ++l) {
+            if (!sh.lk_mine(l)) continue;
+            fe_t* z = LK(l, 6);
+            {
+                PhaseTimer t(pk, PH_LOOKUP);
+                LookupProdArgs la{LK(l, 2), LK(l, 3), LK(l, 0), LK(l, 1), to_dev(ch[EXF_BETA]), to_dev(ch[EXF_GAMMA]), tmp_n, (uint32_t)n};
+                lookup_den_kernel<<<nb(n), PK_THREADS, 0, st>>>(la);
+                ctx->launches++;
+                ZK_TRY(batch_invert_run(ctx, tmp_n, n, 0));
+                lookup_num_kernel<<<nb(n), PK_THREADS, 0, st>>>(la);
+                ctx->launches++;
+                ZK_TRY(prefix_product_run(ctx, tmp_n, z, n, HFr::one()));
+            }
+            ZK_CUDA(ctx, copy_rows(z + (n - bf), rnd + dl.lookup_product_rows(l), bf));
         }
-        ZK_CUDA(ctx, copy_rows(z + (n - bf), rng_take(bf), bf));
-        rng_take(1);
-    }
-    if (L) {
+        if (!L) return B200ZK_OK;
         std::vector<const fe_t*> cols;
         std::vector<int> owners;
-        std::vector<HAffine> pts;
         std::vector<CommPiece> pieces;
         for (uint32_t l = 0; l < L; ++l) { cols.push_back(LK(l, 6)); owners.push_back(sh.lk_owner(l)); pieces.push_back({LK(l, 6), n * sizeof(fe_t), sh.lk_owner(l)}); }
-        ZK_TRY(commit_multi_split(pk, sh, cols, owners, n, true, pts));
-        for (auto& pt : pts) tr.write_point(pt);
-        mark("lookup_product_commits");
+        ZK_TRY(commit_columns(cols, owners, "lookup_product_commits"));
         for (uint32_t l = 0; l < L; ++l) if (sh.lk_mine(l)) ZK_TRY(lagrange_to_coeff(pk, LK(l, 6)));
         ZK_TRY(share(pieces));
-        if (pk->lk_early && lk_rows) {                           // side stream: the product cosets
+        if (pk->lk_early && lk_rows) {                                // side stream: the product cosets
             SideStream side(ctx);
             for (uint32_t l = 0; l < L; ++l) ZK_TRY(my_cosets(LK(l, 6), LKC(l, 0), lj0, lj1));
         }
-    }
-
-    // ---- step 8: vanishing argument, random polynomial
-    if (rpos != rpos_random) return fail(ctx, B200ZK_EINVAL, "create_proof", "rng draw order");
-    const fe_t* random_poly = rng_take(n);
-    rng_take(1);
-    if (!random_early) ZK_TRY(commit_random());
-    tr.write_point(random_pt);
-    ch[EXF_Y] = tr.squeeze_challenge();
-    const HFr y = ch[EXF_Y];
-    if (!pk->gate_exp.empty()) {                                  // the gates' powers of y (ExprArgs::wts)
-        std::vector<HFr> ypow(1, HFr::one());
-        for (uint32_t i = 0; i < cs.gates.size(); ++i) {
-            while (ypow.size() <= pk->gate_exp[i]) ypow.push_back(ypow.back() * y);
-            ((fe_t*)pk->h_wts)[i] = to_dev(ypow[pk->gate_exp[i]]);
-        }
-        ZK_CUDA(ctx, cudaMemcpyAsync(pk->d_wts, pk->h_wts, cs.gates.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
-    }
-
-    // ---- step 10: advice / instance cosets were started on the side stream after the advice commitments
-    ZK_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_join, 0));
-
-    // ---- step 11: evaluate_h
-    // this rank's rows of the quotient: its cosets [cj0, cj1) (all of them on a single GPU)
-    const uint32_t my_row0 = cj0 * (uint32_t)n, my_rows = (cj1 - cj0) * (uint32_t)n;
-    // one gate program per class, each on its own rows (quot_plan.hpp); a class without gates starts its accumulator at 0
-    auto gate_class = [&](uint32_t cls, fe_t* out, uint32_t row0, uint32_t rows) -> int32_t {
-        if (!rows) return B200ZK_OK;
-        PhaseTimer t(pk, PH_QUOT);
-        if (!pk->gate_prog[cls].second) {
-            ZK_CUDA(ctx, cudaMemsetAsync(out + row0, 0, (size_t)rows * sizeof(fe_t), st));
-            return B200ZK_OK;
-        }
-        ExprArgs ea = expr_args(pk, pk->gate_prog[cls].first, pk->gate_prog[cls].second, true, EXM_ACC0, ch, out, nullptr);
-        ea.row0 = row0; ea.rows = rows;
-        expr_kernel<<<nb(rows), PK_THREADS, 0, st>>>(ea);
-        ctx->launches++;
         return B200ZK_OK;
-    };
-    const bool lin_mine = pk->gate_prog[QC_LINEAR].second && sh.coset_owner(0) == sh.R;
-    if (lin_mine) ZK_TRY(gate_class(QC_LINEAR, h_lin, 0, (uint32_t)n));
-    if (my_rows) {
-        ZK_TRY(gate_class(QC_MAIN, h, my_row0, my_rows));
-        PhaseTimer t(pk, PH_QUOT);
-        if (S) {
-            QuotPermAArgs qa{};
-            qa.h = h; qa.y = to_dev(y); qa.l0 = pk->l0; qa.l_last = pk->l_last; qa.nsets = S;
-            qa.rows = my_rows; qa.row0 = my_row0; qa.log_ext = dom->k; qa.rot_scale = rot_scale; qa.last_rot = -(int32_t)(bf + 1);
-            for (uint32_t s = 0; s < S; ++s) qa.z[s] = perm_cosets + (size_t)s * ext;
-            quot_perm_a_kernel<<<nb(my_rows), PK_THREADS, 0, st>>>(qa);
-            ctx->launches++;
-            HFr cd = beta * host::fr_zeta();                      // delta_start = beta * ZETA
-            for (uint32_t s = 0; s < S; ++s) {
-                uint32_t c0 = s * pk->chunk, c1 = std::min<uint32_t>(c0 + pk->chunk, pk->P);
-                QuotPermBArgs qb{};
-                qb.h = h; qb.y = to_dev(y); qb.beta = to_dev(beta); qb.gamma = to_dev(gamma); qb.l_active = pk->l_active;
-                qb.z = perm_cosets + (size_t)s * ext; qb.ncols = c1 - c0; qb.rows = my_rows; qb.row0 = my_row0; qb.log_ext = dom->k; qb.rot_scale = rot_scale;
-                qb.omega_pows = pk->omega_pows; qb.coset_fac = pk->coset_fac;
-                for (uint32_t j = c0; j < c1; ++j) {
-                    qb.values[j - c0] = column_cosets(cs.perm[j].first, cs.perm[j].second);
-                    qb.sigma[j - c0] = pk->perm_cosets + (size_t)j * ext;
-                    qb.cdelta[j - c0] = to_dev(cd);
-                    cd = cd * host::fr_delta();
+    }
+
+    // step 8: vanishing argument, the random polynomial (committed under the advice upload when the columns come from the host)
+    int32_t random_poly() {
+        if (advice_on_device) ZK_TRY(commit_random());
+        tr.write_point(random_pt);
+        return B200ZK_OK;
+    }
+
+    // step 11: evaluate_h on this rank's rows of the quotient: its cosets [cj0, cj1) (all of them on a single GPU)
+    int32_t evaluate_h() {
+        if (!pk->gate_exp.empty()) {                                  // the gates' powers of y (ExprArgs::wts)
+            std::vector<HFr> ypow(1, HFr::one());
+            for (uint32_t i = 0; i < cs.gates.size(); ++i) {
+                while (ypow.size() <= pk->gate_exp[i]) ypow.push_back(ypow.back() * ch[EXF_Y]);
+                ((fe_t*)pk->h_wts)[i] = to_dev(ypow[pk->gate_exp[i]]);
+            }
+            ZK_CUDA(ctx, cudaMemcpyAsync(pk->d_wts, pk->h_wts, cs.gates.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
+        }
+        // step 10: the advice / instance cosets were started on the side stream after the advice commitments
+        ZK_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_join, 0));
+        const uint32_t rot_scale = 1u;                                // rotations stay inside a coset (prover_kernels.cuh)
+        const HFr beta = ch[EXF_BETA], gamma = ch[EXF_GAMMA], y = ch[EXF_Y];
+        const uint32_t my_row0 = cj0 * (uint32_t)n, my_rows = (cj1 - cj0) * (uint32_t)n;
+        if (lin_mine()) ZK_TRY(gate_class(QC_LINEAR, h_lin, 0, (uint32_t)n));
+        if (my_rows) {
+            ZK_TRY(gate_class(QC_MAIN, h, my_row0, my_rows));
+            PhaseTimer t(pk, PH_QUOT);
+            if (S) {
+                QuotPermAArgs qa{};
+                qa.h = h; qa.y = to_dev(y); qa.l0 = pk->l0; qa.l_last = pk->l_last; qa.nsets = S;
+                qa.rows = my_rows; qa.row0 = my_row0; qa.log_ext = dom->k; qa.rot_scale = rot_scale; qa.last_rot = -(int32_t)(bf + 1);
+                for (uint32_t s = 0; s < S; ++s) qa.z[s] = perm_cosets + (size_t)s * ext;
+                quot_perm_a_kernel<<<nb(my_rows), PK_THREADS, 0, st>>>(qa);
+                ctx->launches++;
+                HFr cd = beta * host::fr_zeta();                      // delta_start = beta * ZETA
+                for (uint32_t s = 0; s < S; ++s) {
+                    uint32_t c0 = s * pk->chunk, c1 = std::min<uint32_t>(c0 + pk->chunk, pk->P);
+                    QuotPermBArgs qb{};
+                    qb.h = h; qb.y = to_dev(y); qb.beta = to_dev(beta); qb.gamma = to_dev(gamma); qb.l_active = pk->l_active;
+                    qb.z = perm_cosets + (size_t)s * ext; qb.ncols = c1 - c0; qb.rows = my_rows; qb.row0 = my_row0; qb.log_ext = dom->k; qb.rot_scale = rot_scale;
+                    qb.omega_pows = pk->omega_pows; qb.coset_fac = pk->coset_fac;
+                    for (uint32_t j = c0; j < c1; ++j) {
+                        qb.values[j - c0] = column_cosets(cs.perm[j].first, cs.perm[j].second);
+                        qb.sigma[j - c0] = pk->perm_cosets + (size_t)j * ext;
+                        qb.cdelta[j - c0] = to_dev(cd);
+                        cd = cd * host::fr_delta();
+                    }
+                    quot_perm_b_kernel<<<nb(my_rows), PK_THREADS, 0, st>>>(qb);
+                    ctx->launches++;
                 }
-                quot_perm_b_kernel<<<nb(my_rows), PK_THREADS, 0, st>>>(qb);
+            }
+        }
+        // lookup terms: on all q cosets straight into h, or — when their degree allows — on the first CL cosets into
+        // h_lk, extended to the other cosets after the per-coset iNTT (lookup_extrapolate_row)
+        if (lk_split) ZK_TRY(gate_class(QC_LOW, h_lk, lk_row0, lk_rows));
+        for (uint32_t l = 0; l < L && lk_rows; ++l) {
+            fe_t *zc = LKC(l, 0), *ac = LKC(l, 1), *sc = LKC(l, 2), *tv = LKC(l, 3);
+            if (!pk->lk_early) {
+                ZK_TRY(my_cosets(LK(l, 6), zc, lj0, lj1));
+                ZK_TRY(my_cosets(LK(l, 4), ac, lj0, lj1));
+                ZK_TRY(my_cosets(LK(l, 5), sc, lj0, lj1));
+                lookup_table_value(l);
+            }
+            PhaseTimer t(pk, PH_QUOT);
+            QuotLookupArgs ql{};
+            ql.h = lk_split ? h_lk : h; ql.y = to_dev(y); ql.beta = to_dev(beta); ql.gamma = to_dev(gamma);
+            ql.l0 = pk->l0; ql.l_last = pk->l_last; ql.l_active = pk->l_active; ql.z = zc; ql.a = ac; ql.s = sc; ql.table_value = tv;
+            ql.log_ext = dom->k; ql.rot_scale = rot_scale; ql.rows = lk_rows; ql.row0 = lk_row0;
+            { HFr yp = y * y; for (int i = 0; i < 4; ++i) { ql.ypow[i] = to_dev(yp); yp = yp * y; } }
+            quot_lookup_kernel<<<nb(lk_rows), PK_THREADS, 0, st>>>(ql);
+            ctx->launches++;
+        }
+        ZK_CUDA(ctx, cudaGetLastError());
+        return B200ZK_OK;
+    }
+
+    // step 12: vanishing construct, then the commitments to the q pieces of h
+    int32_t vanishing_construct() {
+        {
+            // divide by the vanishing polynomial (constant c_j^n - 1 on coset j), per-coset iNTT, then
+            // the q x q interpolation across cosets gives the coefficients of h piece by piece
+            PhaseTimer t(pk, PH_NTT);
+            HFr y_lk = HFr::one();                                    // h = h_gates_perm * y^(5 L) + h_lk
+            if (lk_split) {
+                for (uint32_t i = 0; i < 5 * L; ++i) y_lk = y_lk * ch[EXF_Y];  // (the low gates' weights leave this factor to the lookup kernels)
+                for (uint32_t j = lj0; j < lj1; ++j)                           // divided by the vanishing polynomial before the extrapolation
+                    ZK_TRY(intt_scaled(pk, h_lk + j * n, 1, dom->ifft_divisor * pk->coset_t[j]));
+            }
+            for (uint32_t j = cj0; j < cj1; ++j) ZK_TRY(intt_scaled(pk, h + j * n, 1, dom->ifft_divisor * pk->coset_t[j] * y_lk));
+            // the linear gates' part of h, degree < n: coefficients in X / c_0
+            if (lin_mine()) ZK_TRY(intt_scaled(pk, h_lin, 1, dom->ifft_divisor * pk->coset_t[0]));
+            if (sh.on()) {                                            // every coset's coefficients to every rank: q (+ CL) x n elements
+                std::vector<CommPiece> pieces;
+                for (uint32_t j = 0; j < pk->q; ++j) pieces.push_back({h + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
+                if (lk_split) for (uint32_t j = 0; j < CL; ++j) pieces.push_back({h_lk + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
+                if (pk->gate_prog[QC_LINEAR].second) pieces.push_back({h_lin, n * sizeof(fe_t), sh.coset_owner(0)});
+                ZK_TRY(sh.cm->share(ctx, pieces.data(), pieces.size(), st));
+            }
+            if (lk_split) {
+                lookup_extrapolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h_lk, pk->coset_pow_inv, pk->lk_lambda, nullptr, CL, pk->q, n);
                 ctx->launches++;
             }
-        }
-    }
-    // lookup terms: on all q cosets straight into h, or — when their degree allows — on the first CL cosets into
-    // h_lk, extended to the other cosets after the per-coset iNTT (lookup_extrapolate_row)
-    if (lk_split) ZK_TRY(gate_class(QC_LOW, h_lk, lk_row0, lk_rows));
-    for (uint32_t l = 0; l < L && lk_rows; ++l) {
-        fe_t *zc = LKC(l, 0), *ac = LKC(l, 1), *sc = LKC(l, 2), *tv = LKC(l, 3);
-        if (!pk->lk_early) {
-            ZK_TRY(my_cosets(LK(l, 6), zc, lj0, lj1));
-            ZK_TRY(my_cosets(LK(l, 4), ac, lj0, lj1));
-            ZK_TRY(my_cosets(LK(l, 5), sc, lj0, lj1));
-            lookup_table_value(l, ch);
-        }
-        PhaseTimer t(pk, PH_QUOT);
-        QuotLookupArgs ql{};
-        ql.h = lk_split ? h_lk : h; ql.y = to_dev(y); ql.beta = to_dev(beta); ql.gamma = to_dev(gamma);
-        ql.l0 = pk->l0; ql.l_last = pk->l_last; ql.l_active = pk->l_active; ql.z = zc; ql.a = ac; ql.s = sc; ql.table_value = tv;
-        ql.log_ext = dom->k; ql.rot_scale = rot_scale; ql.rows = lk_rows; ql.row0 = lk_row0;
-        { HFr yp = y * y; for (int i = 0; i < 4; ++i) { ql.ypow[i] = to_dev(yp); yp = yp * y; } }
-        quot_lookup_kernel<<<nb(lk_rows), PK_THREADS, 0, st>>>(ql);
-        ctx->launches++;
-    }
-    ZK_CUDA(ctx, cudaGetLastError());
-
-    // ---- step 12: vanishing construct
-    {
-        // divide by the vanishing polynomial (constant c_j^n - 1 on coset j), per-coset iNTT, then
-        // the q x q interpolation across cosets gives the coefficients of h piece by piece
-        PhaseTimer t(pk, PH_NTT);
-        HFr y_lk = HFr::one();                                    // h = h_gates_perm * y^(5 L) + h_lk
-        if (lk_split) {
-            for (uint32_t i = 0; i < 5 * L; ++i) y_lk = y_lk * y;       // (the low gates' weights leave this factor to the lookup kernels)
-            for (uint32_t j = lj0; j < lj1; ++j) {                     // divided by the vanishing polynomial before the extrapolation
-                HFr f = dom->ifft_divisor * pk->coset_t[j];
-                HFr post[3] = {f, f, f};
-                ZK_TRY(ntt_run(ctx, h_lk + j * n, (uint32_t)n, h_lk + j * n, dom->k, dom->omega_inv, nullptr, post));
-            }
-        }
-        for (uint32_t j = cj0; j < cj1; ++j) {
-            HFr f = dom->ifft_divisor * pk->coset_t[j] * y_lk;
-            HFr post[3] = {f, f, f};
-            ZK_TRY(ntt_run(ctx, h + j * n, (uint32_t)n, h + j * n, dom->k, dom->omega_inv, nullptr, post));
-        }
-        if (lin_mine) {                                           // the linear gates' part of h, degree < n: coefficients in X / c_0
-            HFr f = dom->ifft_divisor * pk->coset_t[0];
-            HFr post[3] = {f, f, f};
-            ZK_TRY(ntt_run(ctx, h_lin, (uint32_t)n, h_lin, dom->k, dom->omega_inv, nullptr, post));
-        }
-        if (sh.on()) {                                            // every coset's coefficients to every rank: q (+ CL) x n elements
-            std::vector<CommPiece> pieces;
-            for (uint32_t j = 0; j < pk->q; ++j) pieces.push_back({h + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
-            if (lk_split) for (uint32_t j = 0; j < CL; ++j) pieces.push_back({h_lk + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
-            if (pk->gate_prog[QC_LINEAR].second) pieces.push_back({h_lin, n * sizeof(fe_t), sh.coset_owner(0)});
-            ZK_TRY(sh.cm->share(ctx, pieces.data(), pieces.size(), st));
-        }
-        if (lk_split) {
-            lookup_extrapolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h_lk, pk->coset_pow_inv, pk->lk_lambda, nullptr, CL, pk->q, n);
+            coset_interpolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h, pk->coset_pow_inv, pk->vinv, pk->q, n, lk_cosets, lk_split ? h_lk : nullptr,
+                                                                     pk->gate_prog[QC_LINEAR].second ? h_lin : nullptr);
             ctx->launches++;
+            ZK_CUDA(ctx, cudaGetLastError());
         }
-        coset_interpolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h, pk->coset_pow_inv, pk->vinv, pk->q, n, lk_cosets, lk_split ? h_lk : nullptr,
-                                                                 pk->gate_prog[QC_LINEAR].second ? h_lin : nullptr);
-        ctx->launches++;
-        ZK_CUDA(ctx, cudaGetLastError());
-        h = lk_cosets;                                            // q pieces of n coefficients
-    }
-    const uint32_t q = pk->q;
-    rng_take(q);                                                  // h_blinds
-    {
         std::vector<const fe_t*> cols;
         std::vector<HAffine> pts;
-        for (uint32_t i = 0; i < q; ++i) cols.push_back(h + (size_t)i * n);
+        for (uint32_t i = 0; i < pk->q; ++i) cols.push_back(lk_cosets + (size_t)i * n);
         ZK_TRY(commit_multi_range(pk, sh, cols, n, false, pts));
         for (auto& pt : pts) tr.write_point(pt);
         mark("quotient_and_h_commits");
-    }
-    if (rpos != draws) return fail(ctx, B200ZK_EINVAL, "create_proof", "internal: rng draw count mismatch");
-    const HFr x = tr.squeeze_challenge();
-    const HFr xn = x.pow_u64(n);
-
-    // ---- step 14: evaluations
-    std::unique_ptr<PhaseTimer> open_timer(new PhaseTimer(pk, PH_OPEN));
-    std::map<std::pair<const fe_t*, std::array<uint64_t, 4>>, HFr> eval_cache;
-    auto eval_at = [&](const fe_t* poly, const HFr& pt, HFr* out) -> int32_t {
-        std::array<uint64_t, 4> key = {pt.v[0], pt.v[1], pt.v[2], pt.v[3]};
-        auto it = eval_cache.find({poly, key});
-        if (it != eval_cache.end()) { *out = it->second; return B200ZK_OK; }
-        ZK_TRY(eval_dev(pk, poly, n, pt, out));
-        eval_cache[{poly, key}] = *out;
         return B200ZK_OK;
-    };
-    struct Query { const fe_t* poly; HFr point; };
-    std::vector<Query> queries;
-    int32_t rc = B200ZK_OK;
-    auto finish = [&](int32_t r) { open_timer.reset(); return r; };
-    const HFr x_next = rotate_omega(dom, x, 1), x_prev = rotate_omega(dom, x, -1), x_last = rotate_omega(dom, x, -(int)(bf + 1));
-    // vanishing::evaluate: h_poly = sum_i (x^n)^i h_piece_i
-    fold_pieces_kernel<<<nb(n), PK_THREADS, 0, st>>>(h, q, n, to_dev(xn), h_poly);
-    ctx->launches++;
-    // multiopen queries in upstream order (step 15); every evaluation written in step 14 is one of
-    // them, so all of them are evaluated here in ONE batched launch pair and served from the cache.
-    for (size_t i = 0; i < cs.adv_q.size(); i += 2) queries.push_back({advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1])});
-    for (uint32_t s = 0; s < S; ++s) { queries.push_back({perm_polys + (size_t)s * n, x}); queries.push_back({perm_polys + (size_t)s * n, x_next}); }
-    for (uint32_t s = S; s-- > 0;) if (s + 1 < S) queries.push_back({perm_polys + (size_t)s * n, x_last});
-    for (uint32_t l = 0; l < L; ++l) {
-        queries.push_back({LK(l, 6), x}); queries.push_back({LK(l, 4), x}); queries.push_back({LK(l, 5), x});
-        queries.push_back({LK(l, 4), x_prev}); queries.push_back({LK(l, 6), x_next});
     }
-    for (size_t i = 0; i < cs.fix_q.size(); i += 2) queries.push_back({pk->fixed_polys + (size_t)cs.fix_q[i] * n, rotate_omega(dom, x, cs.fix_q[i + 1])});
-    for (uint32_t j = 0; j < pk->P; ++j) queries.push_back({pk->perm_polys + (size_t)j * n, x});
-    queries.push_back({h_poly, x});
-    queries.push_back({random_poly, x});
-    {
-        std::vector<const fe_t*> bp; std::vector<HFr> bx;
-        std::set<std::pair<const fe_t*, std::array<uint64_t, 4>>> seen;
-        for (auto& qy : queries) {
-            std::array<uint64_t, 4> key = {qy.point.v[0], qy.point.v[1], qy.point.v[2], qy.point.v[3]};
-            if (seen.insert({qy.poly, key}).second) { bp.push_back(qy.poly); bx.push_back(qy.point); }
+
+    // step 14: evaluations
+    int32_t evaluations() {
+        PhaseTimer t(pk, PH_OPEN);
+        const HFr x_next = rotate_omega(dom, x, 1), x_prev = rotate_omega(dom, x, -1), x_last = rotate_omega(dom, x, -(int)(bf + 1));
+        const fe_t* random = rnd + dl.random;
+        // vanishing::evaluate: h_poly = sum_i (x^n)^i h_piece_i
+        fold_pieces_kernel<<<nb(n), PK_THREADS, 0, st>>>(lk_cosets, pk->q, n, to_dev(x.pow_u64(n)), h_poly);
+        ctx->launches++;
+        // multiopen queries in upstream order (step 15); every evaluation the transcript gets is one of them, so their
+        // distinct pairs are evaluated here in ONE batched launch pair
+        for (size_t i = 0; i < cs.adv_q.size(); i += 2) queries.push_back({advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1])});
+        for (uint32_t s = 0; s < S; ++s) { queries.push_back({perm_polys + (size_t)s * n, x}); queries.push_back({perm_polys + (size_t)s * n, x_next}); }
+        for (uint32_t s = S; s-- > 0;) if (s + 1 < S) queries.push_back({perm_polys + (size_t)s * n, x_last});
+        for (uint32_t l = 0; l < L; ++l) {
+            queries.push_back({LK(l, 6), x}); queries.push_back({LK(l, 4), x}); queries.push_back({LK(l, 5), x});
+            queries.push_back({LK(l, 4), x_prev}); queries.push_back({LK(l, 6), x_next});
         }
-        std::vector<HFr> vals(bp.size());
+        for (size_t i = 0; i < cs.fix_q.size(); i += 2) queries.push_back({pk->fixed_polys + (size_t)cs.fix_q[i] * n, rotate_omega(dom, x, cs.fix_q[i + 1])});
+        for (uint32_t j = 0; j < pk->P; ++j) queries.push_back({pk->perm_polys + (size_t)j * n, x});
+        queries.push_back({h_poly, x});
+        queries.push_back({random, x});
+        for (auto& qy : queries)
+            if (std::none_of(pairs.begin(), pairs.end(), [&](const Query& p) { return p.poly == qy.poly && p.point == qy.point; })) pairs.push_back(qy);
+        std::vector<const fe_t*> bp; std::vector<HFr> bx;             // sharded: pair i on rank i mod G, 32 bytes each back to everybody
+        for (size_t i = 0; i < pairs.size(); ++i) if (sh.mine((uint32_t)i)) { bp.push_back(pairs[i].poly); bx.push_back(pairs[i].point); }
+        values.resize(pairs.size());
         if (!sh.on()) {
-            rc = eval_batch_run(ctx, bp.data(), bx.data(), bp.size(), n, vals.data());
-            if (rc != B200ZK_OK) return finish(rc);
-        } else {                                                  // evaluation i on rank i mod G, 32 bytes each back to everybody
-            std::vector<const fe_t*> mp; std::vector<HFr> mx;
-            for (size_t i = 0; i < bp.size(); ++i) if (sh.mine((uint32_t)i)) { mp.push_back(bp[i]); mx.push_back(bx[i]); }
-            const size_t slots = (bp.size() + sh.G - 1) / sh.G;
+            ZK_TRY(eval_batch_run(ctx, bp.data(), bx.data(), bp.size(), n, values.data()));
+        } else {
+            const size_t slots = (pairs.size() + sh.G - 1) / sh.G;
             std::vector<HFr> mv(slots, HFr::zero()), all(slots * sh.G);
-            rc = eval_batch_run(ctx, mp.data(), mx.data(), mp.size(), n, mv.data());
-            if (rc != B200ZK_OK) return finish(rc);
+            ZK_TRY(eval_batch_run(ctx, bp.data(), bx.data(), bp.size(), n, mv.data()));
             for (size_t b0 = 0; b0 < slots; b0 += COMM_HOST_MAX / sizeof(HFr)) {       // in pieces the staging buffers hold
                 const size_t m = std::min(slots - b0, COMM_HOST_MAX / sizeof(HFr));
                 std::vector<HFr> part(m * sh.G);
-                rc = sh.cm->allgather_host(ctx, mv.data() + b0, m * sizeof(HFr), part.data(), st);
-                if (rc != B200ZK_OK) return finish(rc);
+                ZK_TRY(sh.cm->allgather_host(ctx, mv.data() + b0, m * sizeof(HFr), part.data(), st));
                 for (int r = 0; r < sh.G; ++r) for (size_t i = 0; i < m; ++i) all[(size_t)r * slots + b0 + i] = part[(size_t)r * m + i];
             }
-            for (size_t i = 0; i < bp.size(); ++i) vals[i] = all[(i % sh.G) * slots + i / sh.G];
+            for (size_t i = 0; i < pairs.size(); ++i) values[i] = all[(i % sh.G) * slots + i / sh.G];
         }
-        for (size_t i = 0; i < bp.size(); ++i) eval_cache[{bp[i], {bx[i].v[0], bx[i].v[1], bx[i].v[2], bx[i].v[3]}}] = vals[i];
         mark("evaluations");
+        // the transcript's order: advice, fixed, random, sigma, permutation sets, lookups
+        for (size_t i = 0; i < cs.adv_q.size(); i += 2) ZK_TRY(write_eval(advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1])));
+        for (size_t i = 0; i < cs.fix_q.size(); i += 2) ZK_TRY(write_eval(pk->fixed_polys + (size_t)cs.fix_q[i] * n, rotate_omega(dom, x, cs.fix_q[i + 1])));
+        ZK_TRY(write_eval(random, x));
+        for (uint32_t j = 0; j < pk->P; ++j) ZK_TRY(write_eval(pk->perm_polys + (size_t)j * n, x));
+        for (uint32_t s = 0; s < S; ++s) {
+            const fe_t* zp = perm_polys + (size_t)s * n;
+            ZK_TRY(write_eval(zp, x)); ZK_TRY(write_eval(zp, x_next));
+            if (s + 1 < S) ZK_TRY(write_eval(zp, x_last));
+        }
+        for (uint32_t l = 0; l < L; ++l) {                           // product z, permuted input a', permuted table s'
+            ZK_TRY(write_eval(LK(l, 6), x)); ZK_TRY(write_eval(LK(l, 6), x_next));
+            ZK_TRY(write_eval(LK(l, 4), x)); ZK_TRY(write_eval(LK(l, 4), x_prev)); ZK_TRY(write_eval(LK(l, 5), x));
+        }
+        return B200ZK_OK;
     }
-    for (size_t i = 0; i < cs.adv_q.size() && rc == B200ZK_OK; i += 2) {
-        HFr e; rc = eval_at(advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1]), &e);
-        tr.write_scalar(e);
-    }
-    for (size_t i = 0; i < cs.fix_q.size() && rc == B200ZK_OK; i += 2) {
-        HFr e; rc = eval_at(pk->fixed_polys + (size_t)cs.fix_q[i] * n, rotate_omega(dom, x, cs.fix_q[i + 1]), &e);
-        tr.write_scalar(e);
-    }
-    if (rc != B200ZK_OK) return finish(rc);
-    {
-        HFr e; rc = eval_at(random_poly, x, &e); tr.write_scalar(e);
-    }
-    for (uint32_t j = 0; j < pk->P && rc == B200ZK_OK; ++j) {
-        HFr e; rc = eval_at(pk->perm_polys + (size_t)j * n, x, &e); tr.write_scalar(e);
-    }
-    for (uint32_t s = 0; s < S && rc == B200ZK_OK; ++s) {
-        const fe_t* zp = perm_polys + (size_t)s * n;
-        HFr e;
-        rc = eval_at(zp, x, &e); tr.write_scalar(e);
-        if (rc == B200ZK_OK) { rc = eval_at(zp, x_next, &e); tr.write_scalar(e); }
-        if (rc == B200ZK_OK && s + 1 < S) { rc = eval_at(zp, x_last, &e); tr.write_scalar(e); }
-    }
-    for (uint32_t l = 0; l < L && rc == B200ZK_OK; ++l) {
-        HFr e;
-        const fe_t *zp = LK(l, 6), *ap = LK(l, 4), *sp = LK(l, 5);
-        rc = eval_at(zp, x, &e); tr.write_scalar(e);
-        if (rc == B200ZK_OK) { rc = eval_at(zp, x_next, &e); tr.write_scalar(e); }
-        if (rc == B200ZK_OK) { rc = eval_at(ap, x, &e); tr.write_scalar(e); }
-        if (rc == B200ZK_OK) { rc = eval_at(ap, x_prev, &e); tr.write_scalar(e); }
-        if (rc == B200ZK_OK) { rc = eval_at(sp, x, &e); tr.write_scalar(e); }
-    }
-    if (rc != B200ZK_OK) return finish(rc);
 
-    // ---- step 15: ProverSHPLONK::create_proof over `queries` (built above)
-    const HFr sy = tr.squeeze_challenge();
-    // construct_intermediate_sets
-    struct CommSet { const fe_t* poly; std::set<HFr, FrLess> pts; };
-    std::vector<CommSet> comm_sets;
-    std::set<HFr, FrLess> super_points;
-    for (auto& qy : queries) {
-        super_points.insert(qy.point);
-        auto it = std::find_if(comm_sets.begin(), comm_sets.end(), [&](const CommSet& c) { return c.poly == qy.poly; });
-        if (it == comm_sets.end()) { comm_sets.push_back({qy.poly, {}}); it = comm_sets.end() - 1; }
-        it->pts.insert(qy.point);
-    }
-    struct RotSet { std::vector<HFr> pts; std::vector<const fe_t*> polys; };
-    std::vector<RotSet> rot_sets;
-    for (auto& c : comm_sets) {
-        std::vector<HFr> pts(c.pts.begin(), c.pts.end());
-        auto it = std::find_if(rot_sets.begin(), rot_sets.end(), [&](const RotSet& r) {
-            return r.pts.size() == pts.size() && std::equal(pts.begin(), pts.end(), r.pts.begin());
-        });
-        if (it == rot_sets.end()) { rot_sets.push_back({pts, {}}); it = rot_sets.end() - 1; }
-        if (std::find(it->polys.begin(), it->polys.end(), c.poly) == it->polys.end()) it->polys.push_back(c.poly);
-    }
-    if (rot_sets.size() > 8) return finish(fail(ctx, B200ZK_EINVAL, "create_proof", "more than 8 rotation sets"));
-    // low-degree equivalents
-    std::vector<std::vector<std::vector<HFr>>> low(rot_sets.size());
-    for (size_t i = 0; i < rot_sets.size(); ++i) {
-        const size_t m = rot_sets[i].pts.size();
-        if (m > 8) return finish(fail(ctx, B200ZK_EINVAL, "create_proof", "rotation set with more than 8 points"));
-        // the Lagrange basis of the set's points once (m field inversions), then every polynomial of the set is a
-        // combination of it: the same interpolant as arithmetic::lagrange_interpolate per polynomial, without an
-        // inversion per polynomial and point (they were ~2 ms of host time per proof at every size)
-        std::vector<std::vector<HFr>> basis(m);
-        for (size_t j = 0; j < m; ++j) { std::vector<HFr> unit(m, HFr::zero()); unit[j] = HFr::one(); basis[j] = lagrange_interpolate(rot_sets[i].pts, unit); }
-        for (const fe_t* poly : rot_sets[i].polys) {
-            std::vector<HFr> lowp(m, HFr::zero());
-            for (size_t j = 0; j < m; ++j) {
-                HFr e; rc = eval_at(poly, rot_sets[i].pts[j], &e); if (rc != B200ZK_OK) return finish(rc);
-                for (size_t c = 0; c < m; ++c) lowp[c] = lowp[c] + basis[j][c] * e;
-            }
-            low[i].push_back(lowp);
-        }
-    }
-    const HFr sv = tr.squeeze_challenge();
-    fe_t *hx = sh_tmp, *lx = sh_tmp + n, *t0 = sh_tmp + 2 * n, *t1 = sh_tmp + 3 * n;
-    ZK_CUDA(ctx, cudaMemsetAsync(hx, 0, n * sizeof(fe_t), st));
-    {
-        // Sharded: rotation set i (its linear combination A_i and the Kate divisions that give Q_i) lives on rank i mod G; both
-        // polynomials are then broadcast — every rank needs A_i again for the linearisation polynomial — and h1 = sum v^i Q_i
-        // is formed everywhere.
-        HFr v_pow = HFr::one();
-        for (size_t i = 0; i < rot_sets.size(); ++i) {
-            fe_t* sum = set_sums + i * n;                        // A_i = sum_j y^j P_ij
-            if (sh.on() && !sh.mine((uint32_t)i)) continue;
-            HFr y_pow = HFr::one();
-            std::vector<HFr> rlow(rot_sets[i].pts.size(), HFr::zero());   // R_i = sum_j y^j r_ij
-            for (size_t j0 = 0; j0 < rot_sets[i].polys.size(); j0 += 16) {
-                LinCombArgs la{};
-                la.m = (uint32_t)std::min<size_t>(16, rot_sets[i].polys.size() - j0);
-                for (uint32_t j = 0; j < la.m; ++j) {
-                    la.p[j] = rot_sets[i].polys[j0 + j];
-                    la.s[j] = to_dev(y_pow);
-                    for (size_t c = 0; c < low[i][j0 + j].size(); ++c) rlow[c] = rlow[c] + low[i][j0 + j][c] * y_pow;
-                    y_pow = y_pow * sy;
+    // step 15: ProverSHPLONK::create_proof over `queries`
+    int32_t shplonk() {
+        HFr sy, sv, su;
+        {
+            PhaseTimer t(pk, PH_OPEN);
+            sy = tr.squeeze_challenge();
+            ZK_TRY(shplonk_sets());
+            sv = tr.squeeze_challenge();
+            // h1 = sum_i v^i Q_i into hx.  Sharded: rotation set i (its linear combination A_i and the Kate divisions that give Q_i)
+            // lives on rank i mod G; both polynomials are then broadcast — every rank needs A_i again for the linearisation
+            // polynomial — and h1 is formed everywhere.
+            ZK_CUDA(ctx, cudaMemsetAsync(hx, 0, n * sizeof(fe_t), st));
+            HFr v_pow = HFr::one();
+            for (size_t i = 0; i < rot_sets.size(); ++i) {
+                fe_t* sum = set_sums + i * n;                             // A_i = sum_j y^j P_ij
+                if (!sh.mine((uint32_t)i)) continue;
+                HFr y_pow = HFr::one();
+                std::vector<HFr> rlow(rot_sets[i].pts.size(), HFr::zero());   // R_i = sum_j y^j r_ij
+                for (size_t j0 = 0; j0 < rot_sets[i].polys.size(); j0 += 16) {
+                    LinCombArgs la{};
+                    la.m = (uint32_t)std::min<size_t>(16, rot_sets[i].polys.size() - j0);
+                    for (uint32_t j = 0; j < la.m; ++j) {
+                        la.p[j] = rot_sets[i].polys[j0 + j];
+                        la.s[j] = to_dev(y_pow);
+                        for (size_t c = 0; c < low[i][j0 + j].size(); ++c) rlow[c] = rlow[c] + low[i][j0 + j][c] * y_pow;
+                        y_pow = y_pow * sy;
+                    }
+                    lincomb_kernel<<<nb(n), PK_THREADS, 0, st>>>(sum, la, n, j0 == 0 ? 1 : 0);
+                    ctx->launches++;
                 }
-                lincomb_kernel<<<nb(n), PK_THREADS, 0, st>>>(sum, la, n, j0 == 0 ? 1 : 0);
+                // N_i = A_i - R_i ; Q_i = N_i / prod (X - p)
+                ZK_CUDA(ctx, copy_rows(t0, sum, n));
+                LowCoeffs lc{}; lc.m = (uint32_t)rlow.size();
+                for (size_t c = 0; c < rlow.size(); ++c) lc.c[c] = to_dev(rlow[c]);
+                sub_low_kernel<<<1, 8, 0, st>>>(t0, lc);
                 ctx->launches++;
+                fe_t *src = t0, *dst = t1;
+                size_t len = n;
+                for (auto& pt : rot_sets[i].pts) {
+                    ZK_TRY(recurrence_run(ctx, src + 1, dst, len - 1, pt, nullptr));   // kate_division
+                    --len; std::swap(src, dst);
+                }
+                if (sh.on()) {                                            // keep Q_i (zero-padded to n) for the exchange
+                    ZK_CUDA(ctx, cudaMemsetAsync(set_quot + i * n, 0, n * sizeof(fe_t), st));
+                    ZK_CUDA(ctx, copy_rows(set_quot + i * n, src, len));
+                } else {
+                    axpy_kernel<<<nb(len), PK_THREADS, 0, st>>>(hx, src, to_dev(v_pow), len, 0);
+                    ctx->launches++;
+                    v_pow = v_pow * sv;
+                }
             }
-            // N_i = A_i - R_i ; Q_i = N_i / prod (X - p)
-            ZK_CUDA(ctx, copy_rows(t0, sum, n));
-            LowCoeffs lc{}; lc.m = (uint32_t)rlow.size();
-            for (size_t c = 0; c < rlow.size(); ++c) lc.c[c] = to_dev(rlow[c]);
-            sub_low_kernel<<<1, 8, 0, st>>>(t0, lc);
-            ctx->launches++;
-            fe_t *src = t0, *dst = t1;
-            size_t len = n;
-            for (auto& pt : rot_sets[i].pts) {
-                ZK_TRY(recurrence_run(ctx, src + 1, dst, len - 1, pt, nullptr));   // kate_division
-                --len; std::swap(src, dst);
-            }
-            if (sh.on()) {                                        // keep Q_i (zero-padded to n) for the exchange
-                ZK_CUDA(ctx, cudaMemsetAsync(set_quot + i * n, 0, n * sizeof(fe_t), st));
-                ZK_CUDA(ctx, copy_rows(set_quot + i * n, src, len));
-            } else {
-                axpy_kernel<<<nb(len), PK_THREADS, 0, st>>>(hx, src, to_dev(v_pow), len, 0);
-                ctx->launches++;
-                v_pow = v_pow * sv;
+            if (sh.on()) {
+                std::vector<CommPiece> pieces;
+                for (size_t i = 0; i < rot_sets.size(); ++i) {
+                    pieces.push_back({set_sums + i * n, n * sizeof(fe_t), sh.owner((uint32_t)i)});
+                    pieces.push_back({set_quot + i * n, n * sizeof(fe_t), sh.owner((uint32_t)i)});
+                }
+                ZK_TRY(share(pieces));
+                for (size_t i = 0; i < rot_sets.size(); ++i) {
+                    axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(hx, set_quot + i * n, to_dev(v_pow), n, 0);
+                    ctx->launches++;
+                    v_pow = v_pow * sv;
+                }
             }
         }
-        if (sh.on()) {
-            std::vector<CommPiece> pieces;
-            for (size_t i = 0; i < rot_sets.size(); ++i) {
-                pieces.push_back({set_sums + i * n, n * sizeof(fe_t), sh.owner((uint32_t)i)});
-                pieces.push_back({set_quot + i * n, n * sizeof(fe_t), sh.owner((uint32_t)i)});
-            }
-            rc = share(pieces);
-            if (rc != B200ZK_OK) return finish(rc);
-            for (size_t i = 0; i < rot_sets.size(); ++i) {
-                axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(hx, set_quot + i * n, to_dev(v_pow), n, 0);
-                ctx->launches++;
-                v_pow = v_pow * sv;
-            }
-        }
-    }
-    {
-        open_timer.reset();
         std::vector<HAffine> pt;
         ZK_TRY(commit_multi_range(pk, sh, {hx}, n, false, pt));
         tr.write_point(pt[0]);
         mark("shplonk_h1_commit");
-        open_timer.reset(new PhaseTimer(pk, PH_OPEN));
-    }
-    const HFr su = tr.squeeze_challenge();
-    {
-        auto vanish = [&](const std::vector<HFr>& roots) { HFr acc = HFr::one(); for (auto& r : roots) acc = acc * (su - r); return acc; };
-        HFr v_pow = HFr::one(), const_term = HFr::zero(), z0_diff = HFr::zero();
-        for (size_t i = 0; i < rot_sets.size(); ++i) {
-            std::vector<HFr> diffs;
-            for (auto& p : super_points)
-                if (std::find_if(rot_sets[i].pts.begin(), rot_sets[i].pts.end(), [&](const HFr& o) { return o == p; }) == rot_sets[i].pts.end()) diffs.push_back(p);
-            HFr z_i = vanish(diffs);
-            if (i == 0) z0_diff = z_i;
-            HFr y_pow = HFr::one(), c_i = HFr::zero();
-            for (size_t j = 0; j < rot_sets[i].polys.size(); ++j) { c_i = c_i + eval_small(low[i][j], su) * y_pow; y_pow = y_pow * sy; }
-            HFr coef = z_i * v_pow;
-            axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(lx, set_sums + i * n, to_dev(coef), n, i == 0 ? 1 : 0);
+        {
+            // the linearisation polynomial L(X) at u, divided by (X - u) into t0
+            PhaseTimer t(pk, PH_OPEN);
+            su = tr.squeeze_challenge();
+            auto vanish = [&](const std::vector<HFr>& roots) { HFr acc = HFr::one(); for (auto& r : roots) acc = acc * (su - r); return acc; };
+            HFr v_pow = HFr::one(), const_term = HFr::zero(), z0_diff = HFr::zero();
+            for (size_t i = 0; i < rot_sets.size(); ++i) {
+                std::vector<HFr> diffs;
+                for (auto& p : super_points)
+                    if (std::find_if(rot_sets[i].pts.begin(), rot_sets[i].pts.end(), [&](const HFr& o) { return o == p; }) == rot_sets[i].pts.end()) diffs.push_back(p);
+                HFr z_i = vanish(diffs);
+                if (i == 0) z0_diff = z_i;
+                HFr y_pow = HFr::one(), c_i = HFr::zero();
+                for (size_t j = 0; j < rot_sets[i].polys.size(); ++j) { c_i = c_i + eval_small(low[i][j], su) * y_pow; y_pow = y_pow * sy; }
+                HFr coef = z_i * v_pow;
+                axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(lx, set_sums + i * n, to_dev(coef), n, i == 0 ? 1 : 0);
+                ctx->launches++;
+                const_term = const_term + coef * c_i;
+                v_pow = v_pow * sv;
+            }
+            std::vector<HFr> sp(super_points.begin(), super_points.end());
+            HFr zt = vanish(sp);
+            axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(lx, hx, to_dev(zt.neg()), n, 0);
+            LowCoeffs lc{}; lc.m = 1; lc.c[0] = to_dev(const_term);
+            sub_low_kernel<<<1, 8, 0, st>>>(lx, lc);
+            ctx->launches += 2;
+            ZK_TRY(recurrence_run(ctx, lx + 1, t0, n - 1, su, nullptr));              // (L(X)) / (X - u)
+            scale_kernel<<<nb(n - 1), PK_THREADS, 0, st>>>(t0, to_dev(z0_diff.inv()), n - 1);
             ctx->launches++;
-            const_term = const_term + coef * c_i;
-            v_pow = v_pow * sv;
+            ZK_CUDA(ctx, cudaGetLastError());
         }
-        std::vector<HFr> sp(super_points.begin(), super_points.end());
-        HFr zt = vanish(sp);
-        axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(lx, hx, to_dev(zt.neg()), n, 0);
-        LowCoeffs lc{}; lc.m = 1; lc.c[0] = to_dev(const_term);
-        sub_low_kernel<<<1, 8, 0, st>>>(lx, lc);
-        ctx->launches += 2;
-        ZK_TRY(recurrence_run(ctx, lx + 1, t0, n - 1, su, nullptr));              // (L(X)) / (X - u)
-        scale_kernel<<<nb(n - 1), PK_THREADS, 0, st>>>(t0, to_dev(z0_diff.inv()), n - 1);
-        ctx->launches++;
-        ZK_CUDA(ctx, cudaGetLastError());
-        open_timer.reset();
-        std::vector<HAffine> pt;
         ZK_TRY(commit_multi_range(pk, sh, {t0}, n - 1, false, pt));
         tr.write_point(pt[0]);
+        return B200ZK_OK;
     }
+
+    // construct_intermediate_sets, and the low-degree equivalents of the polynomials of each rotation set
+    int32_t shplonk_sets() {
+        struct CommSet { const fe_t* poly; std::set<HFr, FrLess> pts; };
+        std::vector<CommSet> comm_sets;
+        for (auto& qy : queries) {
+            super_points.insert(qy.point);
+            auto it = std::find_if(comm_sets.begin(), comm_sets.end(), [&](const CommSet& c) { return c.poly == qy.poly; });
+            if (it == comm_sets.end()) { comm_sets.push_back({qy.poly, {}}); it = comm_sets.end() - 1; }
+            it->pts.insert(qy.point);
+        }
+        for (auto& c : comm_sets) {
+            std::vector<HFr> pts(c.pts.begin(), c.pts.end());
+            auto it = std::find_if(rot_sets.begin(), rot_sets.end(), [&](const RotSet& r) {
+                return r.pts.size() == pts.size() && std::equal(pts.begin(), pts.end(), r.pts.begin());
+            });
+            if (it == rot_sets.end()) { rot_sets.push_back({pts, {}}); it = rot_sets.end() - 1; }
+            if (std::find(it->polys.begin(), it->polys.end(), c.poly) == it->polys.end()) it->polys.push_back(c.poly);
+        }
+        if (rot_sets.size() > 8) return fail(ctx, B200ZK_EINVAL, "create_proof", "more than 8 rotation sets");
+        low.resize(rot_sets.size());
+        for (size_t i = 0; i < rot_sets.size(); ++i) {
+            const size_t m = rot_sets[i].pts.size();
+            if (m > 8) return fail(ctx, B200ZK_EINVAL, "create_proof", "rotation set with more than 8 points");
+            // the Lagrange basis of the set's points once (m field inversions), then every polynomial of the set is a
+            // combination of it: the same interpolant as arithmetic::lagrange_interpolate per polynomial, without an
+            // inversion per polynomial and point (they were ~2 ms of host time per proof at every size)
+            std::vector<std::vector<HFr>> basis(m);
+            for (size_t j = 0; j < m; ++j) { std::vector<HFr> unit(m, HFr::zero()); unit[j] = HFr::one(); basis[j] = lagrange_interpolate(rot_sets[i].pts, unit); }
+            for (const fe_t* poly : rot_sets[i].polys) {
+                std::vector<HFr> lowp(m, HFr::zero());
+                for (size_t j = 0; j < m; ++j) {
+                    HFr e = HFr::zero();
+                    ZK_TRY(opened(poly, rot_sets[i].pts[j], &e));
+                    for (size_t c = 0; c < m; ++c) lowp[c] = lowp[c] + basis[j][c] * e;
+                }
+                low[i].push_back(lowp);
+            }
+        }
+        return B200ZK_OK;
+    }
+};
+
+static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_device, const void* const* advice_host,
+                     const void* const* instance_columns, const uint32_t* instance_lens, const void* rng_wide, bool rng_on_device,
+                     const HFr& transcript_repr, std::vector<uint8_t>& proof_out) {
+    b200zk_ctx* ctx = pk->ctx;
+    for (uint32_t c = 0; c < pk->cs.I; ++c) if (instance_lens[c] && !instance_columns[c]) return fail(ctx, B200ZK_EINVAL, "create_proof", "null instance column");
+    if (!advice_on_device) for (uint32_t c = 0; c < pk->cs.A; ++c) if (!advice_host[c]) return fail(ctx, B200ZK_EINVAL, "create_proof", "null advice column");
+    cudaStreamSynchronize(ctx->stream2);                          // nothing of an earlier (failed) proof may still be writing the arena
+    if (pk->copy_stream) cudaStreamSynchronize(pk->copy_stream);
+    for (float& f : pk->phase_ms) f = 0;
+    pk->timer_used = 0;
+    ZK_CUDA(ctx, cudaSetDevice(ctx->device));
+    pk->trace.clear();
+    Prover p(pk, advice_on_device, rng_on_device);
+    if (p.sh.on()) ZK_TRY(p.sh.cm->set_window(ctx, pk->arena, pk->arena_bytes));
+    ZK_CUDA(ctx, cudaMemsetAsync(pk->d_err, 0, 4, ctx->stream));
+    ZK_TRY(p.carve());
+    ZK_TRY(p.instances(instance_columns, instance_lens, transcript_repr));
+    ZK_TRY(p.upload_rng(rng_wide, rng_on_device));
+    ZK_TRY(p.advice(d_advice_in, advice_host));
+    p.ch[EXF_THETA] = p.tr.squeeze_challenge();
+    ZK_TRY(p.lookup_permute());
+    p.ch[EXF_BETA] = p.tr.squeeze_challenge();
+    p.ch[EXF_GAMMA] = p.tr.squeeze_challenge();
+    ZK_TRY(p.lookup_cosets_early());
+    ZK_TRY(p.permutation_products());
+    ZK_TRY(p.lookup_products());
+    ZK_TRY(p.random_poly());
+    p.ch[EXF_Y] = p.tr.squeeze_challenge();
+    ZK_TRY(p.evaluate_h());
+    ZK_TRY(p.vanishing_construct());
+    p.x = p.tr.squeeze_challenge();
+    ZK_TRY(p.evaluations());
+    ZK_TRY(p.shplonk());
     phase_timers_collect(pk);
-    mark("end");
-    proof_out = tr.proof();
+    p.mark("end");
+    proof_out = p.tr.proof();
     return B200ZK_OK;
 }
 
@@ -1230,12 +1234,7 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
 // ------------------------------------------------------------------ C ABI
 extern "C" {
 
-size_t b200zk_pk_rng_draws(const b200zk_pk* pk) {
-    if (!pk) return 0;
-    const CsDesc& cs = pk->cs;
-    size_t bf = cs.bf;
-    return cs.A * (bf + 1) + cs.A + pk->L * (2 * (bf + 1) + 2) + pk->S * (bf + 1) + pk->L * (bf + 1) + pk->n + 1 + pk->q;
-}
+size_t b200zk_pk_rng_draws(const b200zk_pk* pk) { return pk ? DrawLayout(pk).total : 0; }
 
 size_t b200zk_pk_proof_size(const b200zk_pk* pk) {
     if (!pk) return 0;
