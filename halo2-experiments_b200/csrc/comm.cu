@@ -22,8 +22,7 @@ struct LocalState {
     int count = 0;
     uint64_t gen = 0;
     bool aborted = false;
-    std::vector<char*> win_base;
-    std::vector<size_t> win_bytes;
+    std::vector<std::vector<CommPiece>> published;       // per rank: the pieces of its current `share`, its own pointers
     std::vector<cudaEvent_t> ev_ready, ev_done;          // per rank, on that rank's device
     std::vector<std::vector<uint8_t>> host;              // per rank allgather_host slot
     // false when a rank aborted (now or earlier): the caller gives up instead of waiting for ever
@@ -48,24 +47,21 @@ struct LocalState {
 
 struct LocalComm : Comm {
     std::shared_ptr<LocalState> s;
-    int32_t set_window(b200zk_ctx*, void* base, size_t bytes) override {
-        s->win_base[rank] = (char*)base; s->win_bytes[rank] = bytes;
-        return B200ZK_OK;
-    }
+    // piece i is copied from the owner's own piece i: the ranks' arenas may be laid out differently (lk_early is decided
+    // per proving key)
     int32_t share(b200zk_ctx* ctx, const CommPiece* pieces, size_t count, cudaStream_t st) override {
         if (world == 1) return B200ZK_OK;
+        s->published[rank].assign(pieces, pieces + count);
         ZK_CUDA(ctx, cudaEventRecord(s->ev_ready[rank], st));
         if (!s->barrier()) return fail(ctx, B200ZK_ECUDA, "comm", "a peer rank failed");
-        char* mine = s->win_base[rank];
         std::vector<char> waited(world, 0);
         for (size_t i = 0; i < count; ++i) {
             const CommPiece& p = pieces[i];
             if (p.owner == rank || p.bytes == 0) continue;
-            size_t off = (char*)p.ptr - mine;
-            if ((char*)p.ptr < mine || off + p.bytes > s->win_bytes[rank] || off + p.bytes > s->win_bytes[p.owner])
-                return fail(ctx, B200ZK_EINVAL, "comm", "shared buffer outside the registered window");
+            const std::vector<CommPiece>& theirs = s->published[p.owner];
+            if (theirs.size() != count || theirs[i].bytes != p.bytes) return fail(ctx, B200ZK_EINVAL, "comm", "ranks disagree on the exchange");
             if (!waited[p.owner]) { ZK_CUDA(ctx, cudaStreamWaitEvent(st, s->ev_ready[p.owner], 0)); waited[p.owner] = 1; }
-            ZK_CUDA(ctx, cudaMemcpyAsync(p.ptr, s->win_base[p.owner] + off, p.bytes, cudaMemcpyDefault, st));
+            ZK_CUDA(ctx, cudaMemcpyAsync(p.ptr, theirs[i].ptr, p.bytes, cudaMemcpyDefault, st));
         }
         // nobody overwrites what it shared before every reader's copy has run
         ZK_CUDA(ctx, cudaEventRecord(s->ev_done[rank], st));
@@ -74,12 +70,14 @@ struct LocalComm : Comm {
         return B200ZK_OK;
     }
     int32_t allgather_host(b200zk_ctx* ctx, const void* mine, size_t bytes, void* all, cudaStream_t st) override {
-        if (bytes > COMM_HOST_MAX) return fail(ctx, B200ZK_EINVAL, "comm", "allgather_host payload too large");
         ZK_CUDA(ctx, cudaStreamSynchronize(st));
         if (world == 1) { memcpy(all, mine, bytes); return B200ZK_OK; }
-        memcpy(s->host[rank].data(), mine, bytes);
+        s->host[rank].assign((const uint8_t*)mine, (const uint8_t*)mine + bytes);
         if (!s->barrier()) return fail(ctx, B200ZK_ECUDA, "comm", "a peer rank failed");
-        for (int r = 0; r < world; ++r) memcpy((char*)all + (size_t)r * bytes, s->host[r].data(), bytes);
+        for (int r = 0; r < world; ++r) {
+            if (s->host[r].size() != bytes) return fail(ctx, B200ZK_EINVAL, "comm", "ranks disagree on the exchange");
+            memcpy((char*)all + (size_t)r * bytes, s->host[r].data(), bytes);
+        }
         if (!s->barrier()) return fail(ctx, B200ZK_ECUDA, "comm", "a peer rank failed");
         return B200ZK_OK;
     }
@@ -129,14 +127,14 @@ static NcclApi* nccl_api() {
 struct NcclComm : Comm {
     NcclApi* api = nullptr;
     ncclComm_t comm = nullptr;
-    char* d_stage = nullptr;            // world * COMM_HOST_MAX
+    static constexpr size_t HOST_MAX = 16 << 10;      // bytes per rank in one all-gather: larger payloads go in pieces
+    char* d_stage = nullptr;            // world * HOST_MAX
     char* h_stage = nullptr;            // pinned, same size
     ~NcclComm() override {
         if (comm && api) api->CommDestroy(comm);
         if (d_stage) cudaFree(d_stage);
         if (h_stage) cudaFreeHost(h_stage);
     }
-    int32_t set_window(b200zk_ctx*, void*, size_t) override { return B200ZK_OK; }
     int32_t share(b200zk_ctx* ctx, const CommPiece* pieces, size_t count, cudaStream_t st) override {
         if (world == 1 || count == 0) return B200ZK_OK;
         ZK_NCCL(ctx, api->GroupStart());
@@ -149,15 +147,16 @@ struct NcclComm : Comm {
         return B200ZK_OK;
     }
     int32_t allgather_host(b200zk_ctx* ctx, const void* mine, size_t bytes, void* all, cudaStream_t st) override {
-        if (bytes > COMM_HOST_MAX) return fail(ctx, B200ZK_EINVAL, "comm", "allgather_host payload too large");
-        if (world == 1) { ZK_CUDA(ctx, cudaStreamSynchronize(st)); memcpy(all, mine, bytes); return B200ZK_OK; }
-        const size_t slot = (bytes + 15) / 16 * 16;
-        memcpy(h_stage + (size_t)rank * slot, mine, bytes);
-        ZK_CUDA(ctx, cudaMemcpyAsync(d_stage + (size_t)rank * slot, h_stage + (size_t)rank * slot, slot, cudaMemcpyHostToDevice, st));
-        ZK_NCCL(ctx, api->AllGather(d_stage + (size_t)rank * slot, d_stage, slot, ncclUint8, comm, st));
-        ZK_CUDA(ctx, cudaMemcpyAsync(h_stage, d_stage, slot * world, cudaMemcpyDeviceToHost, st));
-        ZK_CUDA(ctx, cudaStreamSynchronize(st));
-        for (int r = 0; r < world; ++r) memcpy((char*)all + (size_t)r * bytes, h_stage + (size_t)r * slot, bytes);
+        if (world == 1 || bytes == 0) { ZK_CUDA(ctx, cudaStreamSynchronize(st)); memcpy(all, mine, bytes); return B200ZK_OK; }
+        for (size_t b0 = 0; b0 < bytes; b0 += HOST_MAX) {
+            const size_t m = std::min(bytes - b0, HOST_MAX), slot = (m + 15) / 16 * 16;
+            memcpy(h_stage + (size_t)rank * slot, (const char*)mine + b0, m);
+            ZK_CUDA(ctx, cudaMemcpyAsync(d_stage + (size_t)rank * slot, h_stage + (size_t)rank * slot, slot, cudaMemcpyHostToDevice, st));
+            ZK_NCCL(ctx, api->AllGather(d_stage + (size_t)rank * slot, d_stage, slot, ncclUint8, comm, st));
+            ZK_CUDA(ctx, cudaMemcpyAsync(h_stage, d_stage, slot * world, cudaMemcpyDeviceToHost, st));
+            ZK_CUDA(ctx, cudaStreamSynchronize(st));
+            for (int r = 0; r < world; ++r) memcpy((char*)all + (size_t)r * bytes + b0, h_stage + (size_t)r * slot, m);
+        }
         return B200ZK_OK;
     }
     void abort() override {
@@ -201,7 +200,7 @@ int32_t b200zk_ctx_comm_init(b200zk_ctx* ctx, uint32_t world, uint32_t rank, con
     memcpy(&id, id128, 128);
     ncclResult_t r = api->CommInitRank(&c->comm, (int)world, id, (int)rank);
     if (r != ncclSuccess) { c->comm = nullptr; delete c; return fail(ctx, B200ZK_ECUDA, "ncclCommInitRank", api->GetErrorString ? api->GetErrorString(r) : ""); }
-    if (cudaMalloc(&c->d_stage, (size_t)world * COMM_HOST_MAX) != cudaSuccess || cudaHostAlloc(&c->h_stage, (size_t)world * COMM_HOST_MAX, cudaHostAllocDefault) != cudaSuccess) {
+    if (cudaMalloc(&c->d_stage, (size_t)world * c->HOST_MAX) != cudaSuccess || cudaHostAlloc(&c->h_stage, (size_t)world * c->HOST_MAX, cudaHostAllocDefault) != cudaSuccess) {
         delete c;
         return fail(ctx, B200ZK_ENOMEM, "comm_init", "staging buffers");
     }
@@ -246,9 +245,9 @@ int32_t b200zk_group_create(const int32_t* devices, uint32_t n, b200zk_group** o
     g->state = std::make_shared<LocalState>();
     LocalState& s = *g->state;
     s.world = (int)n;
-    s.win_base.assign(n, nullptr); s.win_bytes.assign(n, 0);
+    s.published.resize(n);
     s.ev_ready.assign(n, nullptr); s.ev_done.assign(n, nullptr);
-    s.host.assign(n, std::vector<uint8_t>(COMM_HOST_MAX));
+    s.host.resize(n);
     g->ctxs.assign(n, nullptr);
     for (uint32_t r = 0; r < n; ++r) {
         int32_t rc = b200zk_ctx_create(devices[r], &g->ctxs[r]);

@@ -224,7 +224,7 @@ static size_t arena_need(const b200zk_pk* pk) {
     size_t draws = DrawLayout(pk).total;
     size_t elems = 2 * A * n + 2 * I * n + draws + 7 * L * n + S * n + S * ext + 3 * n   // columns, lookups, perm, tmp
                    + ext * (1 + A + I + 4 + 1)                                            // h, cosets, lookup cosets + table_value, h_L
-                   + n * (1 + 8 + 4 + 8 + 1);                                                 // h_poly, shplonk set sums, hx/lx/tmp, per-set quotients (sharded), linear gates
+                   + n * (1 + 8 + 4 + 8 + 1);                                                 // h_poly, shplonk set sums, hx/lx/tmp, per-set quotients, linear gates
     if (pk->lk_early) elems += 4 * L * (size_t)pk->lk_cosets_n * n + 64;
     return elems * sizeof(fe_t) + (size_t)draws * 64 + (64 << 10);
 }
@@ -381,49 +381,50 @@ struct Shard {
     // without a coset — 36.5 ms; weighting only the work before the challenge y (2 + 2 + 2 lookups on those ranks, 1 + 1 and the
     // sets on coset owners) 38.0 ms: the coset owners are the busy ranks from start to end, anything added to them costs.
     std::vector<int> lk_own, set_own;
-    std::vector<uint32_t> set_slot;                     // index of set s among its owner's sets
-    uint32_t set_slots = 0;
     void assign(uint32_t L, uint32_t S, uint32_t columns) {
         std::vector<uint64_t> load((size_t)G, 0);
         const uint64_t w_coset = columns + 30, w_lookup = 15, w_set = 8;
         for (int r = 0; r < G; ++r) load[r] = (uint64_t)(coset_lo(r + 1) - coset_lo(r)) * w_coset;
         auto lightest = [&]() { int b = 0; for (int r = 1; r < G; ++r) if (load[r] < load[b]) b = r; return b; };
-        lk_own.resize(L); set_own.resize(S); set_slot.resize(S);
+        lk_own.resize(L); set_own.resize(S);
         for (uint32_t l = 0; l < L; ++l) { int r = lightest(); lk_own[l] = r; load[r] += w_lookup; }
-        std::vector<uint32_t> used((size_t)G, 0);
-        for (uint32_t t = 0; t < S; ++t) { int r = lightest(); set_own[t] = r; set_slot[t] = used[r]++; load[r] += w_set; }
-        for (uint32_t u : used) set_slots = std::max(set_slots, u);
+        for (uint32_t t = 0; t < S; ++t) { int r = lightest(); set_own[t] = r; load[r] += w_set; }
     }
     int lk_owner(uint32_t l) const { return lk_own[l]; }
     bool lk_mine(uint32_t l) const { return lk_own[l] == R; }
     int set_owner(uint32_t t) const { return set_own[t]; }
     bool set_mine(uint32_t t) const { return set_own[t] == R; }
+    // Every rank fills the entries v[i] it owns (owner_of(i) == R); on return every rank holds all of them.  One host
+    // exchange (it synchronises the stream); nothing to do on one rank.
+    template <class T, class OwnerOf> int32_t gather(b200zk_pk* pk, std::vector<T>& v, OwnerOf owner_of) const {
+        if (G == 1) return B200ZK_OK;
+        std::vector<size_t> slot(v.size()), used((size_t)G, 0);
+        for (size_t i = 0; i < v.size(); ++i) slot[i] = used[owner_of(i)]++;
+        const size_t per = *std::max_element(used.begin(), used.end());
+        std::vector<T> mine(per), all(per * G);
+        for (size_t i = 0; i < v.size(); ++i) if (owner_of(i) == R) mine[slot[i]] = v[i];
+        PhaseTimer t(pk, PH_OTHER);
+        ZK_TRY(cm->allgather_host(pk->ctx, mine.data(), per * sizeof(T), all.data(), pk->ctx->stream));
+        for (size_t i = 0; i < v.size(); ++i) v[i] = all[(size_t)owner_of(i) * per + slot[i]];
+        return B200ZK_OK;
+    }
 };
 
 // Commitments to `cols`, column i computed by rank owners[i]; every rank ends up with all of them.  `flag` (optional)
-// is OR-ed over the ranks on the way (the lookup permutation's "input not in table" bit).
+// is OR-ed over the ranks in the same exchange (the lookup permutation's "input not in table" bit).
 static int32_t commit_multi_split(b200zk_pk* pk, const Shard& sh, const std::vector<const fe_t*>& cols, const std::vector<int>& owners,
                                   size_t len, bool lagrange, std::vector<HAffine>& outs, uint32_t* flag = nullptr) {
-    if (!sh.on()) return commit_multi_dev(pk, cols, len, lagrange, outs);
+    const size_t m = cols.size();
     std::vector<const fe_t*> my;
-    std::vector<size_t> slot_of(cols.size());
-    std::vector<size_t> used(sh.G, 0);
-    for (size_t i = 0; i < cols.size(); ++i) { slot_of[i] = used[owners[i]]++; if (owners[i] == sh.R) my.push_back(cols[i]); }
-    size_t slots = 0;
-    for (size_t u : used) slots = std::max(slots, u);
+    for (size_t i = 0; i < m; ++i) if (owners[i] == sh.R) my.push_back(cols[i]);
     std::vector<HAffine> mp;
     ZK_TRY(commit_multi_dev(pk, my, len, lagrange, mp));
-    const size_t bytes = slots * sizeof(HAffine) + 8;
-    std::vector<uint8_t> send(bytes, 0), recv(bytes * sh.G);
-    if (!mp.empty()) memcpy(send.data(), mp.data(), mp.size() * sizeof(HAffine));
-    if (flag) memcpy(send.data() + slots * sizeof(HAffine), flag, 4);
-    {
-        PhaseTimer t(pk, PH_OTHER);
-        ZK_TRY(sh.cm->allgather_host(pk->ctx, send.data(), bytes, recv.data(), pk->ctx->stream));
-    }
-    outs.resize(cols.size());
-    for (size_t i = 0; i < cols.size(); ++i) memcpy(&outs[i], recv.data() + (size_t)owners[i] * bytes + slot_of[i] * sizeof(HAffine), sizeof(HAffine));
-    if (flag) for (int r = 0; r < sh.G; ++r) { uint32_t f; memcpy(&f, recv.data() + (size_t)r * bytes + slots * sizeof(HAffine), 4); *flag |= f; }
+    outs.assign(m + sh.G, HAffine{});                                 // the points, then one entry per rank for its flag
+    for (size_t i = 0, j = 0; i < m; ++i) if (owners[i] == sh.R) outs[i] = mp[j++];
+    if (flag) memcpy(&outs[m + sh.R], flag, 4);
+    ZK_TRY(sh.gather(pk, outs, [&](size_t i) { return i < m ? owners[i] : (int)(i - m); }));
+    if (flag) for (int r = 0; r < sh.G; ++r) { uint32_t f; memcpy(&f, &outs[m + r], 4); *flag |= f; }
+    outs.resize(m);
     return B200ZK_OK;
 }
 
@@ -431,23 +432,18 @@ static int32_t commit_multi_split(b200zk_pk* pk, const Shard& sh, const std::vec
 // column, the G partial sums per column are exchanged (64 bytes each) and added on the host.
 static int32_t commit_multi_range(b200zk_pk* pk, const Shard& sh, const std::vector<const fe_t*>& cols, size_t len, bool lagrange,
                                   std::vector<HAffine>& outs) {
-    if (!sh.on()) return commit_multi_dev(pk, cols, len, lagrange, outs);
     const uint32_t m = (uint32_t)cols.size();
-    std::vector<HAffine> part(m);
+    std::vector<HAffine> part((size_t)m * sh.G);                      // entry (r, i): rank r's sum for column i
     {
         PhaseTimer t(pk, PH_MSM);
-        ZK_TRY(params_commit_range(pk->params, cols.data(), m, sh.pt_lo(len, sh.R), sh.pt_lo(len, sh.R + 1), lagrange, part.data()));
+        ZK_TRY(params_commit_range(pk->params, cols.data(), m, sh.pt_lo(len, sh.R), sh.pt_lo(len, sh.R + 1), lagrange, part.data() + (size_t)sh.R * m));
     }
-    std::vector<HAffine> all((size_t)m * sh.G);
-    {
-        PhaseTimer t(pk, PH_OTHER);
-        ZK_TRY(sh.cm->allgather_host(pk->ctx, part.data(), m * sizeof(HAffine), all.data(), pk->ctx->stream));
-    }
+    ZK_TRY(sh.gather(pk, part, [&](size_t i) { return (int)(i / m); }));
     outs.resize(m);
     for (uint32_t i = 0; i < m; ++i) {
         host::HXyzz acc = host::hx_identity();
         for (int r = 0; r < sh.G; ++r) {
-            const HAffine& a = all[(size_t)r * m + i];
+            const HAffine& a = part[(size_t)r * m + i];
             if (!(a.x.is_zero() && a.y.is_zero())) acc = host::hx_add(acc, host::hx_from_affine(a));
         }
         outs[i] = host::hx_to_affine(acc);
@@ -517,7 +513,7 @@ struct Prover {
         return cudaMemcpyAsync(dst, src, count * sizeof(fe_t), cudaMemcpyDeviceToDevice, st);
     }
     int32_t share(const std::vector<CommPiece>& pieces) {
-        if (!sh.on() || pieces.empty()) return B200ZK_OK;
+        if (sh.G == 1 || pieces.empty()) return B200ZK_OK;
         PhaseTimer t(pk, PH_OTHER);
         return sh.cm->share(ctx, pieces.data(), pieces.size(), ctx->stream);
     }
@@ -595,7 +591,7 @@ struct Prover {
         h_poly = ar.take<fe_t>(n);
         set_sums = ar.take<fe_t>(8 * n);
         fe_t* sh_tmp = ar.take<fe_t>(4 * n);                          // SHPLONK work space: hx lx t0 t1
-        set_quot = ar.take<fe_t>(8 * n);                              // sharded proof: Q_i of every rotation set, computed by its owner
+        set_quot = ar.take<fe_t>(8 * n);                              // SHPLONK: Q_i of every rotation set, computed by its owner
         if (!ar.ok) return fail(ctx, B200ZK_ENOMEM, "create_proof", "arena too small");
         hx = sh_tmp; lx = sh_tmp + n; t0 = sh_tmp + 2 * n; t1 = sh_tmp + 3 * n;
         pk->dbg.clear();
@@ -631,24 +627,18 @@ struct Prover {
         return B200ZK_OK;
     }
 
-    // randomness: Fr::random = from_u512 of the caller's 64-byte draws
+    // randomness: Fr::random = from_u512 of the caller's 64-byte draws.  This rank converts the draws [d0, d1): all of
+    // them, or with split_upload its 1/G of the stream, which the ranks then exchange.
     int32_t upload_rng(const void* rng_wide, bool rng_on_device) {
-        const size_t draws = dl.total;
-        if (split_upload) {
-            const size_t d0 = draws * (size_t)sh.R / sh.G, d1 = draws * (size_t)(sh.R + 1) / sh.G;
-            ZK_CUDA(ctx, cudaMemcpyAsync(wide + d0 * 16, (const char*)rng_wide + d0 * 64, (d1 - d0) * 64, cudaMemcpyHostToDevice, st));
-            if (d1 > d0) { from_u512_kernel<<<nb(d1 - d0), PK_THREADS, 0, st>>>(wide + d0 * 16, rnd + d0, d1 - d0); ctx->launches++; }
-            std::vector<CommPiece> pieces;
-            for (int r = 0; r < sh.G; ++r) {
-                const size_t a0 = draws * (size_t)r / sh.G, a1 = draws * (size_t)(r + 1) / sh.G;
-                pieces.push_back({rnd + a0, (a1 - a0) * sizeof(fe_t), r});
-            }
-            return share(pieces);
-        }
-        ZK_CUDA(ctx, cudaMemcpyAsync(wide, rng_wide, draws * 64, rng_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
-        from_u512_kernel<<<nb(draws), PK_THREADS, 0, st>>>(wide, rnd, draws);
-        ctx->launches++;
-        return B200ZK_OK;
+        const int parts = split_upload ? sh.G : 1, part = split_upload ? sh.R : 0;
+        auto part_lo = [&](int r) { return dl.total * (size_t)r / parts; };
+        const size_t d0 = part_lo(part), d1 = part_lo(part + 1);
+        ZK_CUDA(ctx, cudaMemcpyAsync(wide + d0 * 16, (const char*)rng_wide + d0 * 64, (d1 - d0) * 64,
+                                     rng_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+        if (d1 > d0) { from_u512_kernel<<<nb(d1 - d0), PK_THREADS, 0, st>>>(wide + d0 * 16, rnd + d0, d1 - d0); ctx->launches++; }
+        std::vector<CommPiece> pieces;
+        if (split_upload) for (int r = 0; r < parts; ++r) pieces.push_back({rnd + part_lo(r), (part_lo(r + 1) - part_lo(r)) * sizeof(fe_t), r});
+        return share(pieces);
     }
 
     // step 2: advice columns: blinding rows, blinds, commitments.
@@ -764,12 +754,12 @@ struct Prover {
     }
 
     // step 6: permutation argument.
-    // Upstream chains the sets through z_s[0] = z_{s-1}[n - (bf + 1)].  On one GPU that is a 32-byte read-back per
-    // set.  Sharded, set s lives on rank sh.set_owner(s): every rank runs its sets from z[0] = 1, the S totals
-    // t_s = z'_s[n - (bf + 1)] are exchanged, and set s is scaled by t_0 ... t_{s-1} — the same field elements.
+    // Upstream chains the sets through z_s[0] = z_{s-1}[n - (bf + 1)].  Here set s runs on rank sh.set_owner(s) from
+    // z[0] = 1, the S totals t_s = z'_s[n - (bf + 1)] are read back after one synchronisation (and gathered when
+    // sharded), and set s is scaled by t_0 ... t_{s-1} — the same field elements, without a host round trip per set.
     int32_t permutation_products() {
         const HFr beta = ch[EXF_BETA], gamma = ch[EXF_GAMMA];
-        HFr last_z = HFr::one(), deltaomega = HFr::one();
+        HFr deltaomega = HFr::one();
         for (uint32_t s = 0; s < S; ++s) {
             fe_t* z = perm_polys + (size_t)s * n;
             uint32_t c0 = s * pk->chunk, c1 = std::min<uint32_t>(c0 + pk->chunk, pk->P);
@@ -790,24 +780,15 @@ struct Prover {
                 ZK_TRY(batch_invert_run(ctx, tmp_n, n, 0));
                 perm_num_kernel<<<nb(n), PK_THREADS, 0, st>>>(pa);
                 ctx->launches++;
-                ZK_TRY(prefix_product_run(ctx, tmp_n, z, n, sh.on() ? HFr::one() : last_z));
+                ZK_TRY(prefix_product_run(ctx, tmp_n, z, n, HFr::one()));
             }
-            ZK_CUDA(ctx, cudaMemcpyAsync((fe_t*)ctx->pinned + (sh.on() ? sh.set_slot[s] : 0), z + (n - (bf + 1)), sizeof(fe_t), cudaMemcpyDeviceToHost, st));
-            if (!sh.on()) {
-                ZK_CUDA(ctx, copy_rows(z + (n - bf), rnd + dl.set_rows(s), bf));
-                ZK_CUDA(ctx, cudaStreamSynchronize(st));
-                last_z = HFr::from_limbs(ctx->pinned);
-            }
+            ZK_CUDA(ctx, cudaMemcpyAsync((fe_t*)ctx->pinned + s, z + (n - (bf + 1)), sizeof(fe_t), cudaMemcpyDeviceToHost, st));
         }
-        if (sh.on() && S) {
-            const size_t slots = sh.set_slots;
-            std::vector<HFr> mine_t(slots, HFr::one()), all_t(slots * sh.G);
+        if (S) {
+            std::vector<HFr> totals(S, HFr::one());
             ZK_CUDA(ctx, cudaStreamSynchronize(st));
-            for (uint32_t s = 0; s < S; ++s) if (sh.set_mine(s)) mine_t[sh.set_slot[s]] = HFr::from_limbs((const fe_t*)ctx->pinned + sh.set_slot[s]);
-            {
-                PhaseTimer t(pk, PH_OTHER);
-                ZK_TRY(sh.cm->allgather_host(ctx, mine_t.data(), slots * sizeof(HFr), all_t.data(), st));
-            }
+            for (uint32_t s = 0; s < S; ++s) if (sh.set_mine(s)) totals[s] = HFr::from_limbs((const fe_t*)ctx->pinned + s);
+            ZK_TRY(sh.gather(pk, totals, [&](size_t s) { return sh.set_owner((uint32_t)s); }));
             HFr carry = HFr::one();
             for (uint32_t s = 0; s < S; ++s) {
                 fe_t* z = perm_polys + (size_t)s * n;
@@ -815,11 +796,10 @@ struct Prover {
                     if (s) { scale_kernel<<<nb(n - bf), PK_THREADS, 0, st>>>(z, to_dev(carry), n - bf); ctx->launches++; }
                     ZK_CUDA(ctx, copy_rows(z + (n - bf), rnd + dl.set_rows(s), bf));
                 }
-                carry = carry * all_t[(size_t)sh.set_owner(s) * slots + sh.set_slot[s]];
+                carry = carry * totals[s];
             }
             mark("perm_products");
-        }
-        if (S) {                                                      // the S grand products: one batch of commitments, then coefficients and cosets
+            // the S grand products: one batch of commitments, then coefficients and cosets
             std::vector<const fe_t*> cols;
             std::vector<int> owners;
             for (uint32_t s = 0; s < S; ++s) { cols.push_back(perm_polys + (size_t)s * n); owners.push_back(sh.set_owner(s)); }
@@ -960,13 +940,14 @@ struct Prover {
             for (uint32_t j = cj0; j < cj1; ++j) ZK_TRY(intt_scaled(pk, h + j * n, 1, dom->ifft_divisor * pk->coset_t[j] * y_lk));
             // the linear gates' part of h, degree < n: coefficients in X / c_0
             if (lin_mine()) ZK_TRY(intt_scaled(pk, h_lin, 1, dom->ifft_divisor * pk->coset_t[0]));
-            if (sh.on()) {                                            // every coset's coefficients to every rank: q (+ CL) x n elements
-                std::vector<CommPiece> pieces;
-                for (uint32_t j = 0; j < pk->q; ++j) pieces.push_back({h + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
-                if (lk_split) for (uint32_t j = 0; j < CL; ++j) pieces.push_back({h_lk + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
-                if (pk->gate_prog[QC_LINEAR].second) pieces.push_back({h_lin, n * sizeof(fe_t), sh.coset_owner(0)});
-                ZK_TRY(sh.cm->share(ctx, pieces.data(), pieces.size(), st));
-            }
+        }
+        std::vector<CommPiece> pieces;                                // every coset's coefficients to every rank: q (+ CL) x n elements
+        for (uint32_t j = 0; j < pk->q; ++j) pieces.push_back({h + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
+        if (lk_split) for (uint32_t j = 0; j < CL; ++j) pieces.push_back({h_lk + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
+        if (pk->gate_prog[QC_LINEAR].second) pieces.push_back({h_lin, n * sizeof(fe_t), sh.coset_owner(0)});
+        ZK_TRY(share(pieces));
+        {
+            PhaseTimer t(pk, PH_NTT);
             if (lk_split) {
                 lookup_extrapolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h_lk, pk->coset_pow_inv, pk->lk_lambda, nullptr, CL, pk->q, n);
                 ctx->launches++;
@@ -987,12 +968,8 @@ struct Prover {
 
     // step 14: evaluations
     int32_t evaluations() {
-        PhaseTimer t(pk, PH_OPEN);
         const HFr x_next = rotate_omega(dom, x, 1), x_prev = rotate_omega(dom, x, -1), x_last = rotate_omega(dom, x, -(int)(bf + 1));
         const fe_t* random = rnd + dl.random;
-        // vanishing::evaluate: h_poly = sum_i (x^n)^i h_piece_i
-        fold_pieces_kernel<<<nb(n), PK_THREADS, 0, st>>>(lk_cosets, pk->q, n, to_dev(x.pow_u64(n)), h_poly);
-        ctx->launches++;
         // multiopen queries in upstream order (step 15); every evaluation the transcript gets is one of them, so their
         // distinct pairs are evaluated here in ONE batched launch pair
         for (size_t i = 0; i < cs.adv_q.size(); i += 2) queries.push_back({advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1])});
@@ -1008,23 +985,19 @@ struct Prover {
         queries.push_back({random, x});
         for (auto& qy : queries)
             if (std::none_of(pairs.begin(), pairs.end(), [&](const Query& p) { return p.poly == qy.poly && p.point == qy.point; })) pairs.push_back(qy);
-        std::vector<const fe_t*> bp; std::vector<HFr> bx;             // sharded: pair i on rank i mod G, 32 bytes each back to everybody
+        std::vector<const fe_t*> bp; std::vector<HFr> bx;             // pair i on rank i mod G, 32 bytes each back to everybody
         for (size_t i = 0; i < pairs.size(); ++i) if (sh.mine((uint32_t)i)) { bp.push_back(pairs[i].poly); bx.push_back(pairs[i].point); }
-        values.resize(pairs.size());
-        if (!sh.on()) {
-            ZK_TRY(eval_batch_run(ctx, bp.data(), bx.data(), bp.size(), n, values.data()));
-        } else {
-            const size_t slots = (pairs.size() + sh.G - 1) / sh.G;
-            std::vector<HFr> mv(slots, HFr::zero()), all(slots * sh.G);
+        std::vector<HFr> mv(bp.size());
+        {
+            PhaseTimer t(pk, PH_OPEN);
+            // vanishing::evaluate: h_poly = sum_i (x^n)^i h_piece_i
+            fold_pieces_kernel<<<nb(n), PK_THREADS, 0, st>>>(lk_cosets, pk->q, n, to_dev(x.pow_u64(n)), h_poly);
+            ctx->launches++;
             ZK_TRY(eval_batch_run(ctx, bp.data(), bx.data(), bp.size(), n, mv.data()));
-            for (size_t b0 = 0; b0 < slots; b0 += COMM_HOST_MAX / sizeof(HFr)) {       // in pieces the staging buffers hold
-                const size_t m = std::min(slots - b0, COMM_HOST_MAX / sizeof(HFr));
-                std::vector<HFr> part(m * sh.G);
-                ZK_TRY(sh.cm->allgather_host(ctx, mv.data() + b0, m * sizeof(HFr), part.data(), st));
-                for (int r = 0; r < sh.G; ++r) for (size_t i = 0; i < m; ++i) all[(size_t)r * slots + b0 + i] = part[(size_t)r * m + i];
-            }
-            for (size_t i = 0; i < pairs.size(); ++i) values[i] = all[(i % sh.G) * slots + i / sh.G];
         }
+        values.assign(pairs.size(), HFr::zero());
+        for (size_t i = 0, j = 0; i < pairs.size(); ++i) if (sh.mine((uint32_t)i)) values[i] = mv[j++];
+        ZK_TRY(sh.gather(pk, values, [&](size_t i) { return sh.owner((uint32_t)i); }));
         mark("evaluations");
         // the transcript's order: advice, fixed, random, sigma, permutation sets, lookups
         for (size_t i = 0; i < cs.adv_q.size(); i += 2) ZK_TRY(write_eval(advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1])));
@@ -1051,13 +1024,16 @@ struct Prover {
             sy = tr.squeeze_challenge();
             ZK_TRY(shplonk_sets());
             sv = tr.squeeze_challenge();
-            // h1 = sum_i v^i Q_i into hx.  Sharded: rotation set i (its linear combination A_i and the Kate divisions that give Q_i)
-            // lives on rank i mod G; both polynomials are then broadcast — every rank needs A_i again for the linearisation
-            // polynomial — and h1 is formed everywhere.
+            // h1 = sum_i v^i Q_i into hx.  Rotation set i (its linear combination A_i and the Kate divisions that give Q_i, of
+            // n - |points| coefficients) lives on rank i mod G; both polynomials are then broadcast — every rank needs A_i again
+            // for the linearisation polynomial — and h1 is formed everywhere.
             ZK_CUDA(ctx, cudaMemsetAsync(hx, 0, n * sizeof(fe_t), st));
-            HFr v_pow = HFr::one();
+            std::vector<CommPiece> pieces;
             for (size_t i = 0; i < rot_sets.size(); ++i) {
-                fe_t* sum = set_sums + i * n;                             // A_i = sum_j y^j P_ij
+                fe_t *sum = set_sums + i * n, *quot = set_quot + i * n;     // A_i = sum_j y^j P_ij, Q_i
+                const std::vector<HFr>& pts = rot_sets[i].pts;
+                pieces.push_back({sum, n * sizeof(fe_t), sh.owner((uint32_t)i)});
+                pieces.push_back({quot, (n - pts.size()) * sizeof(fe_t), sh.owner((uint32_t)i)});
                 if (!sh.mine((uint32_t)i)) continue;
                 HFr y_pow = HFr::one();
                 std::vector<HFr> rlow(rot_sets[i].pts.size(), HFr::zero());   // R_i = sum_j y^j r_ij
@@ -1079,33 +1055,20 @@ struct Prover {
                 for (size_t c = 0; c < rlow.size(); ++c) lc.c[c] = to_dev(rlow[c]);
                 sub_low_kernel<<<1, 8, 0, st>>>(t0, lc);
                 ctx->launches++;
-                fe_t *src = t0, *dst = t1;
-                size_t len = n;
-                for (auto& pt : rot_sets[i].pts) {
-                    ZK_TRY(recurrence_run(ctx, src + 1, dst, len - 1, pt, nullptr));   // kate_division
-                    --len; std::swap(src, dst);
-                }
-                if (sh.on()) {                                            // keep Q_i (zero-padded to n) for the exchange
-                    ZK_CUDA(ctx, cudaMemsetAsync(set_quot + i * n, 0, n * sizeof(fe_t), st));
-                    ZK_CUDA(ctx, copy_rows(set_quot + i * n, src, len));
-                } else {
-                    axpy_kernel<<<nb(len), PK_THREADS, 0, st>>>(hx, src, to_dev(v_pow), len, 0);
-                    ctx->launches++;
-                    v_pow = v_pow * sv;
+                fe_t* src = t0;                                           // kate_division by each point, the last one into Q_i
+                for (size_t k = 0; k < pts.size(); ++k) {
+                    fe_t* dst = k + 1 == pts.size() ? quot : src == t0 ? t1 : t0;
+                    ZK_TRY(recurrence_run(ctx, src + 1, dst, n - k - 1, pts[k], nullptr));
+                    src = dst;
                 }
             }
-            if (sh.on()) {
-                std::vector<CommPiece> pieces;
-                for (size_t i = 0; i < rot_sets.size(); ++i) {
-                    pieces.push_back({set_sums + i * n, n * sizeof(fe_t), sh.owner((uint32_t)i)});
-                    pieces.push_back({set_quot + i * n, n * sizeof(fe_t), sh.owner((uint32_t)i)});
-                }
-                ZK_TRY(share(pieces));
-                for (size_t i = 0; i < rot_sets.size(); ++i) {
-                    axpy_kernel<<<nb(n), PK_THREADS, 0, st>>>(hx, set_quot + i * n, to_dev(v_pow), n, 0);
-                    ctx->launches++;
-                    v_pow = v_pow * sv;
-                }
+            ZK_TRY(share(pieces));
+            HFr v_pow = HFr::one();
+            for (size_t i = 0; i < rot_sets.size(); ++i) {
+                const size_t len = n - rot_sets[i].pts.size();
+                axpy_kernel<<<nb(len), PK_THREADS, 0, st>>>(hx, set_quot + i * n, to_dev(v_pow), len, 0);
+                ctx->launches++;
+                v_pow = v_pow * sv;
             }
         }
         std::vector<HAffine> pt;
@@ -1203,7 +1166,6 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
     ZK_CUDA(ctx, cudaSetDevice(ctx->device));
     pk->trace.clear();
     Prover p(pk, advice_on_device, rng_on_device);
-    if (p.sh.on()) ZK_TRY(p.sh.cm->set_window(ctx, pk->arena, pk->arena_bytes));
     ZK_CUDA(ctx, cudaMemsetAsync(pk->d_err, 0, 4, ctx->stream));
     ZK_TRY(p.carve());
     ZK_TRY(p.instances(instance_columns, instance_lens, transcript_repr));

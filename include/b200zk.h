@@ -250,7 +250,7 @@ int32_t b200zk_pk_debug_buffer(b200zk_pk* pk, const char* name, void* host_out, 
  * other (= time spent in / waiting at the exchanges of a sharded proof) */
 int32_t b200zk_pk_last_phase_ms(const b200zk_pk* pk, float* out7);
 /* host wall clock (ms since the call) at the synchronisation points of the last create_proof, as
- * "label:ms;label:ms;...": advice_commits, lookup_permuted_commits, permutation_commits, lookup_product_commits,
+ * "label:ms;label:ms;...": advice_commits, lookup_permuted_commits, perm_products, permutation_commits, lookup_product_commits,
  * quotient_and_h_commits, evaluations, shplonk_h1_commit, end */
 int32_t b200zk_pk_last_trace(const b200zk_pk* pk, char* out, size_t cap);
 /* field multiplications evaluate_h executes per row: {custom gates, permutation terms, all lookups, q, lookup cosets}

@@ -34,11 +34,26 @@ def _single(zk, backend, orc, job, s):
     return proof, wide, inst, tr_repr
 
 
-def _sharded(zk, job, s, world, wide, inst, tr_repr, dev_inputs=False):
+def _proving_key(zk, params, job, lookup_early=None):
+    """A ProvingKey built with B200ZK_LOOKUP_EARLY set to `lookup_early` (None: the library decides by free memory)."""
+    if lookup_early is None:
+        return zk.ProvingKey(params, job.cs, job.k, job.fixed, job.map_col, job.map_row)
+    old = os.environ.get("B200ZK_LOOKUP_EARLY")
+    os.environ["B200ZK_LOOKUP_EARLY"] = lookup_early
+    try:
+        return zk.ProvingKey(params, job.cs, job.k, job.fixed, job.map_col, job.map_row)
+    finally:
+        if old is None:
+            del os.environ["B200ZK_LOOKUP_EARLY"]
+        else:
+            os.environ["B200ZK_LOOKUP_EARLY"] = old
+
+
+def _sharded(zk, job, s, world, wide, inst, tr_repr, dev_inputs=False, lookup_early=None):
     group = zk.Group(_devices(world))
     try:
         params = [zk.ParamsKZG.setup(b, job.k, s) for b in group.backends]
-        pks = [zk.ProvingKey(p, job.cs, job.k, job.fixed, job.map_col, job.map_row) for p in params]
+        pks = [_proving_key(zk, p, job, lookup_early[r] if lookup_early else None) for r, p in enumerate(params)]
         if dev_inputs:
             adv = np.concatenate([np.ascontiguousarray(a).reshape(-1, 4) for a in job.advice])
             d_adv = [b.to_device(adv) for b in group.backends]
@@ -67,6 +82,55 @@ def test_sharded_proof_equals_single_gpu(zk, backend, orc, name, k, worlds):
         got = _sharded(zk, job, s, world, wide, inst, tr_repr)
         assert got == want, f"world {world}: sharded proof differs from the single-GPU proof"
     assert _sharded(zk, job, s, worlds[0], wide, inst, tr_repr, dev_inputs=True) == want
+
+
+def _wide_job(zk, k, advice):
+    """`advice` columns of bits at 2^k rows, every one queried by a single boolean gate (q * sum_i a_i (1 - a_i)); the
+    instance column and advice column 0 in the permutation (two sets of one column)."""
+    synth = _synth(zk)
+    C = importlib.import_module(zk.__name__ + ".circuit")
+    n = 1 << k
+    rng = np.random.Generator(np.random.PCG64(11))
+    cs = C.ConstraintSystem(advice, 1, 1)
+    cs.enable_equality(C.ADVICE, 0)
+    cs.enable_equality(C.INSTANCE, 0)
+    poly = None
+    for c in range(advice):
+        a = cs.query_advice(c, 0)
+        poly = a * (1 - a) if poly is None else poly + a * (1 - a)
+    cs.create_gate([cs.query_fixed(0, 0) * poly])
+    job = synth.Job(cs, k)
+    usable = n - (cs.blinding_factors() + 1)
+    job.fixed = [synth.mont_from_small((np.arange(n) < usable).astype(np.int64))]
+    bits = rng.integers(0, 2, size=(advice, n), dtype=np.int64)
+    job.advice = [synth.mont_from_small(b) for b in bits]
+    job.instances = [[int(bits[0][r]) for r in range(2)]]
+    asm = C.PermutationAssembly(len(cs.permutation), n)
+    for r in range(2):
+        asm.copy(1, r, 0, r)                                             # instance[0][r] == a_0[r]
+    job.map_col, job.map_row = asm.map_col, asm.map_row
+    return job
+
+
+def test_sharded_wide_circuit(zk, backend, orc):
+    """512 advice columns over 2 ranks: 256 commitments (16 KiB) per rank in one host exchange; the proof equals the
+    single-GPU proof."""
+    job = _wide_job(zk, 6, 512)
+    s = orc.random_fr(1, 4321)[0]
+    want, wide, inst, tr_repr = _single(zk, backend, orc, job, s)
+    assert _sharded(zk, job, s, 2, wide, inst, tr_repr) == want
+
+
+def test_sharded_ranks_with_different_arenas(zk, backend, orc):
+    """Ranks whose proving keys differ in B200ZK_LOOKUP_EARLY carve different arenas (the early lookup cosets sit in the
+    middle of it); the exchanges copy from each owner's own buffers, so the proof is still the single-GPU proof."""
+    for name, k in (("small", 6), ("mst_shaped", 9)):
+        job = getattr(_synth(zk), name)(k)
+        s = orc.random_fr(1, 4321)[0]
+        want, wide, inst, tr_repr = _single(zk, backend, orc, job, s)
+        for early in (("1", "0"), ("0", "1", "0")):
+            got = _sharded(zk, job, s, len(early), wide, inst, tr_repr, lookup_early=early)
+            assert got == want, f"{name}: B200ZK_LOOKUP_EARLY per rank {early}"
 
 
 def test_sharded_real_merkle_sum_tree_k11(zk, backend, orc):
