@@ -8,7 +8,8 @@ pins at /root/reference/Cargo.toml:10 and calls from
     best_fft(a, omega, log_n)                     arithmetic.rs
     EvaluationDomain(j, k).lagrange_to_coeff / coeff_to_extended /
         extended_to_coeff / divide_by_vanishing_poly      poly/domain.rs
-    ParamsKZG.load / setup, .commit, .commit_lagrange      poly/kzg/commitment.rs
+    ParamsKZG.load / setup / downsize, .commit, .commit_lagrange      poly/kzg/commitment.rs
+    g_to_lagrange(backend, g, k)                  arithmetic.rs
 
 Arrays are numpy uint64, shape (n, 4) for Fr (Montgomery limbs, the memory layout of
 halo2curves' Fr), (n, 8) for G1Affine, (12,) for a G1 result.  Everything computes on
@@ -199,6 +200,11 @@ class Backend:
 
     def best_fft_dev(self, d_a, omega, log_n):
         self._check(lib().b200zk_fft_dev(self._ctx, d_a.ptr, _p(_fr(omega, 1)), ctypes.c_uint32(log_n)))
+
+    def g_to_lagrange_dev(self, d_g, k, d_out):
+        """arithmetic::g_to_lagrange on 2^k device-resident G1Affine points; d_out may be d_g."""
+        self._check(lib().b200zk_g_to_lagrange_dev(self._ctx, _p(d_g.ptr if d_g is not None else None), ctypes.c_uint32(k),
+                                                   _p(d_out.ptr if d_out is not None else None)))
 
     def eval_polynomial(self, poly, x):
         poly = _fr(poly)
@@ -512,6 +518,13 @@ class ParamsKZG:
         backend._check(lib().b200zk_params_setup(backend._ctx, ctypes.c_uint32(k), _p(_fr(s, 1)), ctypes.byref(h)))
         return cls(backend, h, k)
 
+    def downsize(self, k):
+        """ParamsKZG::downsize(k) as new params: g[..2^k] of these params and its Lagrange basis.  Unlike
+        upstream's in-place downsize, these params stay as they are, and so do proving keys built on them."""
+        h = ctypes.c_void_p()
+        self.backend._check(lib().b200zk_params_downsize(self._h, ctypes.c_uint32(k), ctypes.byref(h)))
+        return ParamsKZG(self.backend, h, k)
+
     def close(self):
         if self._h:
             lib().b200zk_params_destroy(self._h)
@@ -567,6 +580,17 @@ class ParamsKZG:
         out = np.zeros(12, dtype=np.uint64)
         self.backend._check(lib().b200zk_commit_dev(self._h, d_poly.ptr, ctypes.c_size_t(n), ctypes.c_int32(1 if lagrange else 0), _p(out)))
         return out
+
+
+def g_to_lagrange(backend, g, k):
+    """arithmetic::g_to_lagrange(g, k): the Lagrange basis n^-1 * FFT_{w^-1}(g) of n = 2^k G1Affine points,
+    as an (n, 8) array."""
+    g = np.ascontiguousarray(g, dtype=np.uint64).reshape(-1, 8)
+    if g.shape[0] != 1 << k:
+        raise B200zkError(f"g_to_lagrange: expected {1 << k} points, got {g.shape[0]}")
+    out = np.empty((1 << k, 8), dtype=np.uint64)
+    backend._check(lib().b200zk_g_to_lagrange(backend._ctx, _p(g), ctypes.c_uint32(k), _p(out)))
+    return out
 
 
 # ---- verifier side (host only: no Backend, no device) -------------------------------------------

@@ -695,6 +695,53 @@ int32_t b200zk_params_setup(b200zk_ctx* ctx, uint32_t k, const void* s_fr, b200z
     return B200ZK_OK;
 }
 
+int32_t b200zk_g_to_lagrange_dev(b200zk_ctx* ctx, const void* d_g, uint32_t k, void* d_out) {
+    if (!ctx) return B200ZK_EINVAL;
+    if (!d_g || !d_out) return fail(ctx, B200ZK_EINVAL, "g_to_lagrange", "null pointer");
+    if (k > host::FR_TWO_ADICITY) return fail(ctx, B200ZK_EINVAL, "g_to_lagrange", "k exceeds Fr two-adicity");
+    ZK_CUDA(ctx, cudaSetDevice(ctx->device));
+    ZK_TRY(g_to_lagrange_run(ctx, (const affine_t*)d_g, k, (affine_t*)d_out));
+    ZK_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B200ZK_OK;
+}
+
+int32_t b200zk_g_to_lagrange(b200zk_ctx* ctx, const void* g, uint32_t k, void* out) {
+    if (!ctx) return B200ZK_EINVAL;
+    if (!g || !out) return fail(ctx, B200ZK_EINVAL, "g_to_lagrange", "null pointer");
+    if (k > host::FR_TWO_ADICITY) return fail(ctx, B200ZK_EINVAL, "g_to_lagrange", "k exceeds Fr two-adicity");
+    ZK_CUDA(ctx, cudaSetDevice(ctx->device));
+    size_t bytes = sizeof(affine_t) << k;
+    ZK_TRY(ws_reserve(ctx, ctx->io_b, bytes));
+    ZK_CUDA(ctx, cudaMemcpyAsync(ctx->io_b.p, g, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    ZK_TRY(b200zk_g_to_lagrange_dev(ctx, ctx->io_b.p, k, ctx->io_b.p));
+    ZK_CUDA(ctx, cudaMemcpyAsync(out, ctx->io_b.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    ZK_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B200ZK_OK;
+}
+
+int32_t b200zk_params_downsize(const b200zk_params* src, uint32_t k, b200zk_params** out) {
+    if (!src) return B200ZK_EINVAL;
+    b200zk_ctx* ctx = src->ctx;
+    if (!out) return fail(ctx, B200ZK_EINVAL, "params_downsize", "null pointer");
+    if (k > src->k) return fail(ctx, B200ZK_EINVAL, "params_downsize", "k exceeds the source params' k");
+    ZK_CUDA(ctx, cudaSetDevice(ctx->device));
+    b200zk_params* p = new (std::nothrow) b200zk_params();
+    if (!p) return B200ZK_ENOMEM;
+    p->ctx = ctx; p->k = k; p->d_g = nullptr; p->d_g_lagrange = nullptr;
+    size_t bytes = sizeof(affine_t) << k;
+    int32_t rc = B200ZK_OK;
+    cudaError_t e = cudaMalloc(&p->d_g, bytes);
+    if (e == cudaSuccess) e = cudaMalloc(&p->d_g_lagrange, bytes);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_g, src->d_g, bytes, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e != cudaSuccess) rc = fail(ctx, B200ZK_ENOMEM, "params_downsize", cudaGetErrorString(e));
+    if (rc == B200ZK_OK) rc = g_to_lagrange_run(ctx, p->d_g, k, p->d_g_lagrange);
+    if (rc == B200ZK_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = fail(ctx, B200ZK_ECUDA, "params_downsize", "sync failed");
+    if (rc == B200ZK_OK) rc = params_build_tables(p);
+    if (rc != B200ZK_OK) { b200zk_params_destroy(p); return rc; }
+    *out = p;
+    return B200ZK_OK;
+}
+
 // ---- eval_polynomial / kate_division / BatchInvert / grand-product scan ---------------------
 int32_t b200zk_eval_polynomial_dev(b200zk_ctx* ctx, const void* d_poly, size_t len, const void* x_fr, void* out_fr_host) {
     if (!ctx || !x_fr || !out_fr_host || (len && !d_poly)) return B200ZK_EINVAL;

@@ -147,6 +147,8 @@ int32_t eval_batch_run(b200zk_ctx* ctx, const fe_t* const* h_polys, const host::
 // setup.cu -------------------------------------------------------------------
 // ParamsKZG::setup bases on the device: g[i] = [s^i]G, g_lagrange[i] = [l_i(s)]G
 int32_t params_setup_run(b200zk_ctx* ctx, uint32_t k, const host::HFr& s, affine_t* d_g, affine_t* d_g_lagrange);
+// arithmetic::g_to_lagrange: d_out[i] = n^-1 * sum_j w^(-ij) d_g[j] over n = 2^k points (d_out may alias d_g)
+int32_t g_to_lagrange_run(b200zk_ctx* ctx, const affine_t* d_g, uint32_t k, affine_t* d_out);
 
 // out[i] = base^i, i < n (two-level tables built on the device)
 int32_t powers_run(b200zk_ctx* ctx, const host::HFr& base, size_t n, fe_t* d_out);

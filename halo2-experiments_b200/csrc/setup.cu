@@ -5,8 +5,10 @@
 // 2n fixed-base scalar multiplications.  The generator table holds d * 256^w * G for
 // w < 32, d < 256 (8160 affine points, 510 KiB, L1/L2 resident), so each point costs at most
 // 32 mixed additions; results are normalised to affine with one batched Fq inversion.
+// The same normalisation finishes arithmetic::g_to_lagrange (ParamsKZG::downsize), a G1 NTT (g1_ntt.cuh).
 #include "context.hpp"
 #include "poly.cuh"
+#include "g1_ntt.cuh"
 
 namespace b200zk {
 
@@ -145,6 +147,59 @@ int32_t params_setup_run(b200zk_ctx* ctx, uint32_t k, const host::HFr& s, affine
         ctx->launches++;
         ZK_TRY(fixed_base(ctx, sc, n, xyzz, aux, d_g_lagrange));
     }
+    ZK_CUDA(ctx, cudaGetLastError());
+    return B200ZK_OK;
+}
+
+// ---- arithmetic::g_to_lagrange: G1 NTT with w^-1, then n^-1 (g1_ntt.cuh) -----------------------
+__global__ void __launch_bounds__(SETUP_THREADS) g1_ntt_load_kernel(const affine_t* g, size_t n, uint32_t k, xyzz_t* out) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    size_t r = k ? __brevll((unsigned long long)i) >> (64 - k) : 0;
+    out[i] = xyzz_from_affine(g[r]);
+}
+// one butterfly per thread (g1_ntt_stage_body)
+__global__ void __launch_bounds__(SETUP_THREADS) g1_ntt_stage_kernel(xyzz_t* a, const fe_t* tw, uint32_t s, uint32_t k) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < ((size_t)1 << (k - 1))) g1_ntt_stage_body(a, tw, t, s, k);
+}
+// p *= n^-1 (canonical); zzz copied to a dense array for the batched inversion
+__global__ void __launch_bounds__(SETUP_THREADS) g1_ntt_scale_kernel(xyzz_t* a, size_t n, const fe_t n_inv, fe_t* zzz) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    xyzz_t p = xyzz_mul(a[i], n_inv);
+    a[i] = p;
+    zzz[i] = p.zzz;
+}
+
+int32_t g_to_lagrange_run(b200zk_ctx* ctx, const affine_t* d_g, uint32_t k, affine_t* d_out) {
+    using host::HFr;
+    if (k > host::FR_TWO_ADICITY) return fail(ctx, B200ZK_EINVAL, "g_to_lagrange", "k exceeds Fr two-adicity");
+    const size_t n = (size_t)1 << k, half = n / 2;
+    // workspace: xyzz[n] | zzz[n] | tw[n/2]
+    ZK_TRY(ws_reserve(ctx, ctx->setup_ws, n * (sizeof(xyzz_t) + sizeof(fe_t)) + half * sizeof(fe_t)));
+    xyzz_t* xyzz = (xyzz_t*)ctx->setup_ws.p;
+    fe_t* zzz = (fe_t*)(xyzz + n);
+    fe_t* tw = zzz + n;
+    cudaStream_t st = ctx->stream;
+    HFr omega_inv = host::fr_root_of_unity();
+    for (uint32_t i = k; i < host::FR_TWO_ADICITY; ++i) omega_inv = omega_inv.sqr();
+    omega_inv = omega_inv.inv();
+    ZK_TRY(powers_run(ctx, omega_inv, half, tw));
+    g1_ntt_load_kernel<<<nblocks(n, SETUP_THREADS), SETUP_THREADS, 0, st>>>(d_g, n, k, xyzz);
+    ctx->launches++;
+    for (uint32_t s = 0; s < k; ++s) {
+        g1_ntt_stage_kernel<<<nblocks(half, SETUP_THREADS), SETUP_THREADS, 0, st>>>(xyzz, tw, s, k);
+        ctx->launches++;
+    }
+    uint64_t n_inv[4];
+    HFr::from_u64(n).inv().to_canonical(n_inv);
+    fe_t n_inv_d; memcpy(n_inv_d.l, n_inv, 32);
+    g1_ntt_scale_kernel<<<nblocks(n, SETUP_THREADS), SETUP_THREADS, 0, st>>>(xyzz, n, n_inv_d, zzz);
+    ctx->launches++;
+    ZK_TRY(batch_invert_run(ctx, zzz, n, 1));
+    setup_normalize_kernel<<<nblocks(n, SETUP_THREADS), SETUP_THREADS, 0, st>>>(xyzz, zzz, n, d_out);
+    ctx->launches++;
     ZK_CUDA(ctx, cudaGetLastError());
     return B200ZK_OK;
 }

@@ -150,6 +150,16 @@ int32_t b200zk_commit_dev(b200zk_params* p, const void* d_poly, size_t len, int3
  * amount to; d_polys: host array of `count` device pointers, out: count * 96 bytes on the host. */
 int32_t b200zk_commit_many_dev(b200zk_params* p, const void* const* d_polys, uint32_t count, size_t len, int32_t lagrange,
                                void* out_g1_host);
+/* arithmetic::g_to_lagrange(g, k): the Lagrange basis n^-1 · FFT_{ω^-1}(g) of n = 2^k G1Affine points
+ * (any points; identity = (0,0)), as G1Affine.  out may alias g.  k <= 28. */
+int32_t b200zk_g_to_lagrange(b200zk_ctx* ctx, const void* g, uint32_t k, void* out);
+int32_t b200zk_g_to_lagrange_dev(b200zk_ctx* ctx, const void* d_g, uint32_t k, void* d_out);
+/* ParamsKZG::downsize(k): new params on p's ctx holding g[..2^k] of p and its Lagrange basis, with
+ * the fixed-base tables built as params_load builds them.  p is not changed; k <= p's k.
+ * With k = p's k it derives the Lagrange basis of params loaded without one.
+ * Upstream's downsize truncates `&mut self` in place; returning a new handle instead keeps every
+ * proving key built on p valid.  Destroy both handles independently. */
+int32_t b200zk_params_downsize(const b200zk_params* p, uint32_t k, b200zk_params** out);
 
 /* ---- arithmetic::eval_polynomial / kate_division, ff::BatchInvert -----------------
  * eval_polynomial(poly, x) -> Fr (Horner);  kate_division(a, b): quotient of a(X) by

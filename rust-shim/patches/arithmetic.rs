@@ -25,3 +25,14 @@ pub fn best_fft<G: Group>(a: &mut [G], omega: G::Scalar, log_n: u32) {
     }
     best_fft_cpu(a, omega, log_n)
 }
+
+// g_to_lagrange (ParamsKZG::downsize): the G1 NTT and the n^-1 scaling on the device, normalised there as well
+pub fn g_to_lagrange<C: CurveAffine>(g_projective: Vec<C::Curve>, k: u32) -> Vec<C> {
+    if TypeId::of::<C>() == TypeId::of::<halo2curves::bn256::G1Affine>() {
+        let mut g = vec![C::identity(); g_projective.len()];
+        C::Curve::batch_normalize(&g_projective, &mut g);
+        let g = unsafe { &*(g.as_slice() as *const [C] as *const [halo2curves::bn256::G1Affine]) };
+        return gpu::g_to_lagrange(g, k).into_iter().map(|p| unsafe { std::mem::transmute_copy::<halo2curves::bn256::G1Affine, C>(&p) }).collect();
+    }
+    g_to_lagrange_cpu(g_projective, k)
+}

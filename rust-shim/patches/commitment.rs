@@ -1,5 +1,6 @@
 // halo2_proofs/src/poly/kzg/commitment.rs (tag v2023_02_02) — ParamsKZG<Bn256> keeps `g`, `g_lagrange` lazily (read back
-// with b200zk_params_read only if a caller asks for get_g()), plus a device handle `dev: b200zk_shim::Params`.
+// with b200zk_params_read only if a caller asks for get_g()), plus a device handle `dev: b200zk_shim::Params` and
+// `retired: Vec<b200zk_shim::Params>` (device params replaced by downsize, kept for the proving keys built on them).
 impl ParamsKZG<Bn256> {
     pub fn setup<R: RngCore>(k: u32, rng: R) -> Self {
         assert!(k <= Fr::S);
@@ -7,7 +8,18 @@ impl ParamsKZG<Bn256> {
         let dev = b200zk_shim::Params::setup(k, &s);               // g[i] = [s^i]G, g_lagrange[i] = [l_i(s)]G on the device
         let g2 = <Bn256 as Engine>::G2Affine::generator();
         let s_g2 = (g2 * s).into();                                // two G2 operations stay on the CPU
-        Self { k, n: 1 << k, dev, g2, s_g2, g: OnceCell::new(), g_lagrange: OnceCell::new() }
+        Self { k, n: 1 << k, dev, retired: Vec::new(), g2, s_g2, g: OnceCell::new(), g_lagrange: OnceCell::new() }
+    }
+    /// Keeps g[..2^k] and rebuilds g_lagrange with g_to_lagrange, both on the device.  The device params are replaced
+    /// by new ones; the old ones stay alive in `retired`, because device proving keys built before the call use them.
+    pub fn downsize(&mut self, k: u32) {
+        assert!(k <= self.k);
+        let small = self.dev.downsize(k);
+        self.retired.push(std::mem::replace(&mut self.dev, small));
+        self.k = k;
+        self.n = 1 << k;
+        self.g = OnceCell::new();
+        self.g_lagrange = OnceCell::new();
     }
 }
 impl<'params> Params<'params, G1Affine> for ParamsKZG<Bn256> {

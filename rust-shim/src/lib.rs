@@ -52,6 +52,14 @@ pub fn best_fft(a: &mut [Fr], omega: Fr, log_n: u32) {
     check(unsafe { sys::b200zk_fft(ctx(), a.as_mut_ptr() as *mut c_void, &omega as *const Fr as *const c_void, log_n) });
 }
 
+/// arithmetic::g_to_lagrange(g, k) for bn256: the Lagrange basis of 2^k G1Affine points
+pub fn g_to_lagrange(g: &[G1Affine], k: u32) -> Vec<G1Affine> {
+    assert_eq!(g.len(), 1usize << k);
+    let mut out = vec![G1Affine::default(); g.len()];
+    check(unsafe { sys::b200zk_g_to_lagrange(ctx(), g.as_ptr() as *const c_void, k, out.as_mut_ptr() as *mut c_void) });
+    out
+}
+
 /// ParamsKZG with the SRS resident on the device.
 pub struct Params(pub *mut sys::Params, pub u32);
 impl Params {
@@ -66,6 +74,14 @@ impl Params {
         assert_eq!(g_lagrange.len(), 1usize << k);
         let mut p = std::ptr::null_mut();
         check(unsafe { sys::b200zk_params_load(ctx(), k, g.as_ptr() as *const c_void, g_lagrange.as_ptr() as *const c_void, &mut p) });
+        Params(p, k)
+    }
+    /// ParamsKZG::downsize(k) as new params (g[..2^k] and its Lagrange basis); `self` and the proving keys built on
+    /// it stay valid, where upstream truncates in place.
+    pub fn downsize(&self, k: u32) -> Self {
+        assert!(k <= self.1);
+        let mut p = std::ptr::null_mut();
+        check(unsafe { sys::b200zk_params_downsize(self.0, k, &mut p) });
         Params(p, k)
     }
     pub fn commit(&self, poly: &[Fr]) -> G1 {
