@@ -402,6 +402,59 @@ class ProvingKey:
                                                            _p(out), ctypes.c_size_t(out.shape[0]), ctypes.byref(ln)))
         return bytes(out[: ln.value])
 
+    def reserve_lanes(self, want=0):
+        """Reserve up to `want` proof lanes for create_proofs (0 = the planner's default) and keep that request for later
+        batches; returns the number of lanes memory allowed (>= 1)."""
+        got = ctypes.c_uint32()
+        self.backend._check(lib().b200zk_pk_reserve_lanes(self._h, ctypes.c_uint32(want), ctypes.byref(got)))
+        return int(got.value)
+
+    def _batch(self, fn, count, advice_ptrs, instances_list, rng_ptrs, transcript_repr):
+        if len(instances_list) != count:
+            raise B200zkError("one instance list per proof")
+        keep, lens = [], []
+        for instances in instances_list:
+            if len(instances) != self.cs.num_instance:
+                raise B200zkError("instance column count does not match the constraint system")
+            k, _, ln = self._instances(instances)
+            keep += k
+            lens.append(ln)
+        lens = np.concatenate(lens) if lens else np.zeros(0, dtype=np.uint32)
+        out = np.zeros((count, self.proof_size), dtype=np.uint8)
+        status = np.zeros(count, dtype=np.int32)
+        rc = fn(self._h, ctypes.c_uint32(count), advice_ptrs, _ptr_array(keep), _p(lens), rng_ptrs, _p(_fr(transcript_repr, 1)),
+                _p(out), ctypes.c_size_t(out.nbytes), _p(status))
+        if rc != ESYNTH:
+            self.backend._check(rc)
+        return [None if status[i] == ESYNTH else bytes(out[i]) for i in range(count)]
+
+    def create_proofs(self, advice_list, instances_list, rng_list, transcript_repr):
+        """create_proof for several witnesses of this key at once, on concurrent lanes of its device: proof i is exactly
+        create_proof(advice_list[i], instances_list[i], rng_list[i], transcript_repr).  Returns a list of bytes, None
+        where the witness hit ConstraintSystemFailure (or its instances were too large)."""
+        count = len(advice_list)
+        if len(rng_list) != count:
+            raise B200zkError("one rng stream per proof")
+        adv = []
+        for advice in advice_list:
+            cols = [np.ascontiguousarray(a, dtype=np.uint64).reshape(self.n, 4) for a in advice]
+            if len(cols) != self.cs.num_advice:
+                raise B200zkError("advice column count does not match the constraint system")
+            adv += cols
+        wides = [np.ascontiguousarray(w, dtype=np.uint64).reshape(-1, 8) for w in rng_list]
+        if any(w.shape[0] < self.rng_draws for w in wides):
+            raise B200zkError(f"rng stream too short: need {self.rng_draws} draws")
+        return self._batch(lib().b200zk_create_proofs, count, _ptr_array(adv), instances_list, _ptr_array(wides), transcript_repr)
+
+    def create_proofs_dev(self, d_advice_list, instances_list, d_rng_list, transcript_repr):
+        """Same with proof i's A x n advice block and rng stream already in device memory (DeviceBuffers)."""
+        count = len(d_advice_list)
+        if len(d_rng_list) != count:
+            raise B200zkError("one rng stream per proof")
+        adv = (ctypes.c_void_p * max(count, 1))(*[d.ptr.value for d in d_advice_list])
+        rng = (ctypes.c_void_p * max(count, 1))(*[d.ptr.value for d in d_rng_list])
+        return self._batch(lib().b200zk_create_proofs_dev, count, adv, instances_list, rng, transcript_repr)
+
     def vk_commitments(self):
         """keygen_vk's commitments: (fixed (F, 8), sigma (P, 8)) G1Affine Montgomery limbs, computed on the device."""
         fixed = np.zeros((max(self.cs.num_fixed, 1), 8), dtype=np.uint64)

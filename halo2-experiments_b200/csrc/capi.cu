@@ -1,6 +1,7 @@
 // C ABI of libb200zk.so (declarations and reference mapping: include/b200zk.h).
 #include "context.hpp"
 #include "comm.hpp"
+#include <algorithm>
 #include <vector>
 #include <new>
 #include <cuda_profiler_api.h>
@@ -19,6 +20,7 @@ int32_t fail(b200zk_ctx* ctx, int32_t code, const char* what, const char* detail
 }
 
 int32_t ws_reserve(b200zk_ctx* ctx, Workspace& w, size_t bytes) {
+    w.used = std::max(w.used, bytes);
     if (bytes <= w.cap) return B200ZK_OK;
     if (w.p) { ZK_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); ZK_CUDA(ctx, cudaFree(w.p)); w.p = nullptr; w.cap = 0; }
     size_t cap = bytes + bytes / 8;
@@ -157,6 +159,12 @@ int32_t params_commit_range(b200zk_params* p, const fe_t* const* d_polys, uint32
     return msm_run_multi(ctx, cols.data(), ncols, (table ? table : bases) + lo, hi - lo, table ? &p->pre : nullptr, outs, nullptr);
 }
 
+int32_t params_sum_tables(b200zk_params* p) {
+    if (p->sum_table[0].empty()) ZK_TRY(build_sum_table(p, 0, p->d_g, p->d_g_pre));
+    if (p->d_g_lagrange && p->sum_table[1].empty()) ZK_TRY(build_sum_table(p, 1, p->d_g_lagrange, p->d_gl_pre));
+    return B200ZK_OK;
+}
+
 int32_t params_commit_run(b200zk_params* p, const fe_t* d_poly, size_t len, bool lagrange, host::HAffine* out) {
     return params_commit_multi(p, &d_poly, 1, len, lagrange, out);
 }
@@ -208,7 +216,7 @@ void b200zk_ctx_destroy(b200zk_ctx* ctx) {
     cudaStreamSynchronize(ctx->stream);
     if (ctx->comm && ctx->comm_owned) delete ctx->comm;
     ctx->comm = nullptr;
-    for (auto& kv : ctx->ntt_plans) { cudaFree(kv.second.roots); cudaFree(kv.second.tw_lo); cudaFree(kv.second.tw_hi); cudaFree(kv.second.tw_full); cudaFree(kv.second.roots_s); cudaFree(kv.second.tw_full_s); }
+    for (auto& kv : ctx->ntt_plans) if (!kv.second.borrowed) { cudaFree(kv.second.roots); cudaFree(kv.second.tw_lo); cudaFree(kv.second.tw_hi); cudaFree(kv.second.tw_full); cudaFree(kv.second.roots_s); cudaFree(kv.second.tw_full_s); }
     for (Workspace* w : {&ctx->ntt_scratch, &ctx->ntt_scratch2, &ctx->msm_ws, &ctx->msm_ws2, &ctx->lookup_ws, &ctx->io_a, &ctx->io_b, &ctx->poly_ws, &ctx->poly_heads, &ctx->poly_batch, &ctx->setup_ws}) if (w->p) cudaFree(w->p);
     if (ctx->d_gen_table) cudaFree(ctx->d_gen_table);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);

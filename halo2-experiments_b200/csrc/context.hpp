@@ -25,6 +25,7 @@ struct NttPlan {
     bool warp = false;          // passes run on ntt_warp_pass_kernel (ntt_warp.cuh)
     struct fe2_t* roots_s = nullptr;    // {plain value, floor(value * 2^256 / r)} forms of roots / tw_full for Field::mul_shoup
     struct fe2_t* tw_full_s = nullptr;  // (warp plans only; null = CIOS multiplications against the Montgomery tables)
+    bool borrowed = false;      // tables owned by another ctx on the same device (a proof lane's, prover.cu): not freed here
 };
 
 struct fe2_t;
@@ -32,6 +33,7 @@ struct fe2_t;
 struct Workspace {
     void* p = nullptr;
     size_t cap = 0;
+    size_t used = 0;            // largest request since create_proof last reset it (the size a proof lane reserves)
 };
 
 struct Comm;                    // comm.hpp: the exchanges of a proof sharded over several GPUs
@@ -137,6 +139,9 @@ int32_t params_commit_multi(b200zk_params* p, const fe_t* const* d_polys, uint32
 int32_t params_commit_range(b200zk_params* p, const fe_t* const* d_polys, uint32_t ncols, size_t lo, size_t hi, bool lagrange, host::HAffine* outs);
 // builds the fixed-base tables of a params object if memory allows (capi.cu)
 int32_t params_build_tables(b200zk_params* p);
+// builds the sum tables of both bases now (params_commit_multi otherwise builds them on first use), so that params views
+// on other ctxs can copy them and nothing writes them while proofs run concurrently (capi.cu)
+int32_t params_sum_tables(b200zk_params* p);
 
 // poly.cu --------------------------------------------------------------------
 int32_t batch_invert_run(b200zk_ctx* ctx, fe_t* d_a, size_t n, int field /* 0 Fr, 1 Fq */);

@@ -10,9 +10,11 @@
 #include "expr.cuh"
 #include "expr_share.hpp"
 #include "prover_kernels.cuh"
+#include "proof_lanes.hpp"
 #include "quot_plan.hpp"
 #include "transcript.hpp"
 #include <algorithm>
+#include <atomic>
 #include <map>
 #include <new>
 #include <set>
@@ -117,6 +119,47 @@ __global__ void __launch_bounds__(PK_THREADS) sigma_kernel(const uint32_t* mc, c
 }  // namespace b200zk
 
 // ------------------------------------------------------------------ proving key
+namespace b200zk {
+// the workspaces a proof grows (ws_reserve); a proof lane reserves them at the sizes a proof of the pk requested.
+// ntt_scratch2 is grown as well: SideStream swaps it with ntt_scratch for the side stream's transforms.
+using WsMember = Workspace b200zk_ctx::*;
+static const WsMember PROOF_WS[] = {&b200zk_ctx::ntt_scratch, &b200zk_ctx::ntt_scratch2, &b200zk_ctx::msm_ws, &b200zk_ctx::msm_ws2,
+                                    &b200zk_ctx::poly_ws, &b200zk_ctx::poly_heads, &b200zk_ctx::poly_batch, &b200zk_ctx::lookup_ws};
+constexpr size_t N_PROOF_WS = sizeof(PROOF_WS) / sizeof(PROOF_WS[0]);
+
+// The mutable state of one proof in flight.  The pk owns one, on its own ctx and params, which create_proof uses; every
+// further lane of b200zk_create_proofs owns another, on a ctx of its own (ProofLane).  Prover reads the pk as const and
+// writes only here.
+struct ProofState {
+    const b200zk_pk* pk = nullptr;
+    b200zk_ctx* ctx = nullptr;
+    b200zk_params* params = nullptr;
+    char* arena = nullptr;
+    size_t arena_bytes = 0;
+    uint32_t* d_err = nullptr;
+    const fe_t** d_ptrs = nullptr;                    // pointer tables, see PtrTab
+    fe_t* d_wts = nullptr;                            // the gates' weights y^gate_exp[i] for the current proof (ExprArgs::wts)
+    fe_t* h_wts = nullptr;                            // their pinned staging buffer
+    float phase_ms[7] = {0, 0, 0, 0, 0, 0, 0};
+    struct TimerEv { cudaEvent_t e0, e1; int slot; };
+    std::vector<TimerEv> timer_events;                // pool, grown on demand
+    size_t timer_used = 0;
+    // upload pipeline of create_proof: the advice columns arrive on copy_stream one by one (H2D from the caller's
+    // buffers, or D2D), col_events[c] marks column c complete (blinding rows included)
+    cudaStream_t copy_stream = nullptr;
+    cudaEvent_t ev_rnd = nullptr;
+    std::vector<cudaEvent_t> col_events;
+    std::map<std::string, std::pair<const void*, size_t>> dbg;     // buffers of the last proof, for b200zk_pk_debug_buffer
+    std::vector<std::pair<const char*, double>> trace;             // host time (ms since the call) at the proof's synchronisation points
+    bool proved = false;                              // a proof has completed here, and ws_need holds what it requested
+    size_t ws_need[N_PROOF_WS] = {};                  // the largest request of a completed proof to each of PROOF_WS
+    size_t owned_bytes = 0;                           // device bytes in `owned`
+    size_t alloc_limit = SIZE_MAX;                    // a lane's share of B200ZK_LANE_ALLOC_LIMIT (lane_create)
+    std::vector<void*> owned;                         // device allocations above
+};
+struct ProofLane;
+}  // namespace b200zk
+
 struct b200zk_pk {
     b200zk_ctx* ctx = nullptr;
     b200zk_params* params = nullptr;
@@ -143,27 +186,13 @@ struct b200zk_pk {
     uint32_t* d_prog = nullptr;                       // gate programs of the three classes (quot_plan.hpp) | lookup programs
     std::pair<uint32_t, uint32_t> gate_prog[3] = {};             // (off, len) into d_prog, by class
     std::vector<uint32_t> gate_exp;                   // gate i enters the accumulator of its class with weight y^gate_exp[i]
-    fe_t* d_wts = nullptr;                            // those weights for the current proof (ExprArgs::wts)
-    fe_t* h_wts = nullptr;                            // their pinned staging buffer
     std::vector<std::pair<uint32_t, uint32_t>> lookup_prog;     // (off, len) into d_prog
     fe_t* d_consts = nullptr;
     int32_t *d_q_adv = nullptr, *d_q_fix = nullptr, *d_q_inst = nullptr;
-    const fe_t** d_ptrs = nullptr;                    // pointer tables, see PtrTab
-    char* arena = nullptr;
-    size_t arena_bytes = 0;
-    uint32_t* d_err = nullptr;
-    float phase_ms[7] = {0, 0, 0, 0, 0, 0, 0};
-    struct TimerEv { cudaEvent_t e0, e1; int slot; };
-    std::vector<TimerEv> timer_events;                // pool, grown on demand
-    size_t timer_used = 0;
     std::vector<void*> owned;
-    // upload pipeline of create_proof: the advice columns arrive on copy_stream one by one (H2D from the caller's
-    // buffers, or D2D), col_events[c] marks column c complete (blinding rows included)
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_rnd = nullptr;
-    std::vector<cudaEvent_t> col_events;
-    std::map<std::string, std::pair<const void*, size_t>> dbg;     // buffers of the last proof, for b200zk_pk_debug_buffer
-    std::vector<std::pair<const char*, double>> trace;             // host time (ms since the call) at the proof's synchronisation points
+    ProofState ps;                                    // the state of create_proof (and of lane 0 of create_proofs)
+    std::vector<ProofLane*> lanes;                    // lanes 1, 2, ... of create_proofs
+    uint32_t lane_want = 0;                           // b200zk_pk_reserve_lanes' request (0 = the planner's default)
 };
 
 namespace b200zk {
@@ -229,28 +258,28 @@ static size_t arena_need(const b200zk_pk* pk) {
     return elems * sizeof(fe_t) + (size_t)draws * 64 + (64 << 10);
 }
 
-// Per-phase device time without extra synchronisation: event pairs from a pool owned by the pk are
+// Per-phase device time without extra synchronisation: event pairs from a pool owned by the proof state are
 // recorded around each phase and summed once at the end of the proof (phase_timers_collect).
 struct PhaseTimer {
-    b200zk_pk* pk; size_t idx;
-    PhaseTimer(b200zk_pk* pk_, int slot) : pk(pk_) {
-        idx = pk->timer_used++;
-        if (idx >= pk->timer_events.size()) {
+    ProofState* ps; size_t idx;
+    PhaseTimer(ProofState* ps_, int slot) : ps(ps_) {
+        idx = ps->timer_used++;
+        if (idx >= ps->timer_events.size()) {
             cudaEvent_t a, b; cudaEventCreate(&a); cudaEventCreate(&b);
-            pk->timer_events.push_back({a, b, slot});
+            ps->timer_events.push_back({a, b, slot});
         }
-        pk->timer_events[idx].slot = slot;
-        cudaEventRecord(pk->timer_events[idx].e0, pk->ctx->stream);
+        ps->timer_events[idx].slot = slot;
+        cudaEventRecord(ps->timer_events[idx].e0, ps->ctx->stream);
     }
-    ~PhaseTimer() { cudaEventRecord(pk->timer_events[idx].e1, pk->ctx->stream); }
+    ~PhaseTimer() { cudaEventRecord(ps->timer_events[idx].e1, ps->ctx->stream); }
 };
-static void phase_timers_collect(b200zk_pk* pk) {
-    cudaStreamSynchronize(pk->ctx->stream);
-    for (size_t i = 0; i < pk->timer_used; ++i) {
+static void phase_timers_collect(ProofState* ps) {
+    cudaStreamSynchronize(ps->ctx->stream);
+    for (size_t i = 0; i < ps->timer_used; ++i) {
         float ms = 0;
-        if (cudaEventElapsedTime(&ms, pk->timer_events[i].e0, pk->timer_events[i].e1) == cudaSuccess) pk->phase_ms[pk->timer_events[i].slot] += ms;
+        if (cudaEventElapsedTime(&ms, ps->timer_events[i].e0, ps->timer_events[i].e1) == cudaSuccess) ps->phase_ms[ps->timer_events[i].slot] += ms;
     }
-    pk->timer_used = 0;
+    ps->timer_used = 0;
 }
 enum { PH_MSM = 0, PH_NTT = 1, PH_QUOT = 2, PH_LOOKUP = 3, PH_PERM = 4, PH_OPEN = 5, PH_OTHER = 6 };
 
@@ -310,50 +339,53 @@ struct SideStream {
 };
 
 // several full-length columns in one batched launch sequence (msm_run_multi), <= 24 at a time
-static int32_t commit_multi_dev(b200zk_pk* pk, const std::vector<const fe_t*>& cols, size_t len, bool lagrange, std::vector<HAffine>& outs) {
-    PhaseTimer t(pk, PH_MSM);
+static int32_t commit_multi_dev(ProofState* ps, const std::vector<const fe_t*>& cols, size_t len, bool lagrange, std::vector<HAffine>& outs) {
+    PhaseTimer t(ps, PH_MSM);
     outs.resize(cols.size());
     for (size_t b = 0; b < cols.size(); b += 24) {
         uint32_t m = (uint32_t)std::min<size_t>(24, cols.size() - b);
-        ZK_TRY(params_commit_multi(pk->params, cols.data() + b, m, len, lagrange, outs.data() + b));
+        ZK_TRY(params_commit_multi(ps->params, cols.data() + b, m, len, lagrange, outs.data() + b));
     }
     return B200ZK_OK;
 }
 // inverse NTT of `count` contiguous size-n columns in place, every output multiplied by `factor`; more than one column
 // runs as one launch per pass
-static int32_t intt_scaled(b200zk_pk* pk, fe_t* d_a, uint32_t count, const HFr& factor) {
+static int32_t intt_scaled(ProofState* ps, fe_t* d_a, uint32_t count, const HFr& factor) {
+    const b200zk_pk* pk = ps->pk;
     HFr post[3] = {factor, factor, factor};
-    if (count == 1) return ntt_run(pk->ctx, d_a, pk->n, d_a, pk->dom->k, pk->dom->omega_inv, nullptr, post);
-    return ntt_rows_run(pk->ctx, d_a, count, pk->dom->omega_inv, pk->dom->k, post);
+    if (count == 1) return ntt_run(ps->ctx, d_a, pk->n, d_a, pk->dom->k, pk->dom->omega_inv, nullptr, post);
+    return ntt_rows_run(ps->ctx, d_a, count, pk->dom->omega_inv, pk->dom->k, post);
 }
 // `count` contiguous Lagrange columns to coefficient form
-static int32_t lagrange_to_coeff(b200zk_pk* pk, fe_t* d_a, uint32_t count = 1) {
-    PhaseTimer t(pk, PH_NTT);
-    pk->ctx->ntt_sparse_hint = true;
-    int32_t rc = intt_scaled(pk, d_a, count, pk->dom->ifft_divisor);
-    pk->ctx->ntt_sparse_hint = false;
+static int32_t lagrange_to_coeff(ProofState* ps, fe_t* d_a, uint32_t count = 1) {
+    PhaseTimer t(ps, PH_NTT);
+    ps->ctx->ntt_sparse_hint = true;
+    int32_t rc = intt_scaled(ps, d_a, count, ps->pk->dom->ifft_divisor);
+    ps->ctx->ntt_sparse_hint = false;
     return rc;
 }
 // coeff_to_extended restricted to the q cosets the quotient needs: coset j = size-n NTT of a_r * c_j^r
-static int32_t coeff_to_extended(b200zk_pk* pk, const fe_t* d_coeffs, fe_t* d_out, uint32_t cosets = 0) {
-    PhaseTimer t(pk, PH_NTT);
-    return ntt_run_cosets(pk->ctx, d_coeffs, d_out, pk->dom->k, pk->dom->omega, pk->coset_pow, cosets ? cosets : pk->q);
+static int32_t coeff_to_extended(ProofState* ps, const fe_t* d_coeffs, fe_t* d_out, uint32_t cosets = 0) {
+    const b200zk_pk* pk = ps->pk;
+    PhaseTimer t(ps, PH_NTT);
+    return ntt_run_cosets(ps->ctx, d_coeffs, d_out, pk->dom->k, pk->dom->omega, pk->coset_pow, cosets ? cosets : pk->q);
 }
 
-static ExprArgs expr_args(const b200zk_pk* pk, uint32_t prog_off, uint32_t prog_len, bool extended, uint32_t mode,
+static ExprArgs expr_args(const ProofState* ps, uint32_t prog_off, uint32_t prog_len, bool extended, uint32_t mode,
                           const HFr ch[4], fe_t* out0, fe_t* out1) {
+    const b200zk_pk* pk = ps->pk;
     PtrTab pt{pk->cs.F, pk->cs.A, pk->cs.I};
     ExprArgs a{};
     a.prog = pk->d_prog + prog_off; a.prog_len = prog_len; a.consts = pk->d_consts;
-    a.fixed = pk->d_ptrs + (extended ? pt.fixed_cosets() : pt.fixed_values());
-    a.advice = pk->d_ptrs + (extended ? pt.advice_cosets() : pt.advice_values());
-    a.instance = pk->d_ptrs + (extended ? pt.inst_cosets() : pt.inst_values());
+    a.fixed = ps->d_ptrs + (extended ? pt.fixed_cosets() : pt.fixed_values());
+    a.advice = ps->d_ptrs + (extended ? pt.advice_cosets() : pt.advice_values());
+    a.instance = ps->d_ptrs + (extended ? pt.inst_cosets() : pt.inst_values());
     a.q_fixed = pk->d_q_fix; a.q_advice = pk->d_q_adv; a.q_instance = pk->d_q_inst;
     a.log_size = pk->dom->k;
     a.rows = extended ? pk->ext_n : pk->n;
     a.rot_scale = 1u;
     for (int i = 0; i < 4; ++i) a.factors[i] = to_dev(ch[i]);
-    a.wts = pk->d_wts;
+    a.wts = ps->d_wts;
     a.mode = mode; a.out0 = out0; a.out1 = out1;
     return a;
 }
@@ -363,7 +395,7 @@ static ExprArgs expr_args(const b200zk_pk* pk, uint32_t prog_off, uint32_t prog_
 // `mine` test is true, every range is the whole, every exchange is a no-op.
 struct Shard {
     Comm* cm; int G, R; uint32_t q;
-    explicit Shard(b200zk_pk* pk) : cm(pk->ctx->comm), G(cm ? cm->world : 1), R(cm ? cm->rank : 0), q(pk->q) {}
+    explicit Shard(const ProofState* ps) : cm(ps->ctx->comm), G(cm ? cm->world : 1), R(cm ? cm->rank : 0), q(ps->pk->q) {}
     bool on() const { return G > 1; }
     // columns / lookups / permutation sets round-robin
     int owner(uint32_t i) const { return (int)(i % (uint32_t)G); }
@@ -396,15 +428,15 @@ struct Shard {
     bool set_mine(uint32_t t) const { return set_own[t] == R; }
     // Every rank fills the entries v[i] it owns (owner_of(i) == R); on return every rank holds all of them.  One host
     // exchange (it synchronises the stream); nothing to do on one rank.
-    template <class T, class OwnerOf> int32_t gather(b200zk_pk* pk, std::vector<T>& v, OwnerOf owner_of) const {
+    template <class T, class OwnerOf> int32_t gather(ProofState* ps, std::vector<T>& v, OwnerOf owner_of) const {
         if (G == 1) return B200ZK_OK;
         std::vector<size_t> slot(v.size()), used((size_t)G, 0);
         for (size_t i = 0; i < v.size(); ++i) slot[i] = used[owner_of(i)]++;
         const size_t per = *std::max_element(used.begin(), used.end());
         std::vector<T> mine(per), all(per * G);
         for (size_t i = 0; i < v.size(); ++i) if (owner_of(i) == R) mine[slot[i]] = v[i];
-        PhaseTimer t(pk, PH_OTHER);
-        ZK_TRY(cm->allgather_host(pk->ctx, mine.data(), per * sizeof(T), all.data(), pk->ctx->stream));
+        PhaseTimer t(ps, PH_OTHER);
+        ZK_TRY(cm->allgather_host(ps->ctx, mine.data(), per * sizeof(T), all.data(), ps->ctx->stream));
         for (size_t i = 0; i < v.size(); ++i) v[i] = all[(size_t)owner_of(i) * per + slot[i]];
         return B200ZK_OK;
     }
@@ -412,17 +444,17 @@ struct Shard {
 
 // Commitments to `cols`, column i computed by rank owners[i]; every rank ends up with all of them.  `flag` (optional)
 // is OR-ed over the ranks in the same exchange (the lookup permutation's "input not in table" bit).
-static int32_t commit_multi_split(b200zk_pk* pk, const Shard& sh, const std::vector<const fe_t*>& cols, const std::vector<int>& owners,
+static int32_t commit_multi_split(ProofState* ps, const Shard& sh, const std::vector<const fe_t*>& cols, const std::vector<int>& owners,
                                   size_t len, bool lagrange, std::vector<HAffine>& outs, uint32_t* flag = nullptr) {
     const size_t m = cols.size();
     std::vector<const fe_t*> my;
     for (size_t i = 0; i < m; ++i) if (owners[i] == sh.R) my.push_back(cols[i]);
     std::vector<HAffine> mp;
-    ZK_TRY(commit_multi_dev(pk, my, len, lagrange, mp));
+    ZK_TRY(commit_multi_dev(ps, my, len, lagrange, mp));
     outs.assign(m + sh.G, HAffine{});                                 // the points, then one entry per rank for its flag
     for (size_t i = 0, j = 0; i < m; ++i) if (owners[i] == sh.R) outs[i] = mp[j++];
     if (flag) memcpy(&outs[m + sh.R], flag, 4);
-    ZK_TRY(sh.gather(pk, outs, [&](size_t i) { return i < m ? owners[i] : (int)(i - m); }));
+    ZK_TRY(sh.gather(ps, outs, [&](size_t i) { return i < m ? owners[i] : (int)(i - m); }));
     if (flag) for (int r = 0; r < sh.G; ++r) { uint32_t f; memcpy(&f, &outs[m + r], 4); *flag |= f; }
     outs.resize(m);
     return B200ZK_OK;
@@ -430,15 +462,15 @@ static int32_t commit_multi_split(b200zk_pk* pk, const Shard& sh, const std::vec
 
 // Dense commitments sharded by point range (SURVEY.md 8(e)2): every rank multiplies its slice [lo, hi) of every
 // column, the G partial sums per column are exchanged (64 bytes each) and added on the host.
-static int32_t commit_multi_range(b200zk_pk* pk, const Shard& sh, const std::vector<const fe_t*>& cols, size_t len, bool lagrange,
+static int32_t commit_multi_range(ProofState* ps, const Shard& sh, const std::vector<const fe_t*>& cols, size_t len, bool lagrange,
                                   std::vector<HAffine>& outs) {
     const uint32_t m = (uint32_t)cols.size();
     std::vector<HAffine> part((size_t)m * sh.G);                      // entry (r, i): rank r's sum for column i
     {
-        PhaseTimer t(pk, PH_MSM);
-        ZK_TRY(params_commit_range(pk->params, cols.data(), m, sh.pt_lo(len, sh.R), sh.pt_lo(len, sh.R + 1), lagrange, part.data() + (size_t)sh.R * m));
+        PhaseTimer t(ps, PH_MSM);
+        ZK_TRY(params_commit_range(ps->params, cols.data(), m, sh.pt_lo(len, sh.R), sh.pt_lo(len, sh.R + 1), lagrange, part.data() + (size_t)sh.R * m));
     }
-    ZK_TRY(sh.gather(pk, part, [&](size_t i) { return (int)(i / m); }));
+    ZK_TRY(sh.gather(ps, part, [&](size_t i) { return (int)(i / m); }));
     outs.resize(m);
     for (uint32_t i = 0; i < m; ++i) {
         host::HXyzz acc = host::hx_identity();
@@ -455,12 +487,13 @@ static int32_t commit_multi_range(b200zk_pk* pk, const Shard& sh, const std::vec
 // One create_proof on this rank: the state its steps (SURVEY.md §3.2) share.  prove() calls the steps in order and squeezes
 // the challenges between them.
 struct Prover {
-    b200zk_pk* pk;
-    b200zk_ctx* ctx = pk->ctx;
+    ProofState* ps;
+    const b200zk_pk* pk = ps->pk;
+    b200zk_ctx* ctx = ps->ctx;
     const CsDesc& cs = pk->cs;
     const b200zk_domain* dom = pk->dom;
     cudaStream_t st = ctx->stream;
-    Shard sh{pk};
+    Shard sh{ps};
     const DrawLayout dl{pk};
     const bool advice_on_device;
     // Sharded proof from host buffers: the host -> device traffic is split as well — every rank uploads 1/G of the rng
@@ -493,7 +526,7 @@ struct Prover {
     std::vector<std::vector<std::vector<HFr>>> low;
     std::set<HFr, FrLess> super_points;
 
-    Prover(b200zk_pk* p, bool advice_dev, bool rng_dev) : pk(p), advice_on_device(advice_dev), split_upload(sh.on() && !advice_dev && !rng_dev) { sh.assign(L, S, A + I + S + 3 * L); }
+    Prover(ProofState* s, bool advice_dev, bool rng_dev) : ps(s), advice_on_device(advice_dev), split_upload(sh.on() && !advice_dev && !rng_dev) { sh.assign(L, S, A + I + S + 3 * L); }
 
     // arrays of lookup l: LK as listed at lk_bufs; LKC product z, permuted input a', permuted table s', table value
     // (all indexed by global coset row)
@@ -507,38 +540,38 @@ struct Prover {
     bool lin_mine() const { return pk->gate_prog[QC_LINEAR].second && sh.coset_owner(0) == sh.R; }
 
     void mark(const char* label) {                  // called right after a host synchronisation: where the wall clock of the proof goes
-        pk->trace.push_back({label, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count()});
+        ps->trace.push_back({label, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count()});
     }
     cudaError_t copy_rows(fe_t* dst, const fe_t* src, size_t count) {
         return cudaMemcpyAsync(dst, src, count * sizeof(fe_t), cudaMemcpyDeviceToDevice, st);
     }
     int32_t share(const std::vector<CommPiece>& pieces) {
         if (sh.G == 1 || pieces.empty()) return B200ZK_OK;
-        PhaseTimer t(pk, PH_OTHER);
+        PhaseTimer t(ps, PH_OTHER);
         return sh.cm->share(ctx, pieces.data(), pieces.size(), ctx->stream);
     }
     int32_t my_cosets(const fe_t* d_coeffs, fe_t* d_out, uint32_t j0, uint32_t j1) {     // cosets [j0, j1) of d_out
         if (j0 >= j1) return B200ZK_OK;
-        PhaseTimer t(pk, PH_NTT);
+        PhaseTimer t(ps, PH_NTT);
         return ntt_run_cosets(ctx, d_coeffs, d_out + (size_t)j0 * n, dom->k, dom->omega, pk->coset_pow + (size_t)j0 * n, j1 - j0);
     }
     // Lagrange commitments to `cols`, column i computed by rank owners[i], into the transcript
     int32_t commit_columns(const std::vector<const fe_t*>& cols, const std::vector<int>& owners, const char* label, uint32_t* flag = nullptr) {
         std::vector<HAffine> pts;
-        ZK_TRY(commit_multi_split(pk, sh, cols, owners, n, true, pts, flag));
+        ZK_TRY(commit_multi_split(ps, sh, cols, owners, n, true, pts, flag));
         for (auto& pt : pts) tr.write_point(pt);
         mark(label);
         return B200ZK_OK;
     }
     int32_t commit_random() {
         std::vector<HAffine> pts;
-        ZK_TRY(commit_multi_range(pk, sh, {rnd + dl.random}, n, false, pts));
+        ZK_TRY(commit_multi_range(ps, sh, {rnd + dl.random}, n, false, pts));
         random_pt = pts[0];
         return B200ZK_OK;
     }
     void lookup_table_value(uint32_t l) {            // (compressed input + beta)(compressed table + gamma) on this rank's lookup cosets
-        PhaseTimer t(pk, PH_QUOT);
-        ExprArgs ea = expr_args(pk, pk->lookup_prog[l].first, pk->lookup_prog[l].second, true, EXM_LOOKUP_PROD, ch, LKC(l, 3), nullptr);
+        PhaseTimer t(ps, PH_QUOT);
+        ExprArgs ea = expr_args(ps, pk->lookup_prog[l].first, pk->lookup_prog[l].second, true, EXM_LOOKUP_PROD, ch, LKC(l, 3), nullptr);
         ea.row0 = lk_row0; ea.rows = lk_rows;
         expr_kernel<<<nb(lk_rows), PK_THREADS, 0, ctx->stream>>>(ea);
         ctx->launches++;
@@ -546,12 +579,12 @@ struct Prover {
     // one gate program per class, each on its own rows (quot_plan.hpp); a class without gates starts its accumulator at 0
     int32_t gate_class(uint32_t cls, fe_t* out, uint32_t row0, uint32_t rows) {
         if (!rows) return B200ZK_OK;
-        PhaseTimer t(pk, PH_QUOT);
+        PhaseTimer t(ps, PH_QUOT);
         if (!pk->gate_prog[cls].second) {
             ZK_CUDA(ctx, cudaMemsetAsync(out + row0, 0, (size_t)rows * sizeof(fe_t), st));
             return B200ZK_OK;
         }
-        ExprArgs ea = expr_args(pk, pk->gate_prog[cls].first, pk->gate_prog[cls].second, true, EXM_ACC0, ch, out, nullptr);
+        ExprArgs ea = expr_args(ps, pk->gate_prog[cls].first, pk->gate_prog[cls].second, true, EXM_ACC0, ch, out, nullptr);
         ea.row0 = row0; ea.rows = rows;
         expr_kernel<<<nb(rows), PK_THREADS, 0, st>>>(ea);
         ctx->launches++;
@@ -570,7 +603,7 @@ struct Prover {
     }
 
     int32_t carve() {
-        Arena ar{pk->arena, pk->arena_bytes};
+        Arena ar{ps->arena, ps->arena_bytes};
         advice_values = ar.take<fe_t>(A * n);
         advice_polys = ar.take<fe_t>(A * n);
         inst_values = ar.take<fe_t>(I * n);
@@ -594,11 +627,11 @@ struct Prover {
         set_quot = ar.take<fe_t>(8 * n);                              // SHPLONK: Q_i of every rotation set, computed by its owner
         if (!ar.ok) return fail(ctx, B200ZK_ENOMEM, "create_proof", "arena too small");
         hx = sh_tmp; lx = sh_tmp + n; t0 = sh_tmp + 2 * n; t1 = sh_tmp + 3 * n;
-        pk->dbg.clear();
-        pk->dbg["advice_values"] = {advice_values, A * n}; pk->dbg["advice_polys"] = {advice_polys, A * n};
-        pk->dbg["lookups"] = {lk_bufs, 7 * (size_t)L * n}; pk->dbg["perm_polys"] = {perm_polys, (size_t)S * n};
-        pk->dbg["h"] = {h, ext}; pk->dbg["rnd"] = {rnd, dl.total}; pk->dbg["tmp_n"] = {tmp_n, 3 * n};
-        pk->dbg["advice_cosets"] = {advice_cosets, A * ext}; pk->dbg["h_poly"] = {h_poly, n};
+        ps->dbg.clear();
+        ps->dbg["advice_values"] = {advice_values, A * n}; ps->dbg["advice_polys"] = {advice_polys, A * n};
+        ps->dbg["lookups"] = {lk_bufs, 7 * (size_t)L * n}; ps->dbg["perm_polys"] = {perm_polys, (size_t)S * n};
+        ps->dbg["h"] = {h, ext}; ps->dbg["rnd"] = {rnd, dl.total}; ps->dbg["tmp_n"] = {tmp_n, 3 * n};
+        ps->dbg["advice_cosets"] = {advice_cosets, A * ext}; ps->dbg["h_poly"] = {h_poly, n};
 
         // pointer tables for this proof
         PtrTab pt{F, A, I};
@@ -606,7 +639,7 @@ struct Prover {
         for (uint32_t c = 0; c < F; ++c) { tab[pt.fixed_values() + c] = pk->fixed_values + (size_t)c * n; tab[pt.fixed_cosets() + c] = pk->fixed_cosets + (size_t)c * ext; }
         for (uint32_t c = 0; c < A; ++c) { tab[pt.advice_values() + c] = advice_values + (size_t)c * n; tab[pt.advice_cosets() + c] = advice_cosets + (size_t)c * ext; }
         for (uint32_t c = 0; c < I; ++c) { tab[pt.inst_values() + c] = inst_values + (size_t)c * n; tab[pt.inst_cosets() + c] = inst_cosets + (size_t)c * ext; }
-        ZK_CUDA(ctx, cudaMemcpyAsync(pk->d_ptrs, tab.data(), tab.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
+        ZK_CUDA(ctx, cudaMemcpyAsync(ps->d_ptrs, tab.data(), tab.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
         ZK_CUDA(ctx, cudaStreamSynchronize(st));
         return B200ZK_OK;
     }
@@ -623,7 +656,7 @@ struct Prover {
             if (len) ZK_CUDA(ctx, cudaMemcpyAsync(inst_values + (size_t)c * n, v, (size_t)len * sizeof(fe_t), cudaMemcpyHostToDevice, st));
         }
         ZK_CUDA(ctx, cudaMemcpyAsync(inst_polys, inst_values, I * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, st));
-        for (uint32_t c = 0; c < I; ++c) ZK_TRY(lagrange_to_coeff(pk, inst_polys + (size_t)c * n));
+        for (uint32_t c = 0; c < I; ++c) ZK_TRY(lagrange_to_coeff(ps, inst_polys + (size_t)c * n));
         return B200ZK_OK;
     }
 
@@ -649,30 +682,30 @@ struct Prover {
     // the host — on the main stream the commitment to the vanishing argument's random polynomial (step 8), which
     // depends on the rng stream only.  The main stream then waits for the last column and commits all of them.
     int32_t advice(const fe_t* d_advice_in, const void* const* advice_host) {
-        if (!pk->copy_stream) {
-            ZK_CUDA(ctx, cudaStreamCreateWithFlags(&pk->copy_stream, cudaStreamNonBlocking));
-            ZK_CUDA(ctx, cudaEventCreateWithFlags(&pk->ev_rnd, cudaEventDisableTiming));
+        if (!ps->copy_stream) {
+            ZK_CUDA(ctx, cudaStreamCreateWithFlags(&ps->copy_stream, cudaStreamNonBlocking));
+            ZK_CUDA(ctx, cudaEventCreateWithFlags(&ps->ev_rnd, cudaEventDisableTiming));
         }
-        while (pk->col_events.size() < A) {
+        while (ps->col_events.size() < A) {
             cudaEvent_t e;
             ZK_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            pk->col_events.push_back(e);
+            ps->col_events.push_back(e);
         }
-        ZK_CUDA(ctx, cudaEventRecord(pk->ev_rnd, st));
-        ZK_CUDA(ctx, cudaStreamWaitEvent(pk->copy_stream, pk->ev_rnd, 0));      // rnd (and the arena's previous users on st) first
+        ZK_CUDA(ctx, cudaEventRecord(ps->ev_rnd, st));
+        ZK_CUDA(ctx, cudaStreamWaitEvent(ps->copy_stream, ps->ev_rnd, 0));      // rnd (and the arena's previous users on st) first
         for (uint32_t c = 0; c < A; ++c) {
             fe_t* col = advice_values + (size_t)c * n;
             if (split_upload && !sh.mine(c)) continue;                // arrives from its owner below
-            if (advice_on_device) ZK_CUDA(ctx, cudaMemcpyAsync(col, d_advice_in + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, pk->copy_stream));
-            else ZK_CUDA(ctx, cudaMemcpyAsync(col, advice_host[c], n * sizeof(fe_t), cudaMemcpyHostToDevice, pk->copy_stream));
-            ZK_CUDA(ctx, cudaMemcpyAsync(col + usable, rnd + dl.advice_rows(c), (bf + 1) * sizeof(fe_t), cudaMemcpyDeviceToDevice, pk->copy_stream));
-            ZK_CUDA(ctx, cudaEventRecord(pk->col_events[c], pk->copy_stream));
+            if (advice_on_device) ZK_CUDA(ctx, cudaMemcpyAsync(col, d_advice_in + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ps->copy_stream));
+            else ZK_CUDA(ctx, cudaMemcpyAsync(col, advice_host[c], n * sizeof(fe_t), cudaMemcpyHostToDevice, ps->copy_stream));
+            ZK_CUDA(ctx, cudaMemcpyAsync(col + usable, rnd + dl.advice_rows(c), (bf + 1) * sizeof(fe_t), cudaMemcpyDeviceToDevice, ps->copy_stream));
+            ZK_CUDA(ctx, cudaEventRecord(ps->col_events[c], ps->copy_stream));
         }
         if (split_upload) {                                           // random-polynomial commit under the upload, then the column exchange
             ZK_TRY(commit_random());
             std::vector<CommPiece> pieces;
             for (uint32_t c = 0; c < A; ++c) {
-                if (sh.mine(c)) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[c], 0));
+                if (sh.mine(c)) ZK_CUDA(ctx, cudaStreamWaitEvent(st, ps->col_events[c], 0));
                 pieces.push_back({advice_values + (size_t)c * n, n * sizeof(fe_t), sh.owner(c)});
             }
             ZK_TRY(share(pieces));
@@ -683,15 +716,15 @@ struct Prover {
             // (columns from the host keep the per-column pipeline under the upload)
             const bool batch_intt = advice_on_device && A > 1 && ((uint64_t)A << dom->k) <= 0xFFFFFFFFull;
             if (batch_intt) {
-                ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, pk->col_events[A - 1], 0));
+                ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ps->col_events[A - 1], 0));
                 ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys, advice_values, (size_t)A * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
-                ZK_TRY(lagrange_to_coeff(pk, advice_polys, A));
+                ZK_TRY(lagrange_to_coeff(ps, advice_polys, A));
             }
             for (uint32_t c = 0; c < A; ++c) {
                 if (!batch_intt) {
-                    if (!split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, pk->col_events[c], 0));
+                    if (!split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ps->col_events[c], 0));
                     ZK_CUDA(ctx, cudaMemcpyAsync(advice_polys + (size_t)c * n, advice_values + (size_t)c * n, n * sizeof(fe_t), cudaMemcpyDeviceToDevice, ctx->stream));
-                    ZK_TRY(lagrange_to_coeff(pk, advice_polys + (size_t)c * n));
+                    ZK_TRY(lagrange_to_coeff(ps, advice_polys + (size_t)c * n));
                 }
                 ZK_TRY(my_cosets(advice_polys + (size_t)c * n, advice_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.adv_need[c])));
             }
@@ -699,7 +732,7 @@ struct Prover {
             for (uint32_t c = 0; c < I; ++c) ZK_TRY(my_cosets(inst_polys + (size_t)c * n, inst_cosets + (size_t)c * ext, cj0, std::min(cj1, pk->plan.inst_need[c])));
         }
         if (!advice_on_device && !split_upload) ZK_TRY(commit_random());
-        if (A && !split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(st, pk->col_events[A - 1], 0));
+        if (A && !split_upload) ZK_CUDA(ctx, cudaStreamWaitEvent(st, ps->col_events[A - 1], 0));
         std::vector<const fe_t*> cols;
         std::vector<int> owners;
         for (uint32_t c = 0; c < A; ++c) { cols.push_back(advice_values + (size_t)c * n); owners.push_back(sh.owner(c)); }
@@ -712,20 +745,20 @@ struct Prover {
             if (!sh.lk_mine(l)) continue;
             fe_t *cin = LK(l, 0), *ctab = LK(l, 1), *pin = LK(l, 2), *ptab = LK(l, 3), *pin_poly = LK(l, 4), *ptab_poly = LK(l, 5);
             {
-                PhaseTimer t(pk, PH_LOOKUP);
-                ExprArgs ea = expr_args(pk, pk->lookup_prog[l].first, pk->lookup_prog[l].second, false, EXM_ACC01, ch, cin, ctab);
+                PhaseTimer t(ps, PH_LOOKUP);
+                ExprArgs ea = expr_args(ps, pk->lookup_prog[l].first, pk->lookup_prog[l].second, false, EXM_ACC01, ch, cin, ctab);
                 expr_kernel<<<nb(n), PK_THREADS, 0, st>>>(ea);
                 ctx->launches++;
-                ZK_TRY(lookup_permute_run(ctx, cin, ctab, (uint32_t)usable, pin, ptab, pk->d_err));
+                ZK_TRY(lookup_permute_run(ctx, cin, ctab, (uint32_t)usable, pin, ptab, ps->d_err));
             }
             ZK_CUDA(ctx, copy_rows(pin + usable, rnd + dl.lookup_input_rows(l), bf + 1));
             ZK_CUDA(ctx, copy_rows(ptab + usable, rnd + dl.lookup_table_rows(l), bf + 1));
             ZK_CUDA(ctx, copy_rows(pin_poly, pin, n));
-            ZK_TRY(lagrange_to_coeff(pk, pin_poly));
+            ZK_TRY(lagrange_to_coeff(ps, pin_poly));
             ZK_CUDA(ctx, copy_rows(ptab_poly, ptab, n));
-            ZK_TRY(lagrange_to_coeff(pk, ptab_poly));
+            ZK_TRY(lagrange_to_coeff(ps, ptab_poly));
         }
-        ZK_CUDA(ctx, cudaMemcpyAsync(ctx->pinned, pk->d_err, 4, cudaMemcpyDeviceToHost, st));
+        ZK_CUDA(ctx, cudaMemcpyAsync(ctx->pinned, ps->d_err, 4, cudaMemcpyDeviceToHost, st));
         ZK_CUDA(ctx, cudaStreamSynchronize(st));
         uint32_t err = *(const uint32_t*)ctx->pinned;
         if (L) {                                                      // permuted input / table commitments of all lookups, one batch
@@ -773,7 +806,7 @@ struct Prover {
             }
             if (!sh.set_mine(s)) continue;
             {
-                PhaseTimer t(pk, PH_PERM);
+                PhaseTimer t(ps, PH_PERM);
                 pa.beta = to_dev(beta); pa.gamma = to_dev(gamma); pa.omega_pows = pk->omega_pows; pa.out = tmp_n;
                 perm_den_kernel<<<nb(n), PK_THREADS, 0, st>>>(pa);
                 ctx->launches++;
@@ -788,7 +821,7 @@ struct Prover {
             std::vector<HFr> totals(S, HFr::one());
             ZK_CUDA(ctx, cudaStreamSynchronize(st));
             for (uint32_t s = 0; s < S; ++s) if (sh.set_mine(s)) totals[s] = HFr::from_limbs((const fe_t*)ctx->pinned + s);
-            ZK_TRY(sh.gather(pk, totals, [&](size_t s) { return sh.set_owner((uint32_t)s); }));
+            ZK_TRY(sh.gather(ps, totals, [&](size_t s) { return sh.set_owner((uint32_t)s); }));
             HFr carry = HFr::one();
             for (uint32_t s = 0; s < S; ++s) {
                 fe_t* z = perm_polys + (size_t)s * n;
@@ -807,10 +840,10 @@ struct Prover {
         }
         std::vector<CommPiece> pieces;
         const bool batch_intt = !sh.on() && S > 1 && ((uint64_t)S << dom->k) <= 0xFFFFFFFFull;      // one rank: all sets in one launch per pass
-        if (batch_intt) ZK_TRY(lagrange_to_coeff(pk, perm_polys, S));
+        if (batch_intt) ZK_TRY(lagrange_to_coeff(ps, perm_polys, S));
         for (uint32_t s = 0; s < S; ++s) {
             fe_t* z = perm_polys + (size_t)s * n;
-            if (!batch_intt && sh.set_mine(s)) ZK_TRY(lagrange_to_coeff(pk, z));
+            if (!batch_intt && sh.set_mine(s)) ZK_TRY(lagrange_to_coeff(ps, z));
             pieces.push_back({z, n * sizeof(fe_t), sh.set_owner(s)});
         }
         ZK_TRY(share(pieces));
@@ -824,7 +857,7 @@ struct Prover {
             if (!sh.lk_mine(l)) continue;
             fe_t* z = LK(l, 6);
             {
-                PhaseTimer t(pk, PH_LOOKUP);
+                PhaseTimer t(ps, PH_LOOKUP);
                 LookupProdArgs la{LK(l, 2), LK(l, 3), LK(l, 0), LK(l, 1), to_dev(ch[EXF_BETA]), to_dev(ch[EXF_GAMMA]), tmp_n, (uint32_t)n};
                 lookup_den_kernel<<<nb(n), PK_THREADS, 0, st>>>(la);
                 ctx->launches++;
@@ -841,7 +874,7 @@ struct Prover {
         std::vector<CommPiece> pieces;
         for (uint32_t l = 0; l < L; ++l) { cols.push_back(LK(l, 6)); owners.push_back(sh.lk_owner(l)); pieces.push_back({LK(l, 6), n * sizeof(fe_t), sh.lk_owner(l)}); }
         ZK_TRY(commit_columns(cols, owners, "lookup_product_commits"));
-        for (uint32_t l = 0; l < L; ++l) if (sh.lk_mine(l)) ZK_TRY(lagrange_to_coeff(pk, LK(l, 6)));
+        for (uint32_t l = 0; l < L; ++l) if (sh.lk_mine(l)) ZK_TRY(lagrange_to_coeff(ps, LK(l, 6)));
         ZK_TRY(share(pieces));
         if (pk->lk_early && lk_rows) {                                // side stream: the product cosets
             SideStream side(ctx);
@@ -863,9 +896,9 @@ struct Prover {
             std::vector<HFr> ypow(1, HFr::one());
             for (uint32_t i = 0; i < cs.gates.size(); ++i) {
                 while (ypow.size() <= pk->gate_exp[i]) ypow.push_back(ypow.back() * ch[EXF_Y]);
-                ((fe_t*)pk->h_wts)[i] = to_dev(ypow[pk->gate_exp[i]]);
+                ((fe_t*)ps->h_wts)[i] = to_dev(ypow[pk->gate_exp[i]]);
             }
-            ZK_CUDA(ctx, cudaMemcpyAsync(pk->d_wts, pk->h_wts, cs.gates.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
+            ZK_CUDA(ctx, cudaMemcpyAsync(ps->d_wts, ps->h_wts, cs.gates.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
         }
         // step 10: the advice / instance cosets were started on the side stream after the advice commitments
         ZK_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_join, 0));
@@ -875,7 +908,7 @@ struct Prover {
         if (lin_mine()) ZK_TRY(gate_class(QC_LINEAR, h_lin, 0, (uint32_t)n));
         if (my_rows) {
             ZK_TRY(gate_class(QC_MAIN, h, my_row0, my_rows));
-            PhaseTimer t(pk, PH_QUOT);
+            PhaseTimer t(ps, PH_QUOT);
             if (S) {
                 QuotPermAArgs qa{};
                 qa.h = h; qa.y = to_dev(y); qa.l0 = pk->l0; qa.l_last = pk->l_last; qa.nsets = S;
@@ -912,7 +945,7 @@ struct Prover {
                 ZK_TRY(my_cosets(LK(l, 5), sc, lj0, lj1));
                 lookup_table_value(l);
             }
-            PhaseTimer t(pk, PH_QUOT);
+            PhaseTimer t(ps, PH_QUOT);
             QuotLookupArgs ql{};
             ql.h = lk_split ? h_lk : h; ql.y = to_dev(y); ql.beta = to_dev(beta); ql.gamma = to_dev(gamma);
             ql.l0 = pk->l0; ql.l_last = pk->l_last; ql.l_active = pk->l_active; ql.z = zc; ql.a = ac; ql.s = sc; ql.table_value = tv;
@@ -930,16 +963,16 @@ struct Prover {
         {
             // divide by the vanishing polynomial (constant c_j^n - 1 on coset j), per-coset iNTT, then
             // the q x q interpolation across cosets gives the coefficients of h piece by piece
-            PhaseTimer t(pk, PH_NTT);
+            PhaseTimer t(ps, PH_NTT);
             HFr y_lk = HFr::one();                                    // h = h_gates_perm * y^(5 L) + h_lk
             if (lk_split) {
                 for (uint32_t i = 0; i < 5 * L; ++i) y_lk = y_lk * ch[EXF_Y];  // (the low gates' weights leave this factor to the lookup kernels)
                 for (uint32_t j = lj0; j < lj1; ++j)                           // divided by the vanishing polynomial before the extrapolation
-                    ZK_TRY(intt_scaled(pk, h_lk + j * n, 1, dom->ifft_divisor * pk->coset_t[j]));
+                    ZK_TRY(intt_scaled(ps, h_lk + j * n, 1, dom->ifft_divisor * pk->coset_t[j]));
             }
-            for (uint32_t j = cj0; j < cj1; ++j) ZK_TRY(intt_scaled(pk, h + j * n, 1, dom->ifft_divisor * pk->coset_t[j] * y_lk));
+            for (uint32_t j = cj0; j < cj1; ++j) ZK_TRY(intt_scaled(ps, h + j * n, 1, dom->ifft_divisor * pk->coset_t[j] * y_lk));
             // the linear gates' part of h, degree < n: coefficients in X / c_0
-            if (lin_mine()) ZK_TRY(intt_scaled(pk, h_lin, 1, dom->ifft_divisor * pk->coset_t[0]));
+            if (lin_mine()) ZK_TRY(intt_scaled(ps, h_lin, 1, dom->ifft_divisor * pk->coset_t[0]));
         }
         std::vector<CommPiece> pieces;                                // every coset's coefficients to every rank: q (+ CL) x n elements
         for (uint32_t j = 0; j < pk->q; ++j) pieces.push_back({h + (size_t)j * n, n * sizeof(fe_t), sh.coset_owner(j)});
@@ -947,7 +980,7 @@ struct Prover {
         if (pk->gate_prog[QC_LINEAR].second) pieces.push_back({h_lin, n * sizeof(fe_t), sh.coset_owner(0)});
         ZK_TRY(share(pieces));
         {
-            PhaseTimer t(pk, PH_NTT);
+            PhaseTimer t(ps, PH_NTT);
             if (lk_split) {
                 lookup_extrapolate_kernel<<<nb(n), PK_THREADS, 0, st>>>(h_lk, pk->coset_pow_inv, pk->lk_lambda, nullptr, CL, pk->q, n);
                 ctx->launches++;
@@ -960,7 +993,7 @@ struct Prover {
         std::vector<const fe_t*> cols;
         std::vector<HAffine> pts;
         for (uint32_t i = 0; i < pk->q; ++i) cols.push_back(lk_cosets + (size_t)i * n);
-        ZK_TRY(commit_multi_range(pk, sh, cols, n, false, pts));
+        ZK_TRY(commit_multi_range(ps, sh, cols, n, false, pts));
         for (auto& pt : pts) tr.write_point(pt);
         mark("quotient_and_h_commits");
         return B200ZK_OK;
@@ -989,7 +1022,7 @@ struct Prover {
         for (size_t i = 0; i < pairs.size(); ++i) if (sh.mine((uint32_t)i)) { bp.push_back(pairs[i].poly); bx.push_back(pairs[i].point); }
         std::vector<HFr> mv(bp.size());
         {
-            PhaseTimer t(pk, PH_OPEN);
+            PhaseTimer t(ps, PH_OPEN);
             // vanishing::evaluate: h_poly = sum_i (x^n)^i h_piece_i
             fold_pieces_kernel<<<nb(n), PK_THREADS, 0, st>>>(lk_cosets, pk->q, n, to_dev(x.pow_u64(n)), h_poly);
             ctx->launches++;
@@ -997,7 +1030,7 @@ struct Prover {
         }
         values.assign(pairs.size(), HFr::zero());
         for (size_t i = 0, j = 0; i < pairs.size(); ++i) if (sh.mine((uint32_t)i)) values[i] = mv[j++];
-        ZK_TRY(sh.gather(pk, values, [&](size_t i) { return sh.owner((uint32_t)i); }));
+        ZK_TRY(sh.gather(ps, values, [&](size_t i) { return sh.owner((uint32_t)i); }));
         mark("evaluations");
         // the transcript's order: advice, fixed, random, sigma, permutation sets, lookups
         for (size_t i = 0; i < cs.adv_q.size(); i += 2) ZK_TRY(write_eval(advice_polys + (size_t)cs.adv_q[i] * n, rotate_omega(dom, x, cs.adv_q[i + 1])));
@@ -1020,7 +1053,7 @@ struct Prover {
     int32_t shplonk() {
         HFr sy, sv, su;
         {
-            PhaseTimer t(pk, PH_OPEN);
+            PhaseTimer t(ps, PH_OPEN);
             sy = tr.squeeze_challenge();
             ZK_TRY(shplonk_sets());
             sv = tr.squeeze_challenge();
@@ -1072,12 +1105,12 @@ struct Prover {
             }
         }
         std::vector<HAffine> pt;
-        ZK_TRY(commit_multi_range(pk, sh, {hx}, n, false, pt));
+        ZK_TRY(commit_multi_range(ps, sh, {hx}, n, false, pt));
         tr.write_point(pt[0]);
         mark("shplonk_h1_commit");
         {
             // the linearisation polynomial L(X) at u, divided by (X - u) into t0
-            PhaseTimer t(pk, PH_OPEN);
+            PhaseTimer t(ps, PH_OPEN);
             su = tr.squeeze_challenge();
             auto vanish = [&](const std::vector<HFr>& roots) { HFr acc = HFr::one(); for (auto& r : roots) acc = acc * (su - r); return acc; };
             HFr v_pow = HFr::one(), const_term = HFr::zero(), z0_diff = HFr::zero();
@@ -1106,7 +1139,7 @@ struct Prover {
             ctx->launches++;
             ZK_CUDA(ctx, cudaGetLastError());
         }
-        ZK_TRY(commit_multi_range(pk, sh, {t0}, n - 1, false, pt));
+        ZK_TRY(commit_multi_range(ps, sh, {t0}, n - 1, false, pt));
         tr.write_point(pt[0]);
         return B200ZK_OK;
     }
@@ -1153,20 +1186,22 @@ struct Prover {
     }
 };
 
-static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_device, const void* const* advice_host,
+static int32_t prove(ProofState* ps, const fe_t* d_advice_in, bool advice_on_device, const void* const* advice_host,
                      const void* const* instance_columns, const uint32_t* instance_lens, const void* rng_wide, bool rng_on_device,
                      const HFr& transcript_repr, std::vector<uint8_t>& proof_out) {
-    b200zk_ctx* ctx = pk->ctx;
+    const b200zk_pk* pk = ps->pk;
+    b200zk_ctx* ctx = ps->ctx;
     for (uint32_t c = 0; c < pk->cs.I; ++c) if (instance_lens[c] && !instance_columns[c]) return fail(ctx, B200ZK_EINVAL, "create_proof", "null instance column");
     if (!advice_on_device) for (uint32_t c = 0; c < pk->cs.A; ++c) if (!advice_host[c]) return fail(ctx, B200ZK_EINVAL, "create_proof", "null advice column");
     cudaStreamSynchronize(ctx->stream2);                          // nothing of an earlier (failed) proof may still be writing the arena
-    if (pk->copy_stream) cudaStreamSynchronize(pk->copy_stream);
-    for (float& f : pk->phase_ms) f = 0;
-    pk->timer_used = 0;
+    if (ps->copy_stream) cudaStreamSynchronize(ps->copy_stream);
+    for (float& f : ps->phase_ms) f = 0;
+    ps->timer_used = 0;
     ZK_CUDA(ctx, cudaSetDevice(ctx->device));
-    pk->trace.clear();
-    Prover p(pk, advice_on_device, rng_on_device);
-    ZK_CUDA(ctx, cudaMemsetAsync(pk->d_err, 0, 4, ctx->stream));
+    ps->trace.clear();
+    for (auto m : PROOF_WS) (ctx->*m).used = 0;
+    Prover p(ps, advice_on_device, rng_on_device);
+    ZK_CUDA(ctx, cudaMemsetAsync(ps->d_err, 0, 4, ctx->stream));
     ZK_TRY(p.carve());
     ZK_TRY(p.instances(instance_columns, instance_lens, transcript_repr));
     ZK_TRY(p.upload_rng(rng_wide, rng_on_device));
@@ -1185,9 +1220,219 @@ static int32_t prove(b200zk_pk* pk, const fe_t* d_advice_in, bool advice_on_devi
     p.x = p.tr.squeeze_challenge();
     ZK_TRY(p.evaluations());
     ZK_TRY(p.shplonk());
-    phase_timers_collect(pk);
+    phase_timers_collect(ps);
     p.mark("end");
     proof_out = p.tr.proof();
+    for (size_t i = 0; i < N_PROOF_WS; ++i) ps->ws_need[i] = std::max(ps->ws_need[i], (ctx->*PROOF_WS[i]).used);
+    ps->proved = true;
+    return B200ZK_OK;
+}
+
+// ------------------------------------------------------------------ proof states and lanes
+static int32_t proof_state_alloc(ProofState& ps) {
+    const b200zk_pk* pk = ps.pk;
+    auto take = [&](void** p, size_t bytes) -> int32_t {
+        bytes = std::max<size_t>(bytes, 1);
+        // past the limit, ask for more than any device holds: the allocation fails as it does on an exhausted device
+        const bool over = bytes > ps.alloc_limit || ps.owned_bytes > ps.alloc_limit - bytes;
+        cudaError_t e = cudaMalloc(p, over ? ((size_t)1 << 62) : bytes);
+        if (e != cudaSuccess) { *p = nullptr; return fail(ps.ctx, B200ZK_ENOMEM, "cudaMalloc(proof state)", cudaGetErrorString(e)); }
+        ps.owned.push_back(*p);
+        ps.owned_bytes += bytes;
+        return B200ZK_OK;
+    };
+    const size_t G = pk->cs.gates.size();
+    ZK_TRY(take((void**)&ps.d_err, sizeof(uint32_t)));
+    ZK_TRY(take((void**)&ps.d_ptrs, PtrTab{pk->cs.F, pk->cs.A, pk->cs.I}.total() * sizeof(void*)));
+    if (G) {
+        ZK_TRY(take((void**)&ps.d_wts, G * sizeof(fe_t)));
+        ZK_CUDA(ps.ctx, cudaMallocHost((void**)&ps.h_wts, G * sizeof(fe_t)));
+    }
+    ps.arena_bytes = arena_need(pk);
+    return take((void**)&ps.arena, ps.arena_bytes);
+}
+
+static void proof_state_release(ProofState& ps) {
+    if (!ps.ctx) return;
+    if (ps.copy_stream) { cudaStreamSynchronize(ps.copy_stream); cudaStreamDestroy(ps.copy_stream); }
+    if (ps.ev_rnd) cudaEventDestroy(ps.ev_rnd);
+    if (ps.h_wts) cudaFreeHost(ps.h_wts);
+    for (cudaEvent_t e : ps.col_events) cudaEventDestroy(e);
+    cudaStreamSynchronize(ps.ctx->stream2);
+    cudaStreamSynchronize(ps.ctx->stream);
+    for (void* p : ps.owned) cudaFree(p);
+    for (auto& t : ps.timer_events) { cudaEventDestroy(t.e0); cudaEventDestroy(t.e1); }
+    ps = ProofState{};
+}
+
+// Lane j >= 1 of b200zk_create_proofs: a ctx of its own on the pk's device (streams, events, workspaces, pinned staging,
+// error text), a view of the pk's params bound to that ctx, and a proof state.  Everything read-only is shared: the pk,
+// the SRS bases and fixed-base tables, the NTT plans at n.
+struct ProofLane {
+    b200zk_ctx* ctx = nullptr;
+    b200zk_params view{};
+    ProofState ps;
+};
+
+// device bytes of one more lane: its arena and its workspaces (ws_reserve adds an eighth)
+static size_t lane_bytes(const b200zk_pk* pk) {
+    size_t ws = 0;
+    for (size_t i = 0; i < N_PROOF_WS; ++i) ws += pk->ps.ws_need[i];
+    return pk->ps.arena_bytes + ws + ws / 8;
+}
+// a lane's workspaces at the sizes a proof of the pk requested on the pk's ctx (nothing before the first proof)
+static int32_t lane_reserve_ws(const b200zk_pk* pk, b200zk_ctx* lc) {
+    for (size_t i = 0; i < N_PROOF_WS; ++i) ZK_TRY(ws_reserve(lc, lc->*PROOF_WS[i], pk->ps.ws_need[i]));
+    return B200ZK_OK;
+}
+
+static void lane_destroy(ProofLane* ln) {
+    proof_state_release(ln->ps);
+    b200zk_ctx_destroy(ln->ctx);                  // frees its workspaces; the borrowed plans stay with the pk's ctx
+    delete ln;
+}
+
+static void lanes_trim(b200zk_pk* pk, size_t extra) {
+    while (pk->lanes.size() > extra) { lane_destroy(pk->lanes.back()); pk->lanes.pop_back(); }
+}
+
+static int32_t lane_create(b200zk_pk* pk, ProofLane** out) {
+    ProofLane* ln = new (std::nothrow) ProofLane();
+    if (!ln) return B200ZK_ENOMEM;
+    int32_t rc = b200zk_ctx_create(pk->ctx->device, &ln->ctx);
+    if (rc != B200ZK_OK) { delete ln; return fail(pk->ctx, rc, "create_proofs", "cannot create a lane context"); }
+    cudaSetDevice(pk->ctx->device);
+    for (auto& kv : pk->ctx->ntt_plans)                           // the plans at n (omega, omega^-1): pk_create built them
+        if (kv.first[0] == pk->dom->k) { NttPlan plan = kv.second; plan.borrowed = true; ln->ctx->ntt_plans.emplace(kv.first, plan); }
+    ln->ctx->ntt_attr_set = pk->ctx->ntt_attr_set;
+    const b200zk_params* src = pk->params;
+    ln->view.ctx = ln->ctx; ln->view.k = src->k;
+    ln->view.d_g = src->d_g; ln->view.d_g_lagrange = src->d_g_lagrange;
+    ln->view.d_g_pre = src->d_g_pre; ln->view.d_gl_pre = src->d_gl_pre; ln->view.pre = src->pre;
+    ln->view.sum_table[0] = src->sum_table[0]; ln->view.sum_table[1] = src->sum_table[1];
+    ln->ps.pk = pk; ln->ps.ctx = ln->ctx; ln->ps.params = &ln->view;
+    // B200ZK_LANE_ALLOC_LIMIT (a test aid): device bytes the proof states of all extra lanes of the pk may hold together
+    if (const char* lim = getenv("B200ZK_LANE_ALLOC_LIMIT")) {
+        size_t held = 0;
+        for (const ProofLane* other : pk->lanes) held += other->ps.owned_bytes;
+        const size_t cap = (size_t)strtoull(lim, nullptr, 10);
+        ln->ps.alloc_limit = cap > held ? cap - held : 0;
+    }
+    rc = proof_state_alloc(ln->ps);
+    if (rc == B200ZK_OK) rc = lane_reserve_ws(pk, ln->ctx);
+    if (rc != B200ZK_OK) { std::string e = ln->ctx->err; lane_destroy(ln); return fail(pk->ctx, rc, "create_proofs", e.c_str()); }
+    *out = ln;
+    return B200ZK_OK;
+}
+
+// Plans and creates the extra lanes for `count` proofs (0: a reservation) and returns how many lanes run, >= 1.  Fewer
+// lanes than planned when memory runs out is not an error: the failed allocation's error is cleared from this thread,
+// which goes on to run lane 0 (or the next create_proof), so that no later cudaGetLastError reports it.  Nothing runs on the pk's ctx or its lanes meanwhile, so the
+// device synchronisations of cudaFree and of the sum tables' build happen here, never while proofs run side by side.
+static int32_t lanes_plan(b200zk_pk* pk, uint32_t count, uint32_t* used) {
+    ZK_TRY(params_sum_tables(pk->params));                      // nothing builds them lazily while the lanes run
+    size_t free_b = 0, total_b = 0;
+    ZK_CUDA(pk->ctx, cudaMemGetInfo(&free_b, &total_b));
+    uint32_t nl = plan_lanes(count, pk->lane_want, getenv("B200ZK_PROOF_LANES"), free_b, lane_bytes(pk), (uint32_t)pk->lanes.size());
+    if (!count) lanes_trim(pk, nl - 1);
+    for (uint32_t j = 0; j < pk->lanes.size() && j + 1 < nl; ++j)      // lane j + 1 may predate the pk's first proof
+        if (lane_reserve_ws(pk, pk->lanes[j]->ctx) != B200ZK_OK) { cudaGetLastError(); nl = j + 1; break; }
+    while (pk->lanes.size() + 1 < nl) {
+        ProofLane* ln = nullptr;
+        if (lane_create(pk, &ln) != B200ZK_OK) { cudaGetLastError(); nl = 1 + (uint32_t)pk->lanes.size(); break; }
+        pk->lanes.push_back(ln);
+    }
+    *used = std::min<uint32_t>(nl, 1 + (uint32_t)pk->lanes.size());
+    return B200ZK_OK;
+}
+
+// `count` proofs of one pk, each exactly what create_proof returns for its inputs.  Lane 0 is the pk's own state; lanes
+// run on library threads (as group_prove's ranks do) and take proof indices from a shared counter, so that one proof's
+// transcript, host interpolation and synchronisations overlap the others' kernels.  A lane's workspaces have the sizes a
+// proof of the pk requested on the pk's ctx: until one has completed there, lane 0 proves alone.
+struct BatchInputs {
+    bool dev;
+    const void* const* advice;        // host: count * A column pointers; dev: count blocks of A x n
+    const void* const* instance_columns;
+    const uint32_t* instance_lens;
+    const void* const* rng;
+};
+
+static int32_t prove_batch(b200zk_pk* pk, uint32_t count, const BatchInputs& in, const void* transcript_repr, uint8_t* proofs_out,
+                           int32_t* status) {
+    b200zk_ctx* ctx = pk->ctx;
+    ZK_CUDA(ctx, cudaSetDevice(ctx->device));                     // lanes_plan runs on this thread before any proof does
+    const size_t psize = b200zk_pk_proof_size(pk);
+    const uint32_t A = pk->cs.A, I = pk->cs.I;
+    const HFr repr = HFr::from_limbs(transcript_repr);
+    constexpr int32_t NOT_RUN = 1;
+    std::vector<std::string> errs(count);
+    for (uint32_t i = 0; i < count; ++i) status[i] = NOT_RUN;
+    std::atomic<uint32_t> next{0};
+    std::atomic<bool> stop{false};
+    auto run_one = [&](ProofState* ps, uint32_t i) {
+        std::vector<uint8_t> proof;
+        const void* const* inst = in.instance_columns ? in.instance_columns + (size_t)i * I : nullptr;
+        const uint32_t* lens = in.instance_lens ? in.instance_lens + (size_t)i * I : nullptr;
+        int32_t rc = in.dev ? prove(ps, (const fe_t*)in.advice[i], true, nullptr, inst, lens, in.rng[i], true, repr, proof)
+                            : prove(ps, nullptr, false, in.advice ? in.advice + (size_t)i * A : nullptr, inst, lens, in.rng[i], false, repr, proof);
+        if (rc == B200ZK_OK && proof.size() != psize) rc = fail(ps->ctx, B200ZK_ECUDA, "create_proofs", "internal: proof size differs from pk_proof_size");
+        uint8_t* out = proofs_out + (size_t)i * psize;
+        if (rc == B200ZK_OK) memcpy(out, proof.data(), psize);
+        else {
+            memset(out, 0, psize);
+            if (ps->copy_stream) cudaStreamSynchronize(ps->copy_stream);     // the caller's buffers are borrowed for the call only
+            errs[i] = ps->ctx->err;
+            if (rc != B200ZK_ESYNTH) stop = true;
+        }
+        status[i] = rc;
+    };
+    auto lane_loop = [&](ProofState* ps) {
+        cudaSetDevice(ps->ctx->device);
+        for (uint32_t i; !stop && (i = next++) < count;) run_one(ps, i);
+    };
+    for (uint32_t i; !pk->ps.proved && !stop && (i = next++) < count;) run_one(&pk->ps, i);
+    uint32_t nl = 1;
+    if (!stop && next < count && lanes_plan(pk, count, &nl) != B200ZK_OK) { cudaGetLastError(); nl = 1; }     // the lanes only add speed
+    std::vector<uint64_t> launches0(nl, 0);
+    for (uint32_t j = 1; j < nl; ++j) launches0[j] = pk->lanes[j - 1]->ctx->launches;
+    std::vector<std::thread> threads;
+    for (uint32_t j = 1; j < nl; ++j) threads.emplace_back(lane_loop, &pk->lanes[j - 1]->ps);
+    lane_loop(&pk->ps);
+    for (auto& t : threads) t.join();
+    for (uint32_t j = 1; j < nl; ++j) {
+        b200zk_ctx* lc = pk->lanes[j - 1]->ctx;
+        ctx->launches += lc->launches - launches0[j];
+        cudaStreamSynchronize(lc->stream2);
+        cudaStreamSynchronize(lc->stream);
+    }
+    int32_t fatal = B200ZK_OK;
+    long first_fatal = -1, first_synth = -1;
+    for (uint32_t i = 0; i < count; ++i) {
+        if (status[i] == B200ZK_ESYNTH && first_synth < 0) first_synth = i;
+        if (status[i] != B200ZK_OK && status[i] != B200ZK_ESYNTH && status[i] != NOT_RUN && first_fatal < 0) { first_fatal = i; fatal = status[i]; }
+    }
+    for (uint32_t i = 0; i < count; ++i) if (status[i] == NOT_RUN) status[i] = fatal;
+    const long bad = first_fatal >= 0 ? first_fatal : first_synth;
+    if (bad < 0) return B200ZK_OK;
+    const std::string what = "create_proofs: proof " + std::to_string(bad);
+    return fail(ctx, first_fatal >= 0 ? fatal : B200ZK_ESYNTH, what.c_str(), errs[bad].c_str());
+}
+
+// the argument checks every batch entry point shares; B200ZK_EINVAL before any work
+static int32_t batch_check(b200zk_pk* pk, uint32_t count, const void* const* advice, const void* const* instance_columns, const uint32_t* instance_lens,
+                           const void* const* rng, const void* transcript_repr, const uint8_t* proofs_out, size_t proofs_cap, const int32_t* status) {
+    if (!pk) return B200ZK_EINVAL;
+    b200zk_ctx* ctx = pk->ctx;
+    if (!count || !rng || !transcript_repr || !proofs_out || !status || (pk->cs.A && !advice) || (pk->cs.I && (!instance_columns || !instance_lens)))
+        return fail(ctx, B200ZK_EINVAL, "create_proofs", "null argument or count == 0");
+    if (ctx->comm) return fail(ctx, B200ZK_EINVAL, "create_proofs", "the pk's ctx is one rank of a sharded proof: batches are single-GPU");
+    if (proofs_cap / count < b200zk_pk_proof_size(pk)) return fail(ctx, B200ZK_EINVAL, "create_proofs", "proof buffer smaller than count * proof_size");
+    for (uint32_t i = 0; i < count; ++i) {
+        if (!rng[i]) return fail(ctx, B200ZK_EINVAL, "create_proofs", "null rng stream");
+        for (uint32_t c = 0; c < pk->cs.I; ++c)
+            if (instance_lens[(size_t)i * pk->cs.I + c] && !instance_columns[(size_t)i * pk->cs.I + c]) return fail(ctx, B200ZK_EINVAL, "create_proofs", "null instance column");
+    }
     return B200ZK_OK;
 }
 
@@ -1213,8 +1458,8 @@ uint32_t b200zk_pk_degree(const b200zk_pk* pk) { return pk ? pk->cs.degree : 0; 
 // debugging aid: copy a named device buffer of the last proof to the host (elements of 32 bytes)
 int32_t b200zk_pk_debug_buffer(b200zk_pk* pk, const char* name, void* host_out, size_t max_elems, size_t* count) {
     if (!pk || !name || !host_out) return B200ZK_EINVAL;
-    auto it = pk->dbg.find(name);
-    if (it == pk->dbg.end()) return fail(pk->ctx, B200ZK_EINVAL, "debug_buffer", "unknown buffer");
+    auto it = pk->ps.dbg.find(name);
+    if (it == pk->ps.dbg.end()) return fail(pk->ctx, B200ZK_EINVAL, "debug_buffer", "unknown buffer");
     size_t c = std::min(max_elems, it->second.second);
     if (count) *count = it->second.second;
     ZK_CUDA(pk->ctx, cudaMemcpyAsync(host_out, it->second.first, c * sizeof(fe_t), cudaMemcpyDeviceToHost, pk->ctx->stream));
@@ -1254,7 +1499,7 @@ int32_t b200zk_pk_quotient_muls(const b200zk_pk* pk, uint32_t out5[5]) {
 int32_t b200zk_pk_last_trace(const b200zk_pk* pk, char* out, size_t cap) {
     if (!pk || !out || cap == 0) return B200ZK_EINVAL;
     std::string t;
-    for (auto& kv : pk->trace) { char buf[96]; snprintf(buf, sizeof buf, "%s:%.3f;", kv.first, kv.second); t += buf; }
+    for (auto& kv : pk->ps.trace) { char buf[96]; snprintf(buf, sizeof buf, "%s:%.3f;", kv.first, kv.second); t += buf; }
     if (t.size() + 1 > cap) return B200ZK_EINVAL;
     memcpy(out, t.c_str(), t.size() + 1);
     return B200ZK_OK;
@@ -1262,7 +1507,7 @@ int32_t b200zk_pk_last_trace(const b200zk_pk* pk, char* out, size_t cap) {
 
 int32_t b200zk_pk_last_phase_ms(const b200zk_pk* pk, float* out7) {
     if (!pk || !out7) return B200ZK_EINVAL;
-    memcpy(out7, pk->phase_ms, sizeof(pk->phase_ms));
+    memcpy(out7, pk->ps.phase_ms, sizeof(pk->ps.phase_ms));
     return B200ZK_OK;
 }
 
@@ -1277,26 +1522,23 @@ int32_t b200zk_pk_vk_commitments(b200zk_pk* pk, void* fixed_out, void* sigma_out
         std::vector<const fe_t*> cols;
         std::vector<HAffine> pts;
         for (uint32_t c = 0; c < count; ++c) cols.push_back(base + (size_t)c * n);
-        ZK_TRY(commit_multi_dev(pk, cols, n, false, pts));
+        ZK_TRY(commit_multi_dev(&pk->ps, cols, n, false, pts));
         for (uint32_t c = 0; c < count; ++c) { pts[c].x.store((uint8_t*)out + 64 * (size_t)c); pts[c].y.store((uint8_t*)out + 64 * (size_t)c + 32); }
         return B200ZK_OK;
     };
     ZK_TRY(run(pk->fixed_polys, pk->cs.F, fixed_out));
     ZK_TRY(run(pk->perm_polys, pk->P, sigma_out));
-    pk->timer_used = 0;
+    pk->ps.timer_used = 0;
     return B200ZK_OK;
 }
 
 void b200zk_pk_destroy(b200zk_pk* pk) {
     if (!pk) return;
     cudaSetDevice(pk->ctx->device);
-    if (pk->copy_stream) { cudaStreamSynchronize(pk->copy_stream); cudaStreamDestroy(pk->copy_stream); }
-    if (pk->ev_rnd) cudaEventDestroy(pk->ev_rnd);
-    if (pk->h_wts) cudaFreeHost(pk->h_wts);
-    for (cudaEvent_t e : pk->col_events) cudaEventDestroy(e);
+    lanes_trim(pk, 0);
+    proof_state_release(pk->ps);
     cudaStreamSynchronize(pk->ctx->stream);
     for (void* p : pk->owned) cudaFree(p);
-    for (auto& t : pk->timer_events) { cudaEventDestroy(t.e0); cudaEventDestroy(t.e1); }
     if (pk->dom) b200zk_domain_destroy(pk->dom);
     delete pk;
 }
@@ -1309,6 +1551,7 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
     b200zk_pk* pk = new (std::nothrow) b200zk_pk();
     if (!pk) return B200ZK_ENOMEM;
     pk->ctx = ctx; pk->params = params;
+    pk->ps.pk = pk; pk->ps.ctx = ctx; pk->ps.params = params;
     auto bail = [&](int32_t rc) { b200zk_pk_destroy(pk); return rc; };
     if (!parse_cs(cs_blob, blob_words, pk->cs)) return bail(fail(ctx, B200ZK_EINVAL, "pk_create", "malformed constraint-system blob"));
     CsDesc& cs = pk->cs;
@@ -1336,7 +1579,6 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
     PK_TRY(dev_alloc(pk, &pk->perm_values, P * n)); PK_TRY(dev_alloc(pk, &pk->perm_polys, P * n)); PK_TRY(dev_alloc(pk, &pk->perm_cosets, P * ext));
     PK_TRY(dev_alloc(pk, &pk->l0, ext)); PK_TRY(dev_alloc(pk, &pk->l_last, ext)); PK_TRY(dev_alloc(pk, &pk->l_active, ext));
     PK_TRY(dev_alloc(pk, &pk->omega_pows, n));
-    PK_TRY(dev_alloc(pk, &pk->d_err, 1));
     // quotient cosets: powers of c_j and 1/c_j, extended_omega^j, 1/(c_j^n - 1), inverse Vandermonde of c_j^n
     {
         const uint32_t C = pk->q;
@@ -1392,8 +1634,8 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
     for (uint32_t c = 0; c < F; ++c) PK_CUDA(cudaMemcpyAsync(pk->fixed_values + (size_t)c * n, fixed_columns[c], n * sizeof(fe_t), cudaMemcpyHostToDevice, st));
     PK_CUDA(cudaMemcpyAsync(pk->fixed_polys, pk->fixed_values, F * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, st));
     for (uint32_t c = 0; c < F; ++c) {
-        PK_TRY(lagrange_to_coeff(pk, pk->fixed_polys + (size_t)c * n));
-        PK_TRY(coeff_to_extended(pk, pk->fixed_polys + (size_t)c * n, pk->fixed_cosets + (size_t)c * ext));
+        PK_TRY(lagrange_to_coeff(&pk->ps, pk->fixed_polys + (size_t)c * n));
+        PK_TRY(coeff_to_extended(&pk->ps, pk->fixed_polys + (size_t)c * n, pk->fixed_cosets + (size_t)c * ext));
     }
     PK_TRY(powers_run(ctx, dom->omega, n, pk->omega_pows));
     // permutation polynomials: sigma_c[r] = delta^map_col * omega^map_row
@@ -1408,8 +1650,8 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
         ctx->launches++;
         PK_CUDA(cudaMemcpyAsync(pk->perm_polys, pk->perm_values, P * n * sizeof(fe_t), cudaMemcpyDeviceToDevice, st));
         for (uint32_t c = 0; c < P; ++c) {
-            PK_TRY(lagrange_to_coeff(pk, pk->perm_polys + (size_t)c * n));
-            PK_TRY(coeff_to_extended(pk, pk->perm_polys + (size_t)c * n, pk->perm_cosets + (size_t)c * ext));
+            PK_TRY(lagrange_to_coeff(&pk->ps, pk->perm_polys + (size_t)c * n));
+            PK_TRY(coeff_to_extended(&pk->ps, pk->perm_polys + (size_t)c * n, pk->perm_cosets + (size_t)c * ext));
         }
     }
     // l0, l_last, l_blind -> l_active_row
@@ -1422,8 +1664,8 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
             std::vector<fe_t> ones(hi - lo, one);
             ZK_CUDA(ctx, cudaMemcpyAsync(tmp + lo, ones.data(), ones.size() * sizeof(fe_t), cudaMemcpyHostToDevice, st));
             ZK_CUDA(ctx, cudaStreamSynchronize(st));
-            ZK_TRY(lagrange_to_coeff(pk, tmp));
-            return coeff_to_extended(pk, tmp, out_ext);
+            ZK_TRY(lagrange_to_coeff(&pk->ps, tmp));
+            return coeff_to_extended(&pk->ps, tmp, out_ext);
         };
         PK_TRY(indicator(0, 1, pk->l0));
         PK_TRY(indicator(n - cs.bf, n, lb));
@@ -1451,10 +1693,6 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
             if (!ex_share_common(cs.prog, items, prog, true)) return bail(fail(ctx, B200ZK_EINVAL, "pk_create", "malformed expression program"));
             pk->gate_prog[cls] = {off, (uint32_t)prog.size() - off};
         }
-        if (G) {
-            PK_TRY(dev_alloc(pk, &pk->d_wts, G));
-            PK_CUDA(cudaMallocHost((void**)&pk->h_wts, G * sizeof(fe_t)));
-        }
         for (auto& lk : cs.lookups) {
             uint32_t off = (uint32_t)prog.size();
             std::vector<ExFold> items;
@@ -1481,8 +1719,6 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
         PK_CUDA(cudaMemcpyAsync(pk->d_q_fix, cs.fix_q.data(), cs.fix_q.size() * 4, cudaMemcpyHostToDevice, st));
         PK_CUDA(cudaMemcpyAsync(pk->d_q_inst, cs.inst_q.data(), cs.inst_q.size() * 4, cudaMemcpyHostToDevice, st));
         PK_CUDA(cudaStreamSynchronize(st));
-        PtrTab pt{cs.F, cs.A, cs.I};
-        PK_TRY(dev_alloc(pk, &pk->d_ptrs, pt.total()));
     }
     {
         // early lookup cosets when their 4 L CL n elements are a modest share of the device (B200ZK_LOOKUP_EARLY=0/1 overrides)
@@ -1492,8 +1728,7 @@ int32_t b200zk_pk_create(b200zk_params* params, const uint32_t* cs_blob, size_t 
         pk->lk_early = pk->L > 0 && extra <= free_b / 4;
         if (const char* e = getenv("B200ZK_LOOKUP_EARLY")) pk->lk_early = pk->L > 0 && e[0] != '0';
     }
-    pk->arena_bytes = arena_need(pk);
-    PK_TRY(dev_alloc(pk, &pk->arena, pk->arena_bytes));
+    PK_TRY(proof_state_alloc(pk->ps));
     PK_CUDA(cudaStreamSynchronize(st));
     PK_CUDA(cudaGetLastError());
 #undef PK_TRY
@@ -1507,7 +1742,7 @@ static int32_t finish_proof(b200zk_pk* pk, int32_t rc, const std::vector<uint8_t
     if (rc != B200ZK_OK && rc != B200ZK_ESYNTH && pk->ctx->comm) pk->ctx->comm->abort();
     if (rc != B200ZK_OK) {
         // a failed proof may have left column uploads in flight: the caller's buffers are borrowed for the call only
-        if (pk->copy_stream) cudaStreamSynchronize(pk->copy_stream);
+        if (pk->ps.copy_stream) cudaStreamSynchronize(pk->ps.copy_stream);
         return rc;
     }
     if (proof_len) *proof_len = proof.size();
@@ -1521,7 +1756,7 @@ int32_t b200zk_create_proof(b200zk_pk* pk, const void* const* advice_columns, co
                             uint8_t* proof_out, size_t proof_cap, size_t* proof_len) {
     if (!pk || !rng_wide || !transcript_repr || !proof_out || (pk->cs.A && !advice_columns) || (pk->cs.I && (!instance_columns || !instance_lens))) return B200ZK_EINVAL;
     std::vector<uint8_t> proof;
-    int32_t rc = prove(pk, nullptr, false, advice_columns, instance_columns, instance_lens, rng_wide, false, HFr::from_limbs(transcript_repr), proof);
+    int32_t rc = prove(&pk->ps, nullptr, false, advice_columns, instance_columns, instance_lens, rng_wide, false, HFr::from_limbs(transcript_repr), proof);
     return finish_proof(pk, rc, proof, proof_out, proof_cap, proof_len);
 }
 
@@ -1530,7 +1765,7 @@ int32_t b200zk_create_proof_dev(b200zk_pk* pk, const void* d_advice, const void*
                                 uint8_t* proof_out, size_t proof_cap, size_t* proof_len) {
     if (!pk || !d_rng_wide || !transcript_repr || !proof_out || (pk->cs.A && !d_advice) || (pk->cs.I && (!instance_columns || !instance_lens))) return B200ZK_EINVAL;
     std::vector<uint8_t> proof;
-    int32_t rc = prove(pk, (const fe_t*)d_advice, true, nullptr, instance_columns, instance_lens, d_rng_wide, true, HFr::from_limbs(transcript_repr), proof);
+    int32_t rc = prove(&pk->ps, (const fe_t*)d_advice, true, nullptr, instance_columns, instance_lens, d_rng_wide, true, HFr::from_limbs(transcript_repr), proof);
     return finish_proof(pk, rc, proof, proof_out, proof_cap, proof_len);
 }
 
@@ -1553,10 +1788,10 @@ static int32_t group_prove(b200zk_group* g, b200zk_pk* const* pks, const void* c
     auto body = [&](uint32_t r) {
         b200zk_pk* pk = pks[r];
         cudaSetDevice(pk->ctx->device);
-        int32_t rc = d_advice_per_rank ? prove(pk, (const fe_t*)d_advice_per_rank[r], true, nullptr, instance_columns, instance_lens, d_rng_per_rank[r], true, repr, proofs[r])
-                                       : prove(pk, nullptr, false, advice_columns, instance_columns, instance_lens, rng_wide, false, repr, proofs[r]);
+        int32_t rc = d_advice_per_rank ? prove(&pk->ps, (const fe_t*)d_advice_per_rank[r], true, nullptr, instance_columns, instance_lens, d_rng_per_rank[r], true, repr, proofs[r])
+                                       : prove(&pk->ps, nullptr, false, advice_columns, instance_columns, instance_lens, rng_wide, false, repr, proofs[r]);
         if (rc != B200ZK_OK && rc != B200ZK_ESYNTH) pk->ctx->comm->abort();
-        if (rc != B200ZK_OK && pk->copy_stream) cudaStreamSynchronize(pk->copy_stream);
+        if (rc != B200ZK_OK && pk->ps.copy_stream) cudaStreamSynchronize(pk->ps.copy_stream);
         rcs[r] = rc;
     };
     std::vector<std::thread> threads;
@@ -1582,6 +1817,33 @@ int32_t b200zk_group_create_proof_dev(b200zk_group* g, b200zk_pk* const* pks, co
                                       uint8_t* proof_out, size_t proof_cap, size_t* proof_len) {
     if (!d_advice_per_rank || !d_rng_wide_per_rank) return B200ZK_EINVAL;
     return group_prove(g, pks, d_advice_per_rank, nullptr, instance_columns, instance_lens, d_rng_wide_per_rank, nullptr, transcript_repr, proof_out, proof_cap, proof_len);
+}
+
+int32_t b200zk_create_proofs(b200zk_pk* pk, uint32_t count, const void* const* advice_columns, const void* const* instance_columns,
+                             const uint32_t* instance_lens, const void* const* rng_wide, const void* transcript_repr,
+                             uint8_t* proofs_out, size_t proofs_cap, int32_t* status) {
+    ZK_TRY(batch_check(pk, count, advice_columns, instance_columns, instance_lens, rng_wide, transcript_repr, proofs_out, proofs_cap, status));
+    for (size_t i = 0; i < (size_t)count * pk->cs.A; ++i)
+        if (!advice_columns[i]) return fail(pk->ctx, B200ZK_EINVAL, "create_proofs", "null advice column");
+    return prove_batch(pk, count, BatchInputs{false, advice_columns, instance_columns, instance_lens, rng_wide}, transcript_repr, proofs_out, status);
+}
+
+int32_t b200zk_create_proofs_dev(b200zk_pk* pk, uint32_t count, const void* const* d_advice, const void* const* instance_columns,
+                                 const uint32_t* instance_lens, const void* const* d_rng_wide, const void* transcript_repr,
+                                 uint8_t* proofs_out, size_t proofs_cap, int32_t* status) {
+    ZK_TRY(batch_check(pk, count, d_advice, instance_columns, instance_lens, d_rng_wide, transcript_repr, proofs_out, proofs_cap, status));
+    if (pk->cs.A)
+        for (uint32_t i = 0; i < count; ++i)
+            if (!d_advice[i]) return fail(pk->ctx, B200ZK_EINVAL, "create_proofs", "null advice block");
+    return prove_batch(pk, count, BatchInputs{true, d_advice, instance_columns, instance_lens, d_rng_wide}, transcript_repr, proofs_out, status);
+}
+
+int32_t b200zk_pk_reserve_lanes(b200zk_pk* pk, uint32_t want, uint32_t* got) {
+    if (!pk || !got) return B200ZK_EINVAL;
+    if (pk->ctx->comm) return fail(pk->ctx, B200ZK_EINVAL, "pk_reserve_lanes", "the pk's ctx is one rank of a sharded proof: batches are single-GPU");
+    ZK_CUDA(pk->ctx, cudaSetDevice(pk->ctx->device));
+    pk->lane_want = want;
+    return lanes_plan(pk, 0, got);
 }
 
 }  // extern "C"

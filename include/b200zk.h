@@ -210,6 +210,35 @@ int32_t b200zk_create_proof(b200zk_pk* pk, const void* const* advice_columns, co
 int32_t b200zk_create_proof_dev(b200zk_pk* pk, const void* d_advice, const void* const* instance_columns,
                                 const uint32_t* instance_lens, const void* d_rng_wide, const void* transcript_repr,
                                 uint8_t* proof_out, size_t proof_cap, size_t* proof_len);
+/* ---- many proofs of one pk on its device, side by side (an extension: upstream has no such call) --------
+ * Proofs of `count` independent witnesses of one pk, run concurrently on the pk's device.  Proof i is byte for byte
+ * what b200zk_create_proof returns for the inputs of proof i: advice_columns[i*A + c], instance_columns[i*I + c],
+ * instance_lens[i*I + c], rng_wide[i]; one transcript_repr for all (one vk).  proofs_out holds
+ * count * b200zk_pk_proof_size(pk) bytes, proof i starting at i * proof_size; status[i] is 0 or that proof's error.
+ * Returns B200ZK_OK when every proof succeeded, B200ZK_ESYNTH when the only failures were ConstraintSystemFailure /
+ * InstanceTooLarge (status says which; the other proofs are produced), any other code when a proof failed otherwise
+ * (b200zk_last_error(pk's ctx) names the proof; proofs the call did not reach get that code in status).
+ * B200ZK_EINVAL before any work for null pointers, count == 0, proofs_cap < count * proof_size, and for a pk whose ctx
+ * is one rank of a sharded proof.  The pk and its ctx stay usable after any failure.
+ * A lane is what one proof in flight needs: lane 0 is the pk's own state on its ctx; every further lane has an
+ * internal ctx on the same device and its own arena (one arena and the workspaces of one proof, see DESIGN.md),
+ * and shares the key, the SRS tables and the NTT plans.  Lanes run on library threads; the calling thread runs lane 0.
+ * b200zk_pk_last_phase_ms / _last_trace / _debug_buffer describe the last proof lane 0 ran; b200zk_launch_count(ctx)
+ * includes the launches of every lane.  The lane count is min(count, a cap, what fits in half of the free device
+ * memory); B200ZK_PROOF_LANES=N replaces the cap.  Fewer lanes than asked when memory is short is not an error. */
+int32_t b200zk_create_proofs(b200zk_pk* pk, uint32_t count, const void* const* advice_columns, const void* const* instance_columns,
+                             const uint32_t* instance_lens, const void* const* rng_wide, const void* transcript_repr,
+                             uint8_t* proofs_out, size_t proofs_cap, int32_t* status);
+/* d_advice[i] = proof i's A x n advice block, d_rng_wide[i] = its draws, both in device memory (as create_proof_dev) */
+int32_t b200zk_create_proofs_dev(b200zk_pk* pk, uint32_t count, const void* const* d_advice, const void* const* instance_columns,
+                                 const uint32_t* instance_lens, const void* const* d_rng_wide, const void* transcript_repr,
+                                 uint8_t* proofs_out, size_t proofs_cap, int32_t* status);
+/* reserve up to `want` lanes now (0 = the planner's default) and use that request for later batches; *got = what
+ * memory allowed, >= 1.  Before the pk's first proof the planner knows a lane's arena but not the workspaces a proof
+ * needs, so *got is provisional then: a later batch reserves those workspaces and runs on fewer lanes if they do not
+ * fit.  A lane that cannot get its memory is never an error. */
+int32_t b200zk_pk_reserve_lanes(b200zk_pk* pk, uint32_t want, uint32_t* got);
+
 /* ---- one create_proof sharded over several GPUs (BASELINE config 5; SURVEY.md 8(e)) ---------------
  * The reference's single prover call (/root/reference/src/circuits/utils.rs:40-48) spread over G GPUs of
  * one NVLink / NVSwitch box.  Every rank holds the SRS and the proving key (b200zk_params_* / b200zk_pk_create

@@ -142,6 +142,29 @@ impl Pk {
         proof.truncate(len);
         Ok(proof)
     }
+    /// Extension (upstream has no such call): create_proof for several witnesses of this key at once, run side by side
+    /// on lanes of its device (b200zk_create_proofs).  Entry i is exactly `create_proof(&advice[i], &instances[i],
+    /// &rng_wide[i], transcript_repr)`: Err(()) where that witness hits ConstraintSystemFailure / InstanceTooLarge.
+    pub fn create_proofs(&self, advice: &[Vec<Vec<Fr>>], instances: &[Vec<&[Fr]>], rng_wide: &[Vec<u8>], transcript_repr: &Fr) -> Vec<Result<Vec<u8>, ()>> {
+        let count = advice.len();
+        assert!(instances.len() == count && rng_wide.len() == count);
+        assert!(rng_wide.iter().all(|w| w.len() >= 64 * self.rng_draws()));
+        let adv: Vec<*const c_void> = advice.iter().flat_map(|a| a.iter().map(|c| c.as_ptr() as *const c_void)).collect();
+        let inst: Vec<*const c_void> = instances.iter().flat_map(|i| i.iter().map(|c| c.as_ptr() as *const c_void)).collect();
+        let lens: Vec<u32> = instances.iter().flat_map(|i| i.iter().map(|c| c.len() as u32)).collect();
+        let rng: Vec<*const c_void> = rng_wide.iter().map(|w| w.as_ptr() as *const c_void).collect();
+        let size = unsafe { sys::b200zk_pk_proof_size(self.0) };
+        let mut proofs = vec![0u8; size * count];
+        let mut status = vec![0i32; count];
+        let rc = unsafe {
+            sys::b200zk_create_proofs(self.0, count as u32, adv.as_ptr(), inst.as_ptr(), lens.as_ptr(), rng.as_ptr(),
+                                      transcript_repr as *const Fr as *const c_void, proofs.as_mut_ptr(), proofs.len(), status.as_mut_ptr())
+        };
+        if rc != sys::B200ZK_ESYNTH {
+            check(rc);
+        }
+        status.iter().enumerate().map(|(i, &s)| if s == 0 { Ok(proofs[i * size..(i + 1) * size].to_vec()) } else { Err(()) }).collect()
+    }
 }
 impl Drop for Pk {
     fn drop(&mut self) {
