@@ -739,5 +739,44 @@ class VerifyingKey:
             raise B200zkError(f"b200zk_verify_proof: error {rc}")
         return rc == OK
 
+    def verify_proofs(self, backend, instances_list, proofs, transcript_repr=None, rng_wide=None, accumulator=False):
+        """verify_proof for many proofs of this key with AccumulatorStrategy: one pairing check for the whole batch, the
+        point decompression and the per-proof opening sums on backend's device (b200zk_verify_proofs).  rng_wide: (count, 8)
+        uint64, the 512-bit input of each proof's Fr::random; default fresh os.urandom draws (they must be secret).
+        Returns a list of bools, and with accumulator=True also (left, right): two (8,) G1Affine Montgomery limb arrays."""
+        count = len(proofs)
+        if len(instances_list) != count:
+            raise B200zkError("one instance list per proof")
+        if transcript_repr is None:
+            transcript_repr = self.transcript_repr
+        if rng_wide is None:
+            wide = np.frombuffer(os.urandom(64 * max(count, 1)), dtype=np.uint64).reshape(-1, 8)
+        else:
+            wide = np.ascontiguousarray(rng_wide, dtype=np.uint64).reshape(-1, 8)
+            if wide.shape[0] < count:
+                raise B200zkError(f"rng_wide too short: need {count} draws")
+        keep, lens = [], []
+        for instances in instances_list:
+            if len(instances) != len(instances_list[0]):
+                raise B200zkError("every proof needs the same number of instance columns")
+            cols = [np.ascontiguousarray(c, dtype=np.uint64).reshape(-1, 4) for c in instances]
+            lens += [c.shape[0] for c in cols]
+            keep += [c if c.shape[0] else np.zeros((1, 4), dtype=np.uint64) for c in cols]
+        bufs = [np.frombuffer(bytes(p), dtype=np.uint8) for p in proofs]
+        ptrs = (ctypes.c_void_p * max(count, 1))(*[b.ctypes.data if b.shape[0] else None for b in bufs])
+        plens = np.array([b.shape[0] for b in bufs] + [0], dtype=np.uint64)
+        lens = np.array(lens + [0], dtype=np.uint32)
+        fixed = self.fixed if self.fixed.shape[0] else np.zeros((1, 8), dtype=np.uint64)
+        sigma = self.sigma if self.sigma.shape[0] else np.zeros((1, 8), dtype=np.uint64)
+        status = np.zeros(max(count, 1), dtype=np.int32)
+        acc = np.zeros((2, 8), dtype=np.uint64)
+        rc = lib().b200zk_verify_proofs(backend._ctx, _p(self.blob), ctypes.c_size_t(self.blob.shape[0]), _p(fixed), _p(sigma), _p(self.g1),
+                                        _p(self.g2), _p(self.s_g2), ctypes.c_uint32(count), _ptr_array(keep), _p(lens),
+                                        _p(_fr(transcript_repr, 1)), ptrs, _p(plens), _p(wide), _p(status), _p(acc))
+        if rc != EVERIFY:
+            backend._check(rc)
+        ok = [int(s) == OK for s in status[:count]]
+        return (ok, (acc[0], acc[1])) if accumulator else ok
+
 
 _FR_ONE = [0xac96341c4ffffffb, 0x36fc76959f60cd29, 0x666ea36f7879462e, 0x0e0a77c19a07df2f]      # R mod r

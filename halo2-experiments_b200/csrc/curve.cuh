@@ -82,6 +82,38 @@ ZK_D void xyzz_add(xyzz_t& acc, const xyzz_t& q) {
     acc.zzz = Fq::mul(Fq::mul(acc.zzz, q.zzz), ppp);
 }
 
+// G1Affine::from_bytes (halo2curves 0.3.1 compressed form) of one point: x8 = the 32 bytes as 8 little-endian words,
+// x canonical < q with the parity of y in bit 31 of word 7, identity = all zero.  y = sqrt(x^3 + 3) with the stored parity.
+// Returns false (and the identity) for a non-canonical x, a sign bit on the identity or a point off the curve.
+ZK_D bool g1_decompress(const uint32_t x8[8], affine_t* out) {
+    fe_t x;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) x.l[j] = x8[j];
+    const uint32_t sign = x.l[7] >> 31;
+    x.l[7] &= 0x7fffffffu;
+    out->x = Fq::zero(); out->y = Fq::zero();
+    bool ge = true;                                              // x >= q ?
+    for (int j = 7; j >= 0; --j) { uint32_t pj = FqCfg::p(j); if (x.l[j] != pj) { ge = x.l[j] > pj; break; } }
+    if (ge) return false;
+    bool zero = true;
+    for (int j = 0; j < 8; ++j) zero &= x.l[j] == 0;
+    if (zero) return !sign;
+    fe_t xm = Fq::to_mont(x);
+    fe_t three = Fq::add(Fq::add(Fq::one(), Fq::one()), Fq::one());
+    fe_t rhs = Fq::add(Fq::mul(Fq::sqr(xm), xm), three);
+    // (q + 1) / 4
+    const uint32_t e[8] = {0xb61f3f52u, 0x4f082305u, 0x5a1c72a3u, 0x65e05aa4u, 0xa0605617u, 0x6e14116du, 0xb84c680au, 0x0c19139cu};
+    fe_t y = Fq::pow(rhs, e);
+    bool same = true;
+    fe_t y2 = Fq::sqr(y);
+    for (int j = 0; j < 8; ++j) same &= y2.l[j] == rhs.l[j];
+    if (!same) return false;
+    fe_t yc = Fq::from_mont(y);
+    if ((yc.l[0] & 1u) != sign) y = Fq::neg(y);
+    out->x = xm; out->y = y;
+    return true;
+}
+
 // k * p for a small scalar (double-and-add, MSB first)
 ZK_D xyzz_t xyzz_mul_small(const xyzz_t& p, uint32_t k) {
     xyzz_t acc = xyzz_identity();

@@ -33,37 +33,12 @@ __global__ void __launch_bounds__(FMT_THREADS) g1_compress_kernel(const affine_t
 #pragma unroll
     for (int j = 0; j < 8; ++j) out8[8 * i + j] = x.l[j];
 }
-// G1Affine::from_bytes: canonical x < q, y = sqrt(x^3 + 3) with the stored parity; *bad is set for a non-canonical x,
-// a sign bit on the identity or a point off the curve
+// G1Affine::from_bytes (g1_decompress, curve.cuh); *bad is set for any invalid encoding
 __global__ void __launch_bounds__(FMT_THREADS) g1_decompress_kernel(const uint32_t* in8, size_t n, affine_t* out, uint32_t* bad) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    fe_t x;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) x.l[j] = in8[8 * i + j];
-    const uint32_t sign = x.l[7] >> 31;
-    x.l[7] &= 0x7fffffffu;
-    bool ge = true;                                              // x >= q ?
-    for (int j = 7; j >= 0; --j) { uint32_t pj = FqCfg::p(j); if (x.l[j] != pj) { ge = x.l[j] > pj; break; } }
     affine_t r;
-    r.x = Fq::zero(); r.y = Fq::zero();
-    if (ge) { atomicOr(bad, 1u); out[i] = r; return; }
-    bool zero = true;
-    for (int j = 0; j < 8; ++j) zero &= x.l[j] == 0;
-    if (zero) { if (sign) atomicOr(bad, 1u); out[i] = r; return; }
-    fe_t xm = Fq::to_mont(x);
-    fe_t three = Fq::add(Fq::add(Fq::one(), Fq::one()), Fq::one());
-    fe_t rhs = Fq::add(Fq::mul(Fq::sqr(xm), xm), three);
-    // (q + 1) / 4
-    const uint32_t e[8] = {0xb61f3f52u, 0x4f082305u, 0x5a1c72a3u, 0x65e05aa4u, 0xa0605617u, 0x6e14116du, 0xb84c680au, 0x0c19139cu};
-    fe_t y = Fq::pow(rhs, e);
-    bool same = true;
-    fe_t y2 = Fq::sqr(y);
-    for (int j = 0; j < 8; ++j) same &= y2.l[j] == rhs.l[j];
-    if (!same) { atomicOr(bad, 1u); out[i] = r; return; }
-    fe_t yc = Fq::from_mont(y);
-    if ((yc.l[0] & 1u) != sign) y = Fq::neg(y);
-    r.x = xm; r.y = y;
+    if (!g1_decompress(in8 + 8 * i, &r)) atomicOr(bad, 1u);
     out[i] = r;
 }
 

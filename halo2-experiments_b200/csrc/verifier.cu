@@ -6,7 +6,9 @@
 //
 // Verification is O(#queries) field work, one ~100-term G1 combination and two Miller loops: it runs
 // on the caller's thread with no device and no ctx, exactly like the Blake2b transcript of the
-// prover.  The O(n) work a verifying key needs — the commitments to the fixed and permutation
+// prover.  replay_proof (verify_replay.hpp) is the transcript replay; it returns the opening as
+// linear terms, which b200zk_verify_proof evaluates here and b200zk_verify_proofs (verify_batch.cu)
+// evaluates on the device for many proofs at once.  The O(n) work a verifying key needs — the commitments to the fixed and permutation
 // polynomials (keygen_vk) — is done on the device by b200zk_pk_vk_commitments (prover.cu).
 #include <cstring>
 #include <vector>
@@ -14,6 +16,7 @@
 #include "cs_desc.hpp"
 #include "pairing.hpp"
 #include "transcript.hpp"
+#include "verify_replay.hpp"
 
 using namespace b200zk;
 using namespace b200zk::host;
@@ -60,17 +63,42 @@ HXyzz g1_mul(const HAffine& p, const HFr& s) {
     return acc;
 }
 
-// TranscriptRead side of Blake2bRead<_, G1Affine, Challenge255<_>> (src/transcript.rs)
+}  // namespace
+
+namespace b200zk {
+HAffine open_base_point(const VkPoints& vk, const HAffine* proof_points, const OpenBase& b) {
+    auto at = [](const void* base, size_t i) {
+        const uint64_t* p = (const uint64_t*)base + 8 * i;
+        return HAffine{HFq::from_limbs(p), HFq::from_limbs(p + 4)};
+    };
+    switch (b.kind) {
+    case OpenBase::FIXED: return at(vk.fixed, b.idx);
+    case OpenBase::SIGMA: return at(vk.sigma, b.idx);
+    case OpenBase::GEN: return at(vk.g1, 0);
+    default: return proof_points[b.idx];
+    }
+}
+}  // namespace b200zk
+
+namespace {
+
+// TranscriptRead side of Blake2bRead<_, G1Affine, Challenge255<_>> (src/transcript.rs).  Points are decompressed here,
+// or taken from `pre` (the proof's points decompressed by the caller, in read order); either way they are kept in `pts`.
 struct Reader {
     Transcript tr;
     const uint8_t* buf; size_t len, pos = 0; bool ok = true;
-    Reader(const uint8_t* b, size_t l) : buf(b), len(l) {}
-    HAffine read_point() {
+    const HAffine* pre;
+    std::vector<HAffine> pts;
+    Reader(const uint8_t* b, size_t l, const HAffine* p) : buf(b), len(l), pre(p) {}
+    uint32_t read_point() {
         HAffine p = {HFq::zero(), HFq::zero()};
-        if (!ok || pos + 32 > len || !decompress_g1(buf + pos, &p)) { ok = false; return {HFq::zero(), HFq::zero()}; }
-        pos += 32;
-        tr.common_point(p);
-        return p;
+        if (!ok || pos + 32 > len) ok = false;
+        else if (pre) p = pre[pts.size()];
+        else if (!decompress_g1(buf + pos, &p)) ok = false;
+        if (ok) { pos += 32; tr.common_point(p); }
+        else p = {HFq::zero(), HFq::zero()};
+        pts.push_back(p);
+        return (uint32_t)(pts.size() - 1);
     }
     HFr read_scalar() {
         if (!ok || pos + 32 > len) { ok = false; return HFr::zero(); }
@@ -116,8 +144,8 @@ int find_query(const std::vector<int32_t>& q, uint32_t col, int32_t rot) {
     return -1;
 }
 
-struct Query { int cid; HAffine c; HFr pt, eval; };
-struct CommitSet { int cid; HAffine c; std::vector<HFr> pts, evals; };     // one commitment, its points in first-seen order
+struct Query { int cid; OpenBase c; HFr pt, eval; };
+struct CommitSet { int cid; OpenBase c; std::vector<HFr> pts, evals; };     // one commitment, its points in first-seen order
 struct RotSet { std::vector<HFr> pts; std::vector<size_t> members; };        // sorted point set, commitments in first-seen order
 
 std::vector<HFr> interpolate(const std::vector<HFr>& pts, const std::vector<HFr>& evals) {
@@ -166,24 +194,28 @@ int32_t b200zk_pairing_check(const void* g1_points, const void* g2_points, size_
     return pairing_product_is_one(ps.data(), qs.data(), count) ? B200ZK_OK : B200ZK_EVERIFY;
 }
 
-int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const void* fixed_commitments,
-                            const void* sigma_commitments, const void* g1_generator, const void* g2, const void* s_g2,
-                            const void* const* instance_columns, const uint32_t* instance_lens, const void* transcript_repr,
-                            const uint8_t* proof, size_t proof_len) {
-    CsDesc cs;
-    if (!cs_blob || !parse_cs(cs_blob, blob_words, cs)) return B200ZK_EINVAL;
-    if (!g1_generator || !g2 || !s_g2 || !transcript_repr || (!proof && proof_len)) return B200ZK_EINVAL;
-    if ((cs.F && !fixed_commitments) || (!cs.perm.empty() && !sigma_commitments)) return B200ZK_EINVAL;
-    if (cs.I && (!instance_columns || !instance_lens)) return B200ZK_EINVAL;
-    if (cs.k < 1 || cs.k > FR_TWO_ADICITY) return B200ZK_EINVAL;
+
+}  // extern "C"
+
+namespace b200zk {
+
+size_t proof_point_offsets(const CsDesc& cs, std::vector<size_t>* offs) {
+    const size_t L = cs.lookups.size(), P = cs.perm.size(), chunk = cs.degree - 2, S = (P + chunk - 1) / chunk;
+    const size_t commitments = cs.A + 2 * L + S + L + 1 + (cs.degree - 1);
+    const size_t evals = cs.adv_q.size() / 2 + cs.fix_q.size() / 2 + 1 + P + (S ? 3 * S - 1 : 0) + 5 * L;
+    offs->clear();
+    for (size_t i = 0; i < commitments; ++i) offs->push_back(32 * i);
+    offs->push_back(32 * (commitments + evals));           // h1
+    offs->push_back(32 * (commitments + evals + 1));       // h2
+    return 32 * (commitments + evals + 2);
+}
+
+int32_t replay_proof(const CsDesc& cs, const VkPoints& vk, const void* const* instance_columns, const uint32_t* instance_lens,
+                     const void* transcript_repr, const uint8_t* proof, size_t proof_len, const HAffine* points, Opening* out) {
     const uint32_t k = cs.k, bf = cs.bf;
     const uint64_t n = 1ull << k;
     const size_t A = cs.A, L = cs.lookups.size(), P = cs.perm.size();
     const size_t chunk = cs.degree - 2, S = (P + chunk - 1) / chunk, q = cs.degree - 1;
-    auto affine_at = [](const void* base, size_t i) {
-        const uint64_t* p = (const uint64_t*)base + 8 * i;
-        return HAffine{HFq::from_limbs(p), HFq::from_limbs(p + 4)};
-    };
 
     // ---- instances: length check (Error::InstanceTooLarge), absorbed as scalars (KZG: query_instance = false)
     std::vector<std::vector<HFr>> inst(cs.I);
@@ -192,19 +224,19 @@ int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const vo
         if (instance_lens[c] && !instance_columns[c]) return B200ZK_EINVAL;
         for (uint32_t i = 0; i < instance_lens[c]; ++i) inst[c].push_back(HFr::from_limbs((const uint8_t*)instance_columns[c] + 32 * (size_t)i));
     }
-    Reader rd(proof, proof_len);
+    Reader rd(proof, proof_len, points);
     rd.tr.common_scalar(HFr::from_limbs(transcript_repr));
     for (auto& col : inst) for (auto& v : col) rd.tr.common_scalar(v);
 
-    // ---- commitments and challenges, in the prover's order (verifier.rs)
-    std::vector<HAffine> advice_c(A), lk_a(L), lk_s(L), perm_c(S), lk_z(L), h_c(q);
+    // ---- commitments (indices into rd.pts) and challenges, in the prover's order (verifier.rs)
+    std::vector<uint32_t> advice_c(A), lk_a(L), lk_s(L), perm_c(S), lk_z(L), h_c(q);
     for (auto& c : advice_c) c = rd.read_point();
     HFr theta = rd.squeeze();
     for (size_t i = 0; i < L; ++i) { lk_a[i] = rd.read_point(); lk_s[i] = rd.read_point(); }
     HFr beta = rd.squeeze(), gamma = rd.squeeze();
     for (auto& c : perm_c) c = rd.read_point();
     for (auto& c : lk_z) c = rd.read_point();
-    HAffine random_c = rd.read_point();
+    uint32_t random_c = rd.read_point();
     HFr y = rd.squeeze();
     for (auto& c : h_c) c = rd.read_point();
     HFr x = rd.squeeze();
@@ -303,43 +335,39 @@ int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const vo
         fold(l_active * ((e.a - e.s) * (e.a - e.a_prev)));
     }
     expected = expected * (xn - one).inv();
-    // h commitment: pieces folded in x^n
-    HXyzz h_acc = hx_identity();
-    for (size_t i = q; i-- > 0;) {
-        HAffine cur = hx_to_affine(h_acc);
-        h_acc = hx_add(g1_mul(cur, xn), hx_from_affine(h_c[i]));
-    }
-    HAffine h_commit = hx_to_affine(h_acc);
 
-    // ---- queries, in upstream's order (prover and verifier must agree on it: it fixes the y / v powers)
+    // ---- queries, in upstream's order (prover and verifier must agree on it: it fixes the y / v powers).  The h
+    // commitment is sum_i x^(n i) h_i: its query carries the marker H and is expanded into the h pieces below.
+    const OpenBase H = {OpenBase::PROOF, UINT32_MAX};
+    auto pt_of = [](uint32_t i) { return OpenBase{OpenBase::PROOF, i}; };
     std::vector<Query> Q;
     HFr x_next = rotate(x, 1), x_prev = rotate(x, -1), x_last = rotate(x, -(int)(bf + 1));
     int cid_pz = (int)A, cid_lk = cid_pz + (int)S, cid_fix = cid_lk + 3 * (int)L, cid_sig = cid_fix + (int)cs.F, cid_h = cid_sig + (int)P, cid_rand = cid_h + 1;
-    for (size_t i = 0; i < naq; ++i) Q.push_back({cs.adv_q[2 * i], advice_c[cs.adv_q[2 * i]], rotate(x, cs.adv_q[2 * i + 1]), advice_ev[i]});
+    for (size_t i = 0; i < naq; ++i) Q.push_back({cs.adv_q[2 * i], pt_of(advice_c[cs.adv_q[2 * i]]), rotate(x, cs.adv_q[2 * i + 1]), advice_ev[i]});
     for (size_t s = 0; s < S; ++s) {
-        Q.push_back({cid_pz + (int)s, perm_c[s], x, perm_ev[s].z});
-        Q.push_back({cid_pz + (int)s, perm_c[s], x_next, perm_ev[s].z_next});
+        Q.push_back({cid_pz + (int)s, pt_of(perm_c[s]), x, perm_ev[s].z});
+        Q.push_back({cid_pz + (int)s, pt_of(perm_c[s]), x_next, perm_ev[s].z_next});
     }
-    for (size_t s = S > 0 ? S - 1 : 0; s-- > 0;) Q.push_back({cid_pz + (int)s, perm_c[s], x_last, perm_ev[s].z_last});
+    for (size_t s = S > 0 ? S - 1 : 0; s-- > 0;) Q.push_back({cid_pz + (int)s, pt_of(perm_c[s]), x_last, perm_ev[s].z_last});
     for (size_t li = 0; li < L; ++li) {
         int b = cid_lk + 3 * (int)li;
         const LkEv& e = lk_ev[li];
-        Q.push_back({b, lk_z[li], x, e.z});
-        Q.push_back({b + 1, lk_a[li], x, e.a});
-        Q.push_back({b + 2, lk_s[li], x, e.s});
-        Q.push_back({b + 1, lk_a[li], x_prev, e.a_prev});
-        Q.push_back({b, lk_z[li], x_next, e.z_next});
+        Q.push_back({b, pt_of(lk_z[li]), x, e.z});
+        Q.push_back({b + 1, pt_of(lk_a[li]), x, e.a});
+        Q.push_back({b + 2, pt_of(lk_s[li]), x, e.s});
+        Q.push_back({b + 1, pt_of(lk_a[li]), x_prev, e.a_prev});
+        Q.push_back({b, pt_of(lk_z[li]), x_next, e.z_next});
     }
-    for (size_t i = 0; i < nfq; ++i) Q.push_back({cid_fix + cs.fix_q[2 * i], affine_at(fixed_commitments, cs.fix_q[2 * i]), rotate(x, cs.fix_q[2 * i + 1]), fixed_ev[i]});
-    for (size_t j = 0; j < P; ++j) Q.push_back({cid_sig + (int)j, affine_at(sigma_commitments, j), x, sigma_ev[j]});
-    Q.push_back({cid_h, h_commit, x, expected});
-    Q.push_back({cid_rand, random_c, x, random_ev});
+    for (size_t i = 0; i < nfq; ++i) Q.push_back({cid_fix + cs.fix_q[2 * i], {OpenBase::FIXED, (uint32_t)cs.fix_q[2 * i]}, rotate(x, cs.fix_q[2 * i + 1]), fixed_ev[i]});
+    for (size_t j = 0; j < P; ++j) Q.push_back({cid_sig + (int)j, {OpenBase::SIGMA, (uint32_t)j}, x, sigma_ev[j]});
+    Q.push_back({cid_h, H, x, expected});
+    Q.push_back({cid_rand, pt_of(random_c), x, random_ev});
 
     // ---- SHPLONK (shplonk/verifier.rs)
     HFr ch_y = rd.squeeze(), ch_v = rd.squeeze();
-    HAffine h1 = rd.read_point();
+    uint32_t h1 = rd.read_point();
     HFr u = rd.squeeze();
-    HAffine h2 = rd.read_point();
+    uint32_t h2 = rd.read_point();
     if (!rd.ok) return B200ZK_EVERIFY;
     // construct_intermediate_sets: commitments in first-seen order; rotation sets keyed by the point set
     std::vector<CommitSet> csets;
@@ -370,15 +398,18 @@ int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const vo
         for (auto& r : roots) if (!except || !has(*except, r)) acc = acc * (u - r);
         return acc;
     };
-    // L = sum_i v^i z_i sum_j y^j (C_ij - [r_ij(u)] G) - Z_T(u) h1;  accept iff e(h2, [s]_2) = e(u h2 + L / z_0, [1]_2)
-    HAffine G = affine_at(g1_generator, 0);
-    HXyzz Lpt = hx_identity();
-    HFr g_scalar = HFr::zero(), v_pow = HFr::one(), z0 = HFr::zero();
+    // L = sum_i v^i z_i sum_j y^j (C_ij - [r_ij(u)] G) - Z_T(u) h1;  the opening is (h2, u h2 + L / z_0)
+    HFr z0 = vanish(super_pts, rsets.empty() ? nullptr : &rsets[0].pts);
+    if (rsets.empty() || z0.is_zero()) return B200ZK_EVERIFY;
+    const HFr z0_inv = z0.inv();
+    out->points = std::move(rd.pts);
+    out->h2 = h2;
+    out->right.clear();
+    out->right.push_back({pt_of(h2), u});
+    HFr g_scalar = HFr::zero(), v_pow = HFr::one();
     for (size_t ri = 0; ri < rsets.size(); ++ri) {
         const RotSet& rs = rsets[ri];
-        HFr z_i = vanish(super_pts, &rs.pts);
-        if (ri == 0) z0 = z_i;
-        HFr y_pow = HFr::one(), zv = z_i * v_pow;
+        HFr y_pow = HFr::one(), zv = vanish(super_pts, &rs.pts) * v_pow;
         for (size_t ci : rs.members) {
             const CommitSet& c = csets[ci];
             std::vector<HFr> ev(rs.pts.size());
@@ -388,18 +419,45 @@ int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const vo
             HFr r_eval = HFr::zero();
             for (size_t i = low.size(); i-- > 0;) r_eval = r_eval * u + low[i];
             HFr sc = zv * y_pow;
-            Lpt = hx_add(Lpt, g1_mul(c.c, sc));
+            if (c.c.kind == H.kind && c.c.idx == H.idx) {
+                HFr w = sc * z0_inv;
+                for (size_t i = 0; i < q; ++i) { out->right.push_back({pt_of(h_c[i]), w}); w = w * xn; }
+            } else {
+                out->right.push_back({c.c, sc * z0_inv});
+            }
             g_scalar = g_scalar - sc * r_eval;
             y_pow = y_pow * ch_y;
         }
         v_pow = v_pow * ch_v;
     }
-    Lpt = hx_add(Lpt, g1_mul(G, g_scalar));
-    Lpt = hx_add(Lpt, g1_mul(h1, vanish(super_pts, nullptr).neg()));
-    if (z0.is_zero()) return B200ZK_EVERIFY;
-    HXyzz rhs = hx_add(g1_mul(h2, u), g1_mul(hx_to_affine(Lpt), z0.inv()));
+    out->right.push_back({{OpenBase::GEN, 0}, g_scalar * z0_inv});
+    out->right.push_back({pt_of(h1), vanish(super_pts, nullptr).neg() * z0_inv});
+    return B200ZK_OK;
+}
+
+}  // namespace b200zk
+
+extern "C" {
+
+int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const void* fixed_commitments,
+                            const void* sigma_commitments, const void* g1_generator, const void* g2, const void* s_g2,
+                            const void* const* instance_columns, const uint32_t* instance_lens, const void* transcript_repr,
+                            const uint8_t* proof, size_t proof_len) {
+    CsDesc cs;
+    if (!cs_blob || !parse_cs(cs_blob, blob_words, cs)) return B200ZK_EINVAL;
+    if (!g1_generator || !g2 || !s_g2 || !transcript_repr || (!proof && proof_len)) return B200ZK_EINVAL;
+    if ((cs.F && !fixed_commitments) || (!cs.perm.empty() && !sigma_commitments)) return B200ZK_EINVAL;
+    if (cs.I && (!instance_columns || !instance_lens)) return B200ZK_EINVAL;
+    if (cs.k < 1 || cs.k > FR_TWO_ADICITY) return B200ZK_EINVAL;
+    const VkPoints vk = {fixed_commitments, sigma_commitments, g1_generator};
+    Opening op;
+    int32_t rc = replay_proof(cs, vk, instance_columns, instance_lens, transcript_repr, proof, proof_len, nullptr, &op);
+    if (rc != B200ZK_OK) return rc;
+    // accept iff e(h2, [s]_2) = e(right, [1]_2)
+    HXyzz rhs = hx_identity();
+    for (const OpenTerm& t : op.right) rhs = hx_add(rhs, g1_mul(open_base_point(vk, op.points.data(), t.base), t.scalar));
     HAffine rhs_a = hx_to_affine(rhs);
-    HAffine ps[2] = {h2, {rhs_a.x, rhs_a.y.neg()}};
+    HAffine ps[2] = {op.points[op.h2], {rhs_a.x, rhs_a.y.neg()}};
     if (rhs_a.x.is_zero() && rhs_a.y.is_zero()) ps[1] = rhs_a;
     G2A qs[2] = {g2_from_limbs(s_g2), g2_from_limbs(g2)};
     if (!g2_on_curve(qs[0]) || !g2_on_curve(qs[1]) || g2_is_identity(qs[0]) || g2_is_identity(qs[1])) return B200ZK_EINVAL;

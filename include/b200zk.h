@@ -317,6 +317,35 @@ int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const vo
                             const void* sigma_commitments, const void* g1_generator, const void* g2, const void* s_g2,
                             const void* const* instance_columns, const uint32_t* instance_lens,
                             const void* transcript_repr, const uint8_t* proof, size_t proof_len);
+/* ---- many proofs of one verifying key with one pairing check (an extension in the sense of b200zk_create_proofs) ----
+ * Upstream's AccumulatorStrategy (src/poly/kzg/strategy.rs) over VerifierSHPLONK / Blake2bRead / Challenge255.
+ * Inputs: as b200zk_verify_proof, for `count` proofs of one vk.  Proof i uses instance_columns[i*I + c],
+ * instance_lens[i*I + c] (the indexing of b200zk_create_proofs) and proofs[i] / proof_lens[i]; all proofs share
+ * transcript_repr.
+ * Randomness: r_i = Fr::from_bytes_wide(rng_wide[64 i .. 64 i + 64]), one draw per proof, as `process` draws one
+ * Fr::random per proof; the call is a pure function of its inputs.  The draws MUST be fresh and secret for every call
+ * (the Rust shim fills them from OsRng): a prover who can predict them can make a batch with false proofs pass.
+ * Stage 1, per proof, exactly the replay of b200zk_verify_proof: a proof that is malformed or truncated, has a
+ * non-canonical scalar or point, a point off the curve, an instance that is too large, x^n = 1 or z_0 = 0 gets
+ * status[i] = B200ZK_EVERIFY and adds nothing to the accumulator.  Bytes after the last proof element are ignored.
+ * Points are decompressed on the device; the transcripts are replayed on a pool of library threads.
+ * Accumulator: accumulator_out (if not NULL) receives (left, right) = sum_i c_i (h2_i, u_i h2_i + L_i / z0_i) over the
+ * proofs that passed stage 1, c_i = r_{i+1} * ... * r_{count-1}, as two 64-byte G1Affine (identity (0,0)).  When every
+ * proof passes stage 1 this is the DualMSM AccumulatorStrategy holds after `process` on proofs 0 .. count-1 in order.
+ * Stage 2: one pairing check e(left, [s]_2) e(-right, [1]_2) = 1.  If it fails, bisection over the stage-1 survivors
+ * (sums of their c_i-scaled pairs, no device work) finds the failing proofs.  Every status[i] ends 0 or B200ZK_EVERIFY.
+ * Returns B200ZK_OK when every proof is accepted, B200ZK_EVERIFY when at least one is rejected (status says which),
+ * B200ZK_EINVAL before any device work for a bad argument (null pointers, count == 0, a cs blob that does not parse,
+ * proofs[i] == NULL with a nonzero length, an invalid G2 point; b200zk_launch_count does not move), otherwise the CUDA
+ * or memory code.  ctx may be any ctx, a rank of a sharded group or one holding a pk with lanes included: the call uses
+ * only its stream and workspaces and leaves any pk on it untouched. */
+int32_t b200zk_verify_proofs(b200zk_ctx* ctx, const uint32_t* cs_blob, size_t blob_words,
+                             const void* fixed_commitments, const void* sigma_commitments,
+                             const void* g1_generator, const void* g2, const void* s_g2,
+                             uint32_t count, const void* const* instance_columns, const uint32_t* instance_lens,
+                             const void* transcript_repr, const uint8_t* const* proofs, const size_t* proof_lens,
+                             const void* rng_wide /* count * 64 bytes */, int32_t* status /* count */,
+                             void* accumulator_out /* 2 x 64-byte G1Affine (left, right), or NULL */);
 /* ParamsKZG::setup's G2 side: out = s * base (base NULL = the G2 generator, i.e. out = [s]_2). */
 int32_t b200zk_g2_mul(const void* g2_or_null, const void* s_fr, void* out_g2);
 /* prod e(g1_points[i], g2_points[i]) == 1 ?  0 = yes, B200ZK_EVERIFY = no (Engine::pairing product;

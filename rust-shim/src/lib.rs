@@ -4,7 +4,7 @@
 pub mod dump;
 pub mod sys;
 
-use halo2_proofs::halo2curves::bn256::{Fr, G1Affine, G1};
+use halo2_proofs::halo2curves::bn256::{Fr, G1Affine, G2Affine, G1};
 use halo2_proofs::halo2curves::group::Curve;
 use halo2_proofs::plonk::{Any, ConstraintSystem, Expression};
 use rand_core::{CryptoRng, RngCore};
@@ -171,6 +171,37 @@ impl Drop for Pk {
         unsafe { sys::b200zk_pk_destroy(self.0) }
     }
 }
+
+/// Extension in the sense of `Pk::create_proofs`: plonk::verify_proof for many proofs of one verifying key with
+/// AccumulatorStrategy (src/poly/kzg/strategy.rs), one pairing check for the batch (b200zk_verify_proofs).  `fixed` /
+/// `sigma`: the vk's commitments; `g` = params.get_g()[0]; `g2` / `s_g2` = params.g2() / s_g2().  One Fr::random draw
+/// per proof comes from OsRng, as `process` makes it; they must stay secret.  Entry i is verify_proof's verdict on
+/// proof i, the pairing included.
+pub fn verify_proofs(cs: &ConstraintSystem<Fr>, k: u32, fixed: &[G1Affine], sigma: &[G1Affine], g: &G1Affine, g2: &G2Affine,
+                     s_g2: &G2Affine, instances: &[Vec<&[Fr]>], proofs: &[&[u8]], transcript_repr: &Fr) -> Vec<bool> {
+    let count = proofs.len();
+    assert_eq!(instances.len(), count);
+    let blob = cs_blob(cs, k);
+    let inst: Vec<*const c_void> = instances.iter().flat_map(|i| i.iter().map(|c| c.as_ptr() as *const c_void)).collect();
+    let lens: Vec<u32> = instances.iter().flat_map(|i| i.iter().map(|c| c.len() as u32)).collect();
+    let ptrs: Vec<*const u8> = proofs.iter().map(|p| p.as_ptr()).collect();
+    let plens: Vec<usize> = proofs.iter().map(|p| p.len()).collect();
+    let mut rng_wide = vec![0u8; 64 * count];
+    rand_core::OsRng.fill_bytes(&mut rng_wide);
+    let mut status = vec![0i32; count];
+    let rc = unsafe {
+        sys::b200zk_verify_proofs(ctx(), blob.as_ptr(), blob.len(), fixed.as_ptr() as *const c_void, sigma.as_ptr() as *const c_void,
+                                  g as *const G1Affine as *const c_void, g2 as *const G2Affine as *const c_void,
+                                  s_g2 as *const G2Affine as *const c_void, count as u32, inst.as_ptr(), lens.as_ptr(),
+                                  transcript_repr as *const Fr as *const c_void, ptrs.as_ptr(), plens.as_ptr(),
+                                  rng_wide.as_ptr() as *const c_void, status.as_mut_ptr(), std::ptr::null_mut())
+    };
+    if rc != sys::B200ZK_EVERIFY {
+        check(rc);
+    }
+    status.iter().map(|&s| s == 0).collect()
+}
+
 
 // ---------------------------------------------------------------------------------------------------------------------
 // ConstraintSystem -> the word format of halo2-experiments_b200/circuit.py::ConstraintSystem.to_blob (parsed by
