@@ -669,6 +669,21 @@ def pairing_check(g1_points, g2_points):
     return rc == OK
 
 
+def pairing_checks(backend, g1_points, g2_points, m):
+    """Many pairing-product checks on the device (b200zk_pairing_checks): check j is prod_{i < m} e(P[j m + i], Q[j m + i])
+    == 1 over G1Affine (count * m, 8) and G2Affine (count * m, 16) Montgomery limbs.  Returns the int32 status array,
+    0 where the product is one and EVERIFY where it is not."""
+    a = np.ascontiguousarray(g1_points, dtype=np.uint64).reshape(-1, 8)
+    b = np.ascontiguousarray(g2_points, dtype=np.uint64).reshape(-1, 16)
+    if m < 1 or a.shape[0] != b.shape[0] or a.shape[0] % m:
+        raise B200zkError("pairing_checks: the point counts are not count * m")
+    status = np.zeros(a.shape[0] // m, dtype=np.int32)
+    rc = lib().b200zk_pairing_checks(backend._ctx, _p(a), _p(b), ctypes.c_uint32(m), ctypes.c_uint32(status.shape[0]), _p(status))
+    if rc != EVERIFY:
+        backend._check(rc)
+    return status
+
+
 class VerifyingKey:
     """What plonk::verify_proof reads of a VerifyingKey: the constraint system, k, and the commitments to
     the fixed and permutation polynomials (ProvingKey.vk_commitments()); plus the verifier params

@@ -158,6 +158,13 @@ int32_t g_to_lagrange_run(b200zk_ctx* ctx, const affine_t* d_g, uint32_t k, affi
 // out[i] = base^i, i < n (two-level tables built on the device)
 int32_t powers_run(b200zk_ctx* ctx, const host::HFr& base, size_t n, fe_t* d_out);
 
+// pairing.cu ------------------------------------------------------------------
+// for j < count: status[j] = prod_{i < m} e(g1[j m + i], Q_{q[j m + i]}) == 1 ? B200ZK_OK : B200ZK_EVERIFY.  g1: host
+// G1Affine on the curve; q: host indices into the nq G2Affine points g2 (128 B each, on the twist, not the identity), or
+// PC_SKIP (pairing.cuh) for a pair that contributes 1.  Three launches; buffers in io_a and setup_ws.
+int32_t pairing_checks_run(b200zk_ctx* ctx, const void* g1, const uint32_t* q, const void* g2, uint32_t nq, uint32_t m, uint32_t count,
+                           int32_t* status);
+
 // lookup_sort.cu --------------------------------------------------------------
 int32_t lookup_permute_run(b200zk_ctx* ctx, const fe_t* d_in, const fe_t* d_tab, uint32_t u, fe_t* d_pin, fe_t* d_ptab, uint32_t* d_err);
 

@@ -6,8 +6,10 @@
 // verifier.cu), each giving the proof's opening (h2, right) as linear terms over proof points, vk commitments and G.
 // Stage 2: the scalars of proof i are multiplied by c_i = prod_{j > i} r_j on the host; one launch computes every term
 // c_i s * B (one thread per term, xyzz_mul), one launch sums each proof's terms (one warp per segment), so every proof
-// ends with its own pair c_i (left_i, right_i).  The accumulator is the host sum of the pairs; one pairing checks it.
-// If it fails, bisection over the pairs finds the failing proofs with host sums and pairings only.
+// ends with its own pair c_i (left_i, right_i).  The accumulator is the host sum of the pairs; one host pairing checks it
+// (a lone device check is no faster: DESIGN.md §6.5).  If it fails, one device call (pairing_checks_run, pairing.cu)
+// checks every pair on its own, so each proof's status is its own verdict and the launches do not depend on how many
+// proofs fail.
 #include "context.hpp"
 #include "g1_ntt.cuh"
 #include "pairing.hpp"
@@ -78,24 +80,22 @@ unsigned blocks_for(size_t threads) { return (unsigned)((threads + VB_THREADS - 
 
 struct Pair { HXyzz left, right; };
 
-// e(sum left, [s]_2) * e(-sum right, [1]_2) == 1 over pairs[idx[lo .. hi)]
-bool pairs_check(const std::vector<Pair>& pairs, size_t lo, size_t hi, const G2A qs[2]) {
-    HXyzz l = hx_identity(), r = hx_identity();
-    for (size_t i = lo; i < hi; ++i) { l = hx_add(l, pairs[i].left); r = hx_add(r, pairs[i].right); }
-    HAffine la = hx_to_affine(l), ra = hx_to_affine(r);
-    HAffine ps[2] = {la, {ra.x, ra.y.neg()}};
-    return pairing_product_is_one(ps, qs, 2);
-}
+constexpr uint32_t PAIR_SKIP = 0xffffffffu;                    // PC_SKIP of pairing.cuh
 
-// marks the failing pairs of [lo, hi); `fails` = the range is already known to fail.  If a range fails and its left
-// half passes, its right half fails: the pairing check is bilinear, so two passing halves make a passing whole.
-void locate(const std::vector<Pair>& pairs, size_t lo, size_t hi, bool fails, const G2A qs[2], std::vector<bool>* bad) {
-    if (!fails && pairs_check(pairs, lo, hi, qs)) return;
-    if (hi - lo == 1) { (*bad)[lo] = true; return; }
-    const size_t mid = lo + (hi - lo) / 2;
-    if (pairs_check(pairs, lo, mid, qs)) { locate(pairs, mid, hi, true, qs, bad); return; }
-    locate(pairs, lo, mid, true, qs, bad);
-    locate(pairs, mid, hi, false, qs, bad);
+// e(left_j, [s]_2) * e(-right_j, [1]_2) == 1 for every pair, on the device; an identity point contributes 1
+int32_t pairs_check(b200zk_ctx* ctx, const std::vector<Pair>& pairs, const void* s_g2, const void* g2, int32_t* status) {
+    const size_t n = pairs.size();
+    std::vector<HAffine> aff(2 * n);
+    hx_batch_to_affine(&pairs[0].left, 2 * n, aff.data());
+    std::vector<uint32_t> q(2 * n);
+    for (size_t j = 0; j < n; ++j) {
+        aff[2 * j + 1].y = aff[2 * j + 1].y.neg();
+        for (int h = 0; h < 2; ++h) q[2 * j + h] = aff[2 * j + h].x.is_zero() && aff[2 * j + h].y.is_zero() ? PAIR_SKIP : h;
+    }
+    uint8_t qs[256];
+    memcpy(qs, s_g2, 128);
+    memcpy(qs + 128, g2, 128);
+    return pairing_checks_run(ctx, aff.data(), q.data(), qs, 2, 2, (uint32_t)n, status);
 }
 
 void store_affine(const HAffine& a, void* out) { a.x.store(out); a.y.store((uint8_t*)out + 32); }
@@ -251,17 +251,19 @@ extern "C" int32_t b200zk_verify_proofs(b200zk_ctx* ctx, const uint32_t* cs_blob
         ZK_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     }
 
-    // ---- stage 2c: the accumulator, one pairing check, and bisection when it fails
+    // ---- stage 2c: the accumulator and its pairing check; when it fails, every pair's own check on the device
+    HXyzz l = hx_identity(), r = hx_identity();
+    for (const Pair& p : pairs) { l = hx_add(l, p.left); r = hx_add(r, p.right); }
+    const HAffine la = hx_to_affine(l), ra = hx_to_affine(r);
     if (accumulator_out) {
-        HXyzz l = hx_identity(), r = hx_identity();
-        for (const Pair& p : pairs) { l = hx_add(l, p.left); r = hx_add(r, p.right); }
-        store_affine(hx_to_affine(l), accumulator_out);
-        store_affine(hx_to_affine(r), (uint8_t*)accumulator_out + 64);
+        store_affine(la, accumulator_out);
+        store_affine(ra, (uint8_t*)accumulator_out + 64);
     }
-    if (!pairs.empty()) {
-        std::vector<bool> failed(pairs.size(), false);
-        locate(pairs, 0, pairs.size(), false, qs, &failed);
-        for (size_t j = 0; j < pairs.size(); ++j) if (failed[j]) status[surv[j]] = B200ZK_EVERIFY;
+    const HAffine acc[2] = {la, {ra.x, ra.y.neg()}};
+    if (!pairs.empty() && !pairing_product_is_one(acc, qs, 2)) {
+        std::vector<int32_t> own(pairs.size());
+        ZK_TRY(pairs_check(ctx, pairs, s_g2, g2, own.data()));
+        for (size_t j = 0; j < pairs.size(); ++j) if (own[j] != B200ZK_OK) status[surv[j]] = B200ZK_EVERIFY;
     }
     for (uint32_t i = 0; i < count; ++i) if (status[i] != B200ZK_OK) return B200ZK_EVERIFY;
     return B200ZK_OK;

@@ -332,8 +332,10 @@ int32_t b200zk_verify_proof(const uint32_t* cs_blob, size_t blob_words, const vo
  * Accumulator: accumulator_out (if not NULL) receives (left, right) = sum_i c_i (h2_i, u_i h2_i + L_i / z0_i) over the
  * proofs that passed stage 1, c_i = r_{i+1} * ... * r_{count-1}, as two 64-byte G1Affine (identity (0,0)).  When every
  * proof passes stage 1 this is the DualMSM AccumulatorStrategy holds after `process` on proofs 0 .. count-1 in order.
- * Stage 2: one pairing check e(left, [s]_2) e(-right, [1]_2) = 1.  If it fails, bisection over the stage-1 survivors
- * (sums of their c_i-scaled pairs, no device work) finds the failing proofs.  Every status[i] ends 0 or B200ZK_EVERIFY.
+ * Stage 2: one pairing check e(left, [s]_2) e(-right, [1]_2) = 1.  If it fails, one device call (the three kernels of
+ * b200zk_pairing_checks) checks every stage-1 survivor's own c_i-scaled pair, so status[i] is then exactly
+ * verify_proof's verdict for proof i, and the launch count does not depend on how many proofs fail.  Every status[i]
+ * ends 0 or B200ZK_EVERIFY.
  * Returns B200ZK_OK when every proof is accepted, B200ZK_EVERIFY when at least one is rejected (status says which),
  * B200ZK_EINVAL before any device work for a bad argument (null pointers, count == 0, a cs blob that does not parse,
  * proofs[i] == NULL with a nonzero length, an invalid G2 point; b200zk_launch_count does not move), otherwise the CUDA
@@ -351,6 +353,17 @@ int32_t b200zk_g2_mul(const void* g2_or_null, const void* s_fr, void* out_g2);
 /* prod e(g1_points[i], g2_points[i]) == 1 ?  0 = yes, B200ZK_EVERIFY = no (Engine::pairing product;
  * G1Affine 64 B, G2Affine 128 B each). */
 int32_t b200zk_pairing_check(const void* g1_points, const void* g2_points, size_t count);
+/* Many pairing-product checks in one call, on the device (halo2curves' multi_miller_loop(..).final_exponentiation()
+ * compared with the identity, batched; e.g. one DualMSM::check per accumulator of a pile):
+ * for j < count: prod_{i < m} e(g1_points[j*m + i], g2_points[j*m + i]) == 1 ?  status[j] = 0 or B200ZK_EVERIFY.
+ * G1Affine 64 B, G2Affine 128 B (the layout of b200zk_pairing_check); a pair with an identity on either side
+ * contributes 1.  The pairing is b200zk_pairing_check's, so every verdict is the one it gives for the same m pairs.
+ * G2 points are compared by their bytes: each distinct point's Miller-loop lines are computed once per call.
+ * Returns B200ZK_OK when every check holds, B200ZK_EVERIFY when at least one fails, B200ZK_EINVAL before any device
+ * work (b200zk_launch_count does not move) for null pointers, count == 0, m == 0 or a point off its curve, otherwise
+ * the CUDA or memory code.  Runs on the ctx stream with the ctx workspaces; three launches. */
+int32_t b200zk_pairing_checks(b200zk_ctx* ctx, const void* g1_points, const void* g2_points,
+                              uint32_t m, uint32_t count, int32_t* status);
 
 /* ---- formats (SURVEY.md 8(f3)): halo2_proofs v2023_02_02 ParamsKZG::write / read (src/poly/kzg/commitment.rs),
  *      VerifyingKey::write / read commitments (src/plonk.rs), halo2curves G1Affine / G2Affine to_bytes / from_bytes,

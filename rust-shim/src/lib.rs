@@ -202,6 +202,23 @@ pub fn verify_proofs(cs: &ConstraintSystem<Fr>, k: u32, fixed: &[G1Affine], sigm
     status.iter().map(|&s| s == 0).collect()
 }
 
+/// Many `multi_miller_loop(..).final_exponentiation() == Gt::identity()` checks on the device in one call
+/// (b200zk_pairing_checks): check j multiplies the m pairs `pairs[j * m .. (j + 1) * m]`.  One verdict per check.
+pub fn pairing_checks(pairs: &[(G1Affine, G2Affine)], m: usize) -> Vec<bool> {
+    assert!(m > 0 && !pairs.is_empty() && pairs.len() % m == 0);
+    let g1: Vec<G1Affine> = pairs.iter().map(|p| p.0).collect();
+    let g2: Vec<G2Affine> = pairs.iter().map(|p| p.1).collect();
+    let mut status = vec![0i32; pairs.len() / m];
+    let rc = unsafe {
+        sys::b200zk_pairing_checks(ctx(), g1.as_ptr() as *const c_void, g2.as_ptr() as *const c_void, m as u32, status.len() as u32,
+                                   status.as_mut_ptr())
+    };
+    if rc != sys::B200ZK_EVERIFY {
+        check(rc);
+    }
+    status.iter().map(|&s| s == 0).collect()
+}
+
 
 // ---------------------------------------------------------------------------------------------------------------------
 // ConstraintSystem -> the word format of halo2-experiments_b200/circuit.py::ConstraintSystem.to_blob (parsed by
